@@ -62,9 +62,14 @@ typedef struct {
                                      captured_lut the hi-2 variant (maenv:87-199) */
     const float *rank_lut;        /* [14] original mode: normalised true rank 0..12 (entry 13 unused) */
     const float *po_rank_lut;     /* [14] original mode: normalised partially observable rank 0..13 */
+    int32_t obs_dtype;            /* element type of every observation output (partial / full, terminal, sx_observe,
+                                     sx_host_env): SX_DTYPE_F32 (0, the default of a zeroed descriptor), SX_DTYPE_BF16 or
+                                     SX_DTYPE_F16.  A 16-bit element is the round-to-nearest-even conversion of the
+                                     float32 the SX_DTYPE_F32 configuration writes for the same state */
 } sx_config_desc;
 
 enum { SX_CHANNELS_EXTENDED = 0, SX_CHANNELS_ORIGINAL = 1 };
+enum { SX_DTYPE_F32 = 0, SX_DTYPE_BF16 = 1, SX_DTYPE_F16 = 2 }; /* obs_dtype; also the logits types of the samplers */
 
 /* Byte/element strides of the device tensors for one variant. */
 typedef struct {
@@ -75,10 +80,11 @@ typedef struct {
     int32_t board_stride;         /* uint8 per env (cells rounded up to 16) */
     int32_t aux_stride;           /* int16 per env (= 8) */
     int32_t captured_stride;      /* uint16 per env */
-    int32_t po_floats, fo_floats; /* float32 per env of each observation */
+    int32_t po_floats, fo_floats; /* elements per env of each observation (float32 or 16-bit: obs_elem_bytes) */
     int32_t setup_len;            /* usable_rows*cols bytes per setup-table row */
     int32_t pieces_per_side;
     int32_t po_channels, fo_channels; /* 67 / 79, or 32 / 33 in the original channel mode */
+    int32_t obs_elem_bytes;       /* 4 (SX_DTYPE_F32) or 2 (SX_DTYPE_BF16 / SX_DTYPE_F16) */
 } sx_layout;
 
 /* Compact struct-of-arrays device state (DESIGN.md "State layout"). */
@@ -88,10 +94,11 @@ typedef struct {
     uint16_t *captured; /* [num_envs][captured_stride] (cell, owner, type, count) capture entries */
 } sx_state;
 
-/* Per-step outputs; any pointer may be NULL to skip that output. */
+/* Per-step outputs; any pointer may be NULL to skip that output.  The four observation pointers are typed float, but
+ * their elements are of the configuration's obs_dtype (float32, or bfloat16 / float16: 2 bytes each). */
 typedef struct {
-    float *partial_obs;      /* [num_envs][R][C][67 | 32] float32, maenv:461-475 (normalised) */
-    float *full_obs;         /* [num_envs][R][C][79 | 33] float32, maenv:480-492 (normalised) */
+    float *partial_obs;      /* [num_envs][R][C][67 | 32] obs_dtype, maenv:461-475 (normalised) */
+    float *full_obs;         /* [num_envs][R][C][79 | 33] obs_dtype, maenv:480-492 (normalised) */
     uint8_t *valid_mask;     /* [num_envs][R][C][A] uint8 0/1, maenv:454 / impl:400-517 */
     float *reward;           /* [num_envs] player +1's reward when the game ended this step, else 0
                                 (maenv:777-801: +-1, or 0 for an invalid ending) */
@@ -217,7 +224,6 @@ int sx_sample_valid(const uint8_t *mask_d, int64_t num_envs, int32_t mask_len, i
  * keyed by (seed, env_base + b, step, entry)); invalid entries have probability exactly 0.  logits_d is
  * [num_envs][n_actions] of logits_dtype; logprob_d (optional) receives log p(action).  actions_d[b] = -1 when a
  * mask row has no valid entry. */
-enum { SX_DTYPE_F32 = 0, SX_DTYPE_BF16 = 1, SX_DTYPE_F16 = 2 };
 int sx_sample_logits(const void *logits_d, int32_t logits_dtype, const uint8_t *mask_d, int64_t num_envs,
                      int32_t n_actions, int64_t env_base, uint64_t seed, uint32_t step, float temperature,
                      int32_t *actions_d, float *logprob_d, void *stream);

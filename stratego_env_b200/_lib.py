@@ -15,19 +15,21 @@ SX_AUTO_RESET, SX_SAMPLE_NEXT, SX_ALLOW_OSCILLATION, SX_RESET_RANDOM_SHUFFLE, SX
 SX_SAME_SETUP, SX_REPEAT_OTHER_SIDE = 32, 64
 OBS_PO, OBS_FO, OBS_MASK = 1, 2, 4
 SX_CHANNELS_EXTENDED, SX_CHANNELS_ORIGINAL = 0, 1
+SX_DTYPE_F32, SX_DTYPE_BF16, SX_DTYPE_F16 = 0, 1, 2
 
 
 class SxConfigDesc(C.Structure):
     _fields_ = [("rows", _i32), ("cols", _i32), ("max_turns", _i32), ("usable_rows", _i32),
                 ("piece_amounts", _i32 * 13), ("obstacles", _vp), ("captured_lut", _vp), ("recent_lut", _vp),
                 ("unit_lut", _vp), ("p2_rot180", _i32), ("capture_capacity", _i32), ("obs_channel_mode", _i32),
-                ("rank_lut", _vp), ("po_rank_lut", _vp)]
+                ("rank_lut", _vp), ("po_rank_lut", _vp), ("obs_dtype", _i32)]
 
 
 class SxLayout(C.Structure):
     _fields_ = [(n, _i32) for n in ("rows", "cols", "cells", "spatial_channels", "spatial_actions", "action_size",
                                     "board_stride", "aux_stride", "captured_stride", "po_floats", "fo_floats",
-                                    "setup_len", "pieces_per_side", "po_channels", "fo_channels")]
+                                    "setup_len", "pieces_per_side", "po_channels", "fo_channels",
+                                    "obs_elem_bytes")]
 
 
 class SxState(C.Structure):

@@ -4,7 +4,8 @@
 launch of the fused sm_100a kernel (action decode -> move / combat -> outcome -> auto-reset -> next
 player's mask + observations [-> uniform valid-action sample]) and everything it returns is a torch CUDA
 tensor -- nothing crosses PCIe unless the caller asks.  Observation keys and layouts are the reference's
-(``ObservationComponents``; HWC float32 observations; the mask is uint8 instead of the reference's int64).
+(``ObservationComponents``; HWC float32 observations, or bfloat16 / float16 with ``obs_dtype``; the mask is uint8
+instead of the reference's int64).
 
 Semantics that differ from the one-game API because many games advance at once:
   * obs / mask / ``player`` are always for the player to move next in each game, in that player's frame;
@@ -27,7 +28,7 @@ import torch
 
 from . import sharding
 from .config import HUMAN_INIT_TABLE, VERSION_CONFIGS, as_version
-from .engine import DeviceState, StrategoEngine, load_setup_table
+from .engine import DeviceState, StrategoEngine, load_setup_table, obs_dtype_code
 from .enums import GameVersions, ObservationComponents, ObservationModes
 from .stratego_multiagent_env import DEFAULT_CONFIG, with_base_config
 
@@ -37,7 +38,9 @@ OC = ObservationComponents
 class BatchedStrategoEnv:
     def __init__(self, env_config=None, num_envs: int = 1024, device=None, seed: int = 0, env_base: int = 0,
                  auto_reset: bool = True, sample_actions: bool = False, raise_on_illegal: bool = False,
-                 terminal_observations: bool = False):
+                 terminal_observations: bool = False, obs_dtype=torch.float32):
+        """obs_dtype: element type of the observations (torch.float32, torch.bfloat16 or torch.float16; StrategoEngine)"""
+        obs_dtype_code(obs_dtype)  # a bad dtype is a ValueError before anything needs a device
         cfg = with_base_config(DEFAULT_CONFIG, env_config if env_config else {})
         cfg['version'] = as_version(cfg['version'])
         self.version = cfg['version']
@@ -68,7 +71,8 @@ class BatchedStrategoEnv:
         self.num_envs, self.seed, self.env_base = int(num_envs), int(seed), int(env_base)
         self.auto_reset, self.sample_actions, self.raise_on_illegal = auto_reset, sample_actions, raise_on_illegal
         self.engine = StrategoEngine({k: cfg[k] for k in version_config}, device=device,
-                                     p2_rot180=not self.human_inits, obs_channel_mode=cfg['obs_channel_mode'])
+                                     p2_rot180=not self.human_inits, obs_channel_mode=cfg['obs_channel_mode'],
+                                     obs_dtype=obs_dtype)
         self.device = self.engine.device
         self.rows, self.columns = self.engine.rows, self.engine.columns
         self.spatial_action_size = self.engine.spatial_action_size

@@ -237,6 +237,11 @@ __device__ __forceinline__ void st_hint(uint32_t *p, uint32_t v, uint64_t pol)
     if (!SX_HINT_ST) { *p = v; return; }
     asm volatile("st.global.L2::cache_hint.b32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
 }
+__device__ __forceinline__ void st_hint(uint16_t *p, uint16_t v, uint64_t pol)
+{
+    if (!SX_HINT_ST) { *p = v; return; }
+    asm volatile("st.global.L2::cache_hint.b16 [%0], %1, %2;" ::"l"(p), "h"(v), "l"(pol) : "memory");
+}
 __device__ __forceinline__ void st_hint(uint4 *p, uint4 v, uint64_t pol)
 {
     if (!SX_HINT_ST) { *p = v; return; }
@@ -291,6 +296,31 @@ static __device__ __noinline__ void emit_tile(uint8_t *gdst, const uint8_t *ssrc
         const int off = head + body + ((lane - 4) << 2);
         *reinterpret_cast<uint32_t *>(gdst + off) = *reinterpret_cast<const uint32_t *>(ssrc + off);
     }
+    if (body > 0 && lane == 0) bulk_store(gdst + head, ssrc + head, uint32_t(body), pol);
+}
+
+// emit_tile for 16-bit observations: src, dst and bytes are even, and the callers pick a source congruent to the
+// destination mod 16 (align_cells16), so the head and tail (at most 7 half-words each; a lane group has >= 8 lanes)
+// go out as one half-word store per lane and the body as one TMA bulk copy.  A destination no image row can match (a
+// caller's buffer that starts inside a 64-byte cell of the 32-channel mode) is copied with half-word stores.
+template <class GT>
+static __device__ __noinline__ void emit_tile16(uint8_t *gdst, const uint8_t *ssrc, int bytes, uint64_t pol)
+{
+    const int lane = GT::lane();
+    const uintptr_t g = reinterpret_cast<uintptr_t>(gdst);
+    const uint32_t s = static_cast<uint32_t>(__cvta_generic_to_shared(ssrc));
+    uint16_t *gd = reinterpret_cast<uint16_t *>(gdst);
+    const uint16_t *sd = reinterpret_cast<const uint16_t *>(ssrc);
+    if (((g ^ s) & 15) != 0) {
+        for (int i = lane; i < (bytes >> 1); i += GT::L) gd[i] = sd[i];
+        return;
+    }
+    int head = int((16 - (g & 15)) & 15);
+    if (head > bytes) head = bytes;
+    const int body = (bytes - head) & ~15;
+    const int tail_at = (head + body) >> 1;
+    if (lane < (head >> 1)) gd[lane] = sd[lane];
+    if (lane < ((bytes - head - body) >> 1)) gd[tail_at + lane] = sd[tail_at + lane];
     if (body > 0 && lane == 0) bulk_store(gdst + head, ssrc + head, uint32_t(body), pol);
 }
 
@@ -902,8 +932,25 @@ __device__ __forceinline__ int align_rows(int channels, int a)
     return c == 3 ? ((4 - a) & 3) : c == 1 ? a : 0;
 }
 
+// The same for 16-bit observations, whose rows start at any even address: a cell is `channels` half-words, so k cells
+// shift the phase by k * channels half-words mod 8, and a destination h half-words past a 16-byte boundary needs
+// k * channels = h (mod 8).  For the odd channel counts (67, 79, 33) k = h * channels mod 8 solves it (an odd c has
+// c * c = 1 mod 8), so up to 7 skipped cells (carve_tile: 7 extra image rows).  32 channels are 64 bytes per cell:
+// no skip changes the phase, and none is needed, since every game row of such a tensor starts 16-byte aligned.
+__host__ __device__ inline int align_cells16(int channels, int h) { return (channels & 1) ? ((h * channels) & 7) : 0; }
+
+// Observation element type T: float (the LUT values as they are) or uint16_t, the bfloat16 / float16 bit pattern that
+// sx_config_create has put into the low half of each LUT word (sx_config_desc::obs_dtype).
+template <class T> __device__ __forceinline__ T obs_value(float lut_word);
+template <> __device__ __forceinline__ float obs_value<float>(float lut_word) { return lut_word; }
+template <> __device__ __forceinline__ uint16_t obs_value<uint16_t>(float lut_word) { return uint16_t(__float_as_uint(lut_word)); }
+
+// extra cells at the end of a background image, for the alignment skip of align_rows / align_cells16
+template <class T> __host__ __device__ constexpr int bg_extra_cells() { return sizeof(T) == 4 ? 3 : 7; }
+
 // fills a tile with what an empty board looks like after normalisation
-static __device__ __noinline__ void fill_background(const DevConfig &cfg, float *tile, const ObsMap om, int first, int stride,
+template <class T = float>
+static __device__ __noinline__ void fill_background(const DevConfig &cfg, T *tile, const ObsMap om, int first, int stride,
                                                     int cells)
 {
     const int total = cells * om.channels;
@@ -918,33 +965,43 @@ static __device__ __noinline__ void fill_background(const DevConfig &cfg, float 
             if (ch == om.own_true || ch == om.enemy_true) v = cfg.rank_lut[0];
             else if (ch == om.own_po || ch == om.enemy_po) v = cfg.po_rank_lut[0];
         }
-        tile[i] = v;
+        tile[i] = obs_value<T>(v);
     }
+}
+
+// One game's background copy of a 16-bit observation of `elems` elements to `g`: the image row that makes the copy's
+// source congruent to g mod 16 is chosen, so the body leaves as one TMA bulk copy.
+template <class GT>
+__device__ __forceinline__ void emit_obs16(uint16_t *g, const uint16_t *bg, int channels, int elems, uint64_t pol)
+{
+    const int k = align_cells16(channels, int((reinterpret_cast<uintptr_t>(g) >> 1) & 7));
+    emit_tile16<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg + k * channels), elems * 2, pol);
 }
 
 // Writes the sparse, state-dependent entries of observer `me`'s observation on top of the background
 // image at `tile` (global memory).
 // ORIG = the deprecated 'original' channel mode: rank planes carry the normalised rank instead of one-hot groups.
-template <int K, class GT, bool ORIG = false>
-__device__ __forceinline__ void patch_obs(const DevConfig &cfg, const WarpMem &m, const Aux &a, float *tile,
+template <int K, class GT, bool ORIG = false, class T = float>
+__device__ __forceinline__ void patch_obs(const DevConfig &cfg, const WarpMem &m, const Aux &a, T *tile,
                                           const ObsMap om, int me, uint64_t pol)
 {
     const int lane = GT::lane(), flip = me, CH = om.channels;
-    const float one = cfg.unit_lut[1];
+    const T one = obs_value<T>(cfg.unit_lut[1]);
 #pragma unroll UNROLL_K
     for (int k = 0; k < K; ++k) {
         const int p = lane * K + k;
         if (p < cfg.N) {
             const uint32_t b = m.board[view(p, flip, cfg.N)];
-            float *cell = tile + p * CH;
+            T *cell = tile + p * CH;
             if (b & CELL_OBST) st_hint(cell + om.obstacle, one, pol);
             const int rank = b & CELL_RANK;
             if (rank) {
                 const int po = (b & CELL_REVEALED) ? rank : SP_UNKNOWN;
                 const bool own = int((b >> 4) & 1) == me;
                 if (ORIG) {  // impl:1178-1195 / impl:1102-1121 + maenv:499-508
-                    if (own || om.enemy_true >= 0) st_hint(cell + (own ? om.own_true : om.enemy_true), cfg.rank_lut[rank], pol);
-                    st_hint(cell + (own ? om.own_po : om.enemy_po), cfg.po_rank_lut[po], pol);
+                    if (own || om.enemy_true >= 0)
+                        st_hint(cell + (own ? om.own_true : om.enemy_true), obs_value<T>(cfg.rank_lut[rank]), pol);
+                    st_hint(cell + (own ? om.own_po : om.enemy_po), obs_value<T>(cfg.po_rank_lut[po]), pol);
                     if (b & CELL_STILL) st_hint(cell + (own ? om.own_still : om.enemy_still), one, pol);
                 } else if (own) {
                     st_hint(cell + om.own_true + rank - 1, one, pol);
@@ -964,13 +1021,13 @@ __device__ __forceinline__ void patch_obs(const DevConfig &cfg, const WarpMem &m
         const int code = (lane & 1) ? -a.rcode[who] : 1;
         if (cell_abs != NO_CELL)
             st_hint(tile + view(cell_abs, flip, cfg.N) * CH + (lane < 2 ? om.own_recent : om.enemy_recent),
-                    cfg.recent_lut[code + 3], pol);
+                    obs_value<T>(cfg.recent_lut[code + 3]), pol);
     }
     for (int e = lane; e < a.ncap; e += GT::L) {
         const uint32_t ent = m.cap[e];
         const int cell_abs = ent & 0xff, owner = (ent >> 8) & 1, type0 = (ent >> 9) & 15, count = int(ent >> 13) + 1;
         st_hint(tile + view(cell_abs, flip, cfg.N) * CH + (owner == me ? om.own_cap : om.enemy_cap) + type0,
-                cfg.cap_lut[type0 * 9 + count], pol);
+                obs_value<T>(cfg.cap_lut[type0 * 9 + count]), pol);
     }
 }
 

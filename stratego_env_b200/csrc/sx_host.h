@@ -18,6 +18,7 @@ struct sx_config {
     sx_layout layout;
     int cells_per_lane;  // K
     int games_per_warp;  // G
+    int obs_elem_bytes = 4;  // 4: float32 observations; 2: bfloat16 / float16 (the LUT words of `dev` hold 16-bit patterns)
     bool compact_movers;  // gen_moves<.., COMPACT>: dense 10x10 boards (sx_device.cuh)
     bool compact_forced = false;  // sx_config_set_tuning chose compact_movers: it then applies to every launch mode
     sx_state start_states{nullptr, nullptr, nullptr};  // sx_config_set_start_states: curriculum table (device)

@@ -6,6 +6,8 @@
 // go to HBM through the TMA engine (cp.async.bulk shared->global, ~30 KB per game for three instructions), the
 // 50-250 state-dependent entries follow as plain stores that merge in L2.  No tensor cores, no CPU fallback.
 // DESIGN.md section 3 has the design, the measurements behind each choice and the dead ends.
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -67,16 +69,20 @@ struct KernelArgs {
 };
 
 // the block's background images: [partial obs][full obs][mask zeros + 16 bytes of alignment slack]
+// EB = bytes per observation element (4, or 2 for the 16-bit observations)
+template <int EB = 4>
 __host__ __device__ inline int carve_tile(const DevConfig &cfg, uint32_t ops, uint8_t *base, Tile *t)
 {
     int off = 0;
     if (t) t->po = reinterpret_cast<float *>(base + off);
     // three extra cell rows: the image is periodic in the cell (67 or 79 floats = 12 mod 16 bytes), so starting the
     // copy k rows in gives a source congruent mod 16 to ANY 4-byte aligned destination (5x5 and 15x15 observations
-    // are not multiples of 16 bytes, so their rows in the output tensor are 4-, 8- or 12-byte misaligned)
-    off += (ops & OP_PO) ? round16((cfg.N + 3) * cfg.po_ch * 4) : 0;
+    // are not multiples of 16 bytes, so their rows in the output tensor are 4-, 8- or 12-byte misaligned); seven for
+    // 16-bit elements, whose rows start at any even address (align_cells16)
+    constexpr int extra = EB == 4 ? 3 : 7;
+    off += (ops & OP_PO) ? round16((cfg.N + extra) * cfg.po_ch * EB) : 0;
     if (t) t->fo = reinterpret_cast<float *>(base + off);
-    off += (ops & OP_FO) ? round16((cfg.N + 3) * cfg.fo_ch * 4) : 0;
+    off += (ops & OP_FO) ? round16((cfg.N + extra) * cfg.fo_ch * EB) : 0;
     if (t) t->mask = base + off;
     off += (ops & OP_MASK) ? round16(cfg.mask_bytes + 16) : 0;
     return off;
@@ -105,8 +111,8 @@ __device__ __noinline__ bool gen_moves_cold(const DevConfig *cfg, uint8_t *warp_
 // Both players' observations of the game staged in the warp slice (its final position) into the terminal side buffers
 // [env][player index 0 / 1][R][C][channels], same "background by TMA + sparse entries" rendering as the regular outputs.
 // Out of line: a game ends once in hundreds of steps.
-template <int K, class GT>
-static __device__ __noinline__ void render_terminal(const KernelArgs *args, const float *bg_po, const float *bg_fo,
+template <int K, class GT, class T = float>
+static __device__ __noinline__ void render_terminal(const KernelArgs *args, const T *bg_po, const T *bg_fo,
                                                     uint8_t *warp_base, uint4 auxw, long long env, bool original)
 {
     const DevConfig &cfg = args->cfg;
@@ -117,29 +123,34 @@ static __device__ __noinline__ void render_terminal(const KernelArgs *args, cons
     aux_unpack(w, a);
     const ObsMap pom = original ? po_map_original() : po_map(), fom = original ? fo_map_original() : fo_map();
     const uint64_t pol = l2_policy(0);
-    float *tpo = args->out.terminal_partial_obs, *tfo = args->out.terminal_full_obs;
+    T *tpo = reinterpret_cast<T *>(args->out.terminal_partial_obs), *tfo = reinterpret_cast<T *>(args->out.terminal_full_obs);
 #pragma unroll 1
     for (int side = 0; side < 2; ++side) {
-        float *gpo = tpo ? tpo + (env * 2 + side) * cfg.po_floats : nullptr;
-        float *gfo = tfo ? tfo + (env * 2 + side) * cfg.fo_floats : nullptr;
-        if (gpo) {
-            const int k = align_rows(pom.channels, int((reinterpret_cast<uintptr_t>(gpo) >> 2) & 3));
-            emit_tile<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<const uint8_t *>(bg_po + k * pom.channels), cfg.po_floats * 4, pol);
-        }
-        if (gfo) {
-            const int k = align_rows(fom.channels, int((reinterpret_cast<uintptr_t>(gfo) >> 2) & 3));
-            emit_tile<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<const uint8_t *>(bg_fo + k * fom.channels), cfg.fo_floats * 4, pol);
+        T *gpo = tpo ? tpo + (env * 2 + side) * cfg.po_floats : nullptr;
+        T *gfo = tfo ? tfo + (env * 2 + side) * cfg.fo_floats : nullptr;
+        if constexpr (sizeof(T) == 2) {
+            if (gpo) emit_obs16<GT>(gpo, bg_po, pom.channels, cfg.po_floats, pol);
+            if (gfo) emit_obs16<GT>(gfo, bg_fo, fom.channels, cfg.fo_floats, pol);
+        } else {
+            if (gpo) {
+                const int k = align_rows(pom.channels, int((reinterpret_cast<uintptr_t>(gpo) >> 2) & 3));
+                emit_tile<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<const uint8_t *>(bg_po + k * pom.channels), cfg.po_floats * 4, pol);
+            }
+            if (gfo) {
+                const int k = align_rows(fom.channels, int((reinterpret_cast<uintptr_t>(gfo) >> 2) & 3));
+                emit_tile<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<const uint8_t *>(bg_fo + k * fom.channels), cfg.fo_floats * 4, pol);
+            }
         }
         if (GT::lane() == 0) bulk_commit();
         GT::sync();  // commit_group and wait_group are kept apart (SX_TUNE_COMMIT_GAP)
         if (GT::lane() == 0) bulk_wait_all();
         GT::sync();
         if (original) {
-            if (gpo) patch_obs<K, GT, true>(cfg, m, a, gpo, pom, side, pol);
-            if (gfo) patch_obs<K, GT, true>(cfg, m, a, gfo, fom, side, pol);
+            if (gpo) patch_obs<K, GT, true, T>(cfg, m, a, gpo, pom, side, pol);
+            if (gfo) patch_obs<K, GT, true, T>(cfg, m, a, gfo, fom, side, pol);
         } else {
-            if (gpo) patch_obs<K, GT>(cfg, m, a, gpo, pom, side, pol);
-            if (gfo) patch_obs<K, GT>(cfg, m, a, gfo, fom, side, pol);
+            if (gpo) patch_obs<K, GT, false, T>(cfg, m, a, gpo, pom, side, pol);
+            if (gfo) patch_obs<K, GT, false, T>(cfg, m, a, gfo, fom, side, pol);
         }
         GT::sync();
     }
@@ -252,7 +263,9 @@ __device__ __forceinline__ int32_t *start_index_slot(const KernelArgs &args, lon
     return (args.start_index != nullptr && i >= 0 && i < args.start_index_len) ? args.start_index + i : nullptr;
 }
 
-template <int K, int MODE, int G, bool CM = false>  // CM: gen_moves hands movers to lanes (dense 10x10 boards)
+// CM: gen_moves hands movers to lanes (dense 10x10 boards).  T: observation element, float or uint16_t (bfloat16 /
+// float16 bit patterns); the 16-bit instantiations exist only for the modes that render observations.
+template <int K, int MODE, int G, bool CM = false, class T = float>
 __global__ void __launch_bounds__(K > 2 ? SX_MAX_THREADS : G == 1 ? SX_K2_THREADS : SX_KG_THREADS, 1)
 sx_fused_kernel(const __grid_constant__ KernelArgs args)
 {
@@ -281,10 +294,11 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
 
     // the block's read-only background images
     Tile bg;
-    carve_tile(cfg, ops, smem, &bg);
+    carve_tile<sizeof(T)>(cfg, ops, smem, &bg);
     if (do_tile) {
-        if (do_po) fill_background(cfg, bg.po, pom, threadIdx.x, blockDim.x, cfg.N + 3);  // + 3 rows: see carve_tile
-        if (do_fo) fill_background(cfg, bg.fo, fom, threadIdx.x, blockDim.x, cfg.N + 3);
+        // + 3 (7) rows: see carve_tile
+        if (do_po) fill_background<T>(cfg, reinterpret_cast<T *>(bg.po), pom, threadIdx.x, blockDim.x, cfg.N + bg_extra_cells<T>());
+        if (do_fo) fill_background<T>(cfg, reinterpret_cast<T *>(bg.fo), fom, threadIdx.x, blockDim.x, cfg.N + bg_extra_cells<T>());
         if (do_mask)
             for (int i = threadIdx.x; i < (mask_tile_bytes >> 4); i += blockDim.x)
                 reinterpret_cast<uint4 *>(bg.mask)[i] = make_uint4(0, 0, 0, 0);
@@ -322,17 +336,22 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
             uint8_t *gmask = args.out.valid_mask + e * cfg.mask_bytes;
             emit_tile<GT>(gmask, bg.mask + (reinterpret_cast<uintptr_t>(gmask) & 15), cfg.mask_bytes, pol_bg);
         }
-        if (do_po) {
-            float *g = args.out.partial_obs + e * cfg.po_floats;
-            const int k = align_rows(pom.channels, int((reinterpret_cast<uintptr_t>(g) >> 2) & 3));
-            emit_tile<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg.po + k * pom.channels),
-                          cfg.po_floats * 4, pol_bg);
-        }
-        if (do_fo) {
-            float *g = args.out.full_obs + e * cfg.fo_floats;
-            const int k = align_rows(fom.channels, int((reinterpret_cast<uintptr_t>(g) >> 2) & 3));
-            emit_tile<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg.fo + k * fom.channels),
-                          cfg.fo_floats * 4, pol_bg);
+        if constexpr (sizeof(T) == 2) {
+            if (do_po) emit_obs16<GT>(reinterpret_cast<T *>(args.out.partial_obs) + e * cfg.po_floats, reinterpret_cast<const T *>(bg.po), pom.channels, cfg.po_floats, pol_bg);
+            if (do_fo) emit_obs16<GT>(reinterpret_cast<T *>(args.out.full_obs) + e * cfg.fo_floats, reinterpret_cast<const T *>(bg.fo), fom.channels, cfg.fo_floats, pol_bg);
+        } else {
+            if (do_po) {
+                float *g = args.out.partial_obs + e * cfg.po_floats;
+                const int k = align_rows(pom.channels, int((reinterpret_cast<uintptr_t>(g) >> 2) & 3));
+                emit_tile<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg.po + k * pom.channels),
+                              cfg.po_floats * 4, pol_bg);
+            }
+            if (do_fo) {
+                float *g = args.out.full_obs + e * cfg.fo_floats;
+                const int k = align_rows(fom.channels, int((reinterpret_cast<uintptr_t>(g) >> 2) & 3));
+                emit_tile<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg.fo + k * fom.channels),
+                              cfg.fo_floats * 4, pol_bg);
+            }
         }
         if (lane == 0) bulk_commit();
     };
@@ -476,7 +495,7 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
             uint32_t w[4];
             aux_pack(a, w);
             GT::sync();
-            render_terminal<K, GT>(&args, bg.po, bg.fo, warp_base, make_uint4(w[0], w[1], w[2], w[3]), env, original);
+            render_terminal<K, GT, T>(&args, reinterpret_cast<const T *>(bg.po), reinterpret_cast<const T *>(bg.fo), warp_base, make_uint4(w[0], w[1], w[2], w[3]), env, original);
         }
         if (done && (flags & SX_AUTO_RESET)) {
             // A drawn setup in which the player to move has no move cannot be played in the reference either (the only
@@ -535,11 +554,11 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
             GT::sync();
             if (SX_EXP(flags, 0x80000u)) continue;  // experiment: wait but skip the sparse stores
             if (original) {
-                if (do_po) patch_obs<K, GT, true>(cfg, m, a, args.out.partial_obs + env * cfg.po_floats, pom, viewer, pol_stream);
-                if (do_fo) patch_obs<K, GT, true>(cfg, m, a, args.out.full_obs + env * cfg.fo_floats, fom, viewer, pol_stream);
+                if (do_po) patch_obs<K, GT, true, T>(cfg, m, a, reinterpret_cast<T *>(args.out.partial_obs) + env * cfg.po_floats, pom, viewer, pol_stream);
+                if (do_fo) patch_obs<K, GT, true, T>(cfg, m, a, reinterpret_cast<T *>(args.out.full_obs) + env * cfg.fo_floats, fom, viewer, pol_stream);
             } else {
-                if (do_po) patch_obs<K, GT>(cfg, m, a, args.out.partial_obs + env * cfg.po_floats, pom, viewer, pol_stream);
-                if (do_fo) patch_obs<K, GT>(cfg, m, a, args.out.full_obs + env * cfg.fo_floats, fom, viewer, pol_stream);
+                if (do_po) patch_obs<K, GT, false, T>(cfg, m, a, reinterpret_cast<T *>(args.out.partial_obs) + env * cfg.po_floats, pom, viewer, pol_stream);
+                if (do_fo) patch_obs<K, GT, false, T>(cfg, m, a, reinterpret_cast<T *>(args.out.full_obs) + env * cfg.fo_floats, fom, viewer, pol_stream);
             }
             if (do_mask) {
                 uint8_t *gmask = args.out.valid_mask + env * cfg.mask_bytes;
@@ -570,7 +589,8 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
 #ifndef SX_TOY_THREADS
 #define SX_TOY_THREADS 384
 #endif
-template <int MODE>
+// T: observation element, float or uint16_t (bfloat16 / float16 bit patterns)
+template <int MODE, class T = float>
 __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_constant__ KernelArgs args)
 {
     using GT = Grp<1>;
@@ -580,6 +600,7 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
     constexpr uint32_t ops = mode_ops(MODE);
     constexpr bool do_mask = (ops & OP_MASK) != 0, do_po = (ops & OP_PO) != 0, do_fo = (ops & OP_FO) != 0;
     constexpr bool do_tile = do_mask || do_po || do_fo;
+    constexpr bool half = sizeof(T) == 2;
     const uint32_t flags = args.flags;
     const bool do_sample = (flags & SX_SAMPLE_NEXT) && args.out.next_action != nullptr;
     const bool allow_osc = flags & SX_ALLOW_OSCILLATION;
@@ -587,10 +608,10 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
     const uint64_t pol = l2_policy(0);
 
     Tile bg;
-    carve_tile(cfg, ops, smem, &bg);
+    carve_tile<sizeof(T)>(cfg, ops, smem, &bg);
     if (do_tile) {
-        if (do_po) fill_background(cfg, bg.po, pom, threadIdx.x, blockDim.x, cfg.N + 3);
-        if (do_fo) fill_background(cfg, bg.fo, fom, threadIdx.x, blockDim.x, cfg.N + 3);
+        if (do_po) fill_background<T>(cfg, reinterpret_cast<T *>(bg.po), pom, threadIdx.x, blockDim.x, cfg.N + bg_extra_cells<T>());
+        if (do_fo) fill_background<T>(cfg, reinterpret_cast<T *>(bg.fo), fom, threadIdx.x, blockDim.x, cfg.N + bg_extra_cells<T>());
     }
     __syncthreads();
 
@@ -599,25 +620,37 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
     const int mask_total = toy::GAMES * cfg.mask_bytes;
     const int mask_img_bytes = do_mask ? round16(mask_total + 16) : 0;
     uint8_t *const tiles = mask_img + mask_img_bytes;
-    const int po_bytes = do_po ? cfg.po_floats * 4 : 0, fo_bytes = do_fo ? cfg.fo_floats * 4 : 0;
-    const int tile_stride = po_bytes + fo_bytes;
+    const int po_bytes = do_po ? cfg.po_floats * int(sizeof(T)) : 0, fo_bytes = do_fo ? cfg.fo_floats * int(sizeof(T)) : 0;
+    // 16-bit rows are 8 mod 16 bytes long on the 12-cell board (toy::tile_slot), so a tile starts at the residue its
+    // games' rows have in the output tensor; float32 rows of these boards are whole multiples of 16 bytes
+    const int po_slot = half ? toy::tile_slot(po_bytes) : po_bytes, fo_slot = half ? toy::tile_slot(fo_bytes) : fo_bytes;
+    const int tile_stride = po_slot + fo_slot;
     // the warp's two observation tiles hold the background image for the whole launch
     // T tiles per warp.  Measured and not kept (profiles/r1l_toy_sweeps.txt, r2g_*, r2x_*, r2y_*): 4 or 8 tiles per warp
     // (Micro 1 198 M / 847 M vs 1 448 M env-steps/s), two or four consecutive games per tile set leaving as ONE larger bulk
     // copy (1 234 M / 914 M), two games rendered per pass by the half-warps (1 360 M).  Every one of them needs more
     // shared memory per warp, and the block's shared memory comes out of the SM's 256 KB L1: this kernel keeps ~100 bytes
     // of per-thread arrays in local memory, so it wants the L1 that 150 KB of shared memory leaves.
-    constexpr int T = SX_TOY_TILES;
-    uint32_t undo_po[T], undo_fo[T];
+    constexpr int NT = SX_TOY_TILES;
+    uint32_t undo_po[NT], undo_fo[NT];
 #pragma unroll
-    for (int h = 0; h < T; ++h) undo_po[h] = undo_fo[h] = lane < 16 ? 0u : toy::UNDO_NONE;  // cell lanes: "channel 0" four times
-    for (int h = 0; h < T; ++h) {
-        if (do_po)
-            for (int i = lane; i < (po_bytes >> 4); i += 32)
-                reinterpret_cast<uint4 *>(tiles + h * tile_stride)[i] = reinterpret_cast<const uint4 *>(bg.po)[i];
-        if (do_fo)
-            for (int i = lane; i < (fo_bytes >> 4); i += 32)
-                reinterpret_cast<uint4 *>(tiles + h * tile_stride + po_bytes)[i] = reinterpret_cast<const uint4 *>(bg.fo)[i];
+    for (int h = 0; h < NT; ++h) undo_po[h] = undo_fo[h] = lane < 16 ? 0u : toy::UNDO_NONE;  // cell lanes: "channel 0" four times
+    for (int h = 0; h < NT; ++h) {
+        if constexpr (half) {  // tiles 8-byte aligned (tile_slot), rows a multiple of 8 bytes (cells a multiple of 4)
+            if (do_po)
+                for (int i = lane; i < (po_bytes >> 3); i += 32)
+                    reinterpret_cast<uint2 *>(tiles + h * tile_stride + ((h * po_bytes) & 15))[i] = reinterpret_cast<const uint2 *>(bg.po)[i];
+            if (do_fo)
+                for (int i = lane; i < (fo_bytes >> 3); i += 32)
+                    reinterpret_cast<uint2 *>(tiles + h * tile_stride + po_slot + ((h * fo_bytes) & 15))[i] = reinterpret_cast<const uint2 *>(bg.fo)[i];
+        } else {
+            if (do_po)
+                for (int i = lane; i < (po_bytes >> 4); i += 32)
+                    reinterpret_cast<uint4 *>(tiles + h * tile_stride)[i] = reinterpret_cast<const uint4 *>(bg.po)[i];
+            if (do_fo)
+                for (int i = lane; i < (fo_bytes >> 4); i += 32)
+                    reinterpret_cast<uint4 *>(tiles + h * tile_stride + po_bytes)[i] = reinterpret_cast<const uint4 *>(bg.fo)[i];
+        }
     }
     __syncwarp();
 
@@ -756,27 +789,42 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
             if (lane == 0) bulk_commit();
         }
         if (do_po || do_fo) {
-            float *gpo = do_po ? args.out.partial_obs + env0 * cfg.po_floats : nullptr;  // walked, not re-multiplied, per game
-            float *gfo = do_fo ? args.out.full_obs + env0 * cfg.fo_floats : nullptr;
+            T *gpo = do_po ? reinterpret_cast<T *>(args.out.partial_obs) + env0 * cfg.po_floats : nullptr;  // walked, not re-multiplied, per game
+            T *gfo = do_fo ? reinterpret_cast<T *>(args.out.full_obs) + env0 * cfg.fo_floats : nullptr;
 #pragma unroll 1
-            for (int g = 0; g < toy::GAMES; g += T) {
+            for (int g = 0; g < toy::GAMES; g += NT) {
 #pragma unroll
-                for (int h = 0; h < T; ++h) {  // T tiles: one is patched while the others' copies are read
+                for (int h = 0; h < NT; ++h) {  // NT tiles: one is patched while the others' copies are read
                     uint8_t *tile = tiles + h * tile_stride;
-                    if (lane == 0) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(T - 1) : "memory");  // the copy T games ago left this tile
+                    if (lane == 0) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(NT - 1) : "memory");  // the copy NT games ago left this tile
                     __syncwarp();
-                    if (do_po) toy::restore_tile(cfg, reinterpret_cast<float *>(tile), pom, lane, undo_po[h]);
-                    if (do_fo) toy::restore_tile(cfg, reinterpret_cast<float *>(tile + po_bytes), fom, lane, undo_fo[h]);
-                    __syncwarp();  // an entry being undone and a new entry of another lane may share an address
-                    const uint8_t *st = stage + (g + h) * toy::STAGE_BYTES;
-                    if (do_po) undo_po[h] = toy::patch_tile(cfg, st, reinterpret_cast<float *>(tile), pom, lane);
-                    if (do_fo) undo_fo[h] = toy::patch_tile(cfg, st, reinterpret_cast<float *>(tile + po_bytes), fom, lane);
-                    fence_async_smem();
-                    __syncwarp();
-                    if (lane == 0) {
-                        if (do_po) bulk_store(gpo, tile, uint32_t(po_bytes), pol);
-                        if (do_fo) bulk_store(gfo, tile + po_bytes, uint32_t(fo_bytes), pol);
-                        bulk_commit();
+                    if constexpr (half) {  // the tile at its row's residue mod 16: aligned body by TMA, head / tail by the lanes
+                        T *tpo = reinterpret_cast<T *>(tile + ((h * po_bytes) & 15)), *tfo = reinterpret_cast<T *>(tile + po_slot + ((h * fo_bytes) & 15));
+                        if (do_po) toy::restore_tile(cfg, tpo, pom, lane, undo_po[h]);
+                        if (do_fo) toy::restore_tile(cfg, tfo, fom, lane, undo_fo[h]);
+                        __syncwarp();
+                        const uint8_t *st = stage + (g + h) * toy::STAGE_BYTES;
+                        if (do_po) undo_po[h] = toy::patch_tile(cfg, st, tpo, pom, lane);
+                        if (do_fo) undo_fo[h] = toy::patch_tile(cfg, st, tfo, fom, lane);
+                        fence_async_smem();
+                        __syncwarp();
+                        if (do_po) emit_tile16<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<uint8_t *>(tpo), po_bytes, pol);
+                        if (do_fo) emit_tile16<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<uint8_t *>(tfo), fo_bytes, pol);
+                        if (lane == 0) bulk_commit();
+                    } else {
+                        if (do_po) toy::restore_tile(cfg, reinterpret_cast<float *>(tile), pom, lane, undo_po[h]);
+                        if (do_fo) toy::restore_tile(cfg, reinterpret_cast<float *>(tile + po_bytes), fom, lane, undo_fo[h]);
+                        __syncwarp();  // an entry being undone and a new entry of another lane may share an address
+                        const uint8_t *st = stage + (g + h) * toy::STAGE_BYTES;
+                        if (do_po) undo_po[h] = toy::patch_tile(cfg, st, reinterpret_cast<float *>(tile), pom, lane);
+                        if (do_fo) undo_fo[h] = toy::patch_tile(cfg, st, reinterpret_cast<float *>(tile + po_bytes), fom, lane);
+                        fence_async_smem();
+                        __syncwarp();
+                        if (lane == 0) {
+                            if (do_po) bulk_store(gpo, tile, uint32_t(po_bytes), pol);
+                            if (do_fo) bulk_store(gfo, tile + po_bytes, uint32_t(fo_bytes), pol);
+                            bulk_commit();
+                        }
                     }
                     if (do_po) gpo += cfg.po_floats;
                     if (do_fo) gfo += cfg.fo_floats;
@@ -1065,6 +1113,27 @@ extern "C" int sx_config_create(const sx_config_desc *desc, sx_config **out)
     std::memcpy(d.cap_lut, desc->captured_lut, sizeof(d.cap_lut));
     std::memcpy(d.recent_lut, desc->recent_lut, sizeof(d.recent_lut));
     std::memcpy(d.unit_lut, desc->unit_lut, sizeof(d.unit_lut));
+    if (desc->obs_dtype != SX_DTYPE_F32 && desc->obs_dtype != SX_DTYPE_BF16 && desc->obs_dtype != SX_DTYPE_F16) {
+        delete c;
+        return fail("sx_config_create: obs_dtype must be SX_DTYPE_F32 (0), SX_DTYPE_BF16 (1) or SX_DTYPE_F16 (2)");
+    }
+    c->obs_elem_bytes = desc->obs_dtype == SX_DTYPE_F32 ? 4 : 2;
+    if (c->obs_elem_bytes == 2) {
+        // 16-bit observations: every LUT word becomes the round-to-nearest-even bit pattern in its low half (obs_value),
+        // so the kernels only store 16-bit words and bfloat16 / float16 share one code path
+        const bool bf16 = desc->obs_dtype == SX_DTYPE_BF16;
+        auto to16 = [bf16](float &v) {
+            uint32_t bits;
+            if (bf16) { const __nv_bfloat16_raw r = __float2bfloat16_rn(v); bits = r.x; }
+            else { const __half_raw r = __float2half_rn(v); bits = r.x; }
+            std::memcpy(&v, &bits, sizeof(v));
+        };
+        for (float &v : d.cap_lut) to16(v);
+        for (float &v : d.recent_lut) to16(v);
+        for (float &v : d.unit_lut) to16(v);
+        for (float &v : d.rank_lut) to16(v);
+        for (float &v : d.po_rank_lut) to16(v);
+    }
     for (int i = 0; i < d.N; ++i) d.obstacles[i] = desc->obstacles[i] ? 1 : 0;
     // games per warp: small boards share a warp (each game needs max(R, C) <= lanes / 2 and N <= 2 * lanes)
     const int side = std::max(d.R, d.C);
@@ -1082,6 +1151,7 @@ extern "C" int sx_config_create(const sx_config_desc *desc, sx_config **out)
     l.action_size = d.action_size; l.board_stride = d.board_stride; l.aux_stride = 8; l.captured_stride = d.cap_stride;
     l.po_floats = d.po_floats; l.fo_floats = d.fo_floats; l.setup_len = d.setup_len; l.pieces_per_side = pieces;
     l.po_channels = d.po_ch; l.fo_channels = d.fo_ch;
+    l.obs_elem_bytes = c->obs_elem_bytes;
     *out = c;
     return 0;
 }
@@ -1131,27 +1201,33 @@ extern "C" int sx_config_layout(const sx_config *cfg, sx_layout *out)
 }
 
 typedef void (*fused_fn)(const KernelArgs);
-template <int K, int G, bool CM = false>
-static fused_fn fused_for_mode(int mode)
+// the modes without observations (lean step, mask only) share the float instantiation whatever the element type
+template <int K, int G, bool CM, class T>
+static fused_fn fused_for_mode_typed(int mode)
 {
     switch (mode) {
-    case MODE_STEP_PO_MASK: return sx_fused_kernel<K, MODE_STEP_PO_MASK, G, CM>;
-    case MODE_STEP_PO_FO_MASK: return sx_fused_kernel<K, MODE_STEP_PO_FO_MASK, G, CM>;
+    case MODE_STEP_PO_MASK: return sx_fused_kernel<K, MODE_STEP_PO_MASK, G, CM, T>;
+    case MODE_STEP_PO_FO_MASK: return sx_fused_kernel<K, MODE_STEP_PO_FO_MASK, G, CM, T>;
     case MODE_STEP_LEAN: return sx_fused_kernel<K, MODE_STEP_LEAN, G, CM>;
     case MODE_MASK: return sx_fused_kernel<K, MODE_MASK, G, CM>;
-    case MODE_OBSERVE_PO_MASK: return sx_fused_kernel<K, MODE_OBSERVE_PO_MASK, G, CM>;
-    default: return sx_fused_kernel<K, MODE_GENERIC, G, CM>;
+    case MODE_OBSERVE_PO_MASK: return sx_fused_kernel<K, MODE_OBSERVE_PO_MASK, G, CM, T>;
+    default: return sx_fused_kernel<K, MODE_GENERIC, G, CM, T>;
     }
+}
+template <int K, int G, bool CM = false>
+static fused_fn fused_for_mode(int mode, int obs_elem_bytes)
+{
+    return obs_elem_bytes == 2 ? fused_for_mode_typed<K, G, CM, uint16_t>(mode) : fused_for_mode_typed<K, G, CM, float>(mode);
 }
 // (cells per lane, games per warp) instantiations: (2,4) boards up to 4x4, (2,2) up to 5x5 (both dimensions must fit
 // in half a group's lanes), (2,1) up to 64 cells, (4,1) 10x10, (8,1) 15x15
 static fused_fn fused_for(const sx_config *cfg, int mode)
 {
-    const int k = cfg->cells_per_lane, g = cfg->games_per_warp;
-    if (g == 4) return fused_for_mode<2, 4>(mode);
-    if (g == 2) return fused_for_mode<2, 2>(mode);
+    const int k = cfg->cells_per_lane, g = cfg->games_per_warp, eb = cfg->obs_elem_bytes;
+    if (g == 4) return fused_for_mode<2, 4>(mode, eb);
+    if (g == 2) return fused_for_mode<2, 2>(mode, eb);
     switch (k) {
-    case 2: return fused_for_mode<2, 1>(mode);
+    case 2: return fused_for_mode<2, 1>(mode, eb);
     case 4: {
         // measured on the shipped library (profiles/r3o_shipped_tuning_sweep.txt): Standard with one observation 169.0 ->
         // 176.0 M env-steps/s with compact movers, with both observations 89.9 -> 88.1 M (6 warps per SM there)
@@ -1159,9 +1235,9 @@ static fused_fn fused_for(const sx_config *cfg, int mode)
         // -> 0.188 ms, profiles/r3p_all_boards.txt)
         const bool compact = cfg->compact_movers &&
                              (cfg->compact_forced || (mode != MODE_STEP_PO_FO_MASK && mode != MODE_OBSERVE_PO_MASK));
-        return compact ? fused_for_mode<4, 1, true>(mode) : fused_for_mode<4, 1>(mode);
+        return compact ? fused_for_mode<4, 1, true>(mode, eb) : fused_for_mode<4, 1>(mode, eb);
     }
-    default: return fused_for_mode<8, 1>(mode);
+    default: return fused_for_mode<8, 1>(mode, eb);
     }
 }
 
@@ -1179,6 +1255,24 @@ static int mode_for(const sx_config *cfg, const KernelArgs &a)
 }
 
 
+
+// Launch shape of the 16-bit observations, per board class: resident warps per SM and where a stepping game's
+// background copy is issued (0 late, 1 after the outcome, 2 top of the game; sx_fused_kernel).  Half the bytes per game
+// move the optimum of the float32 rule ("~230 KB in flight per SM", plan_launch_uncached), so these come from their own
+// sweep (tools/bench_obs_dtype.py --sweep, profiles/r5a_obs_dtype_sweep.txt; B200 at 1 000 W).  16 warps is the most
+// the 128-register kernels keep resident.  Barrage bf16: 10 warps (the float32 rule) 1.226 ms, 12: 1.057, 16: 0.895 ms;
+// Standard 2.523 / 2.213 / 2.056 ms; Standard PO + full 10: 1.917, 12: 1.851, 16: 1.966 ms; 8x8 16 warps 1.414 ms
+// (12: 1.674); issue point 1 is best or within 0.5 % everywhere but on 15x15 (late 1.268, 1: 1.276 ms).
+struct Shape16 {
+    int warps, issue;
+};
+static Shape16 shape16(const DevConfig &d, uint32_t ops)
+{
+    const bool both = (ops & OP_PO) && (ops & OP_FO);
+    if (d.N > 128) return {both ? 10 : 16, 0};  // 15x15 (both observations not swept: the float32 choice)
+    if (d.N >= 100) return {both ? 12 : 16, 1};  // 10x10
+    return {16, 1};                              // 8x8, 6x6, 5x5 and the warp-level path of the toy boards
+}
 
 // Block shape: one block per SM with as many warps as the register file allows (SX_WARPS overrides; a
 // tuning aid); the block's shared memory is the background images plus one small slice per warp.
@@ -1206,10 +1300,15 @@ static int plan_launch(const sx_config *cfg, uint32_t ops, int mode, long long n
     return 0;
 }
 
+static int tile_bytes_for(const sx_config *cfg, uint32_t ops)
+{
+    return cfg->obs_elem_bytes == 2 ? carve_tile<2>(cfg->dev, ops, nullptr, nullptr) : carve_tile<4>(cfg->dev, ops, nullptr, nullptr);
+}
+
 static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan)
 {
     const int warp_bytes = carve_warp(cfg->dev, nullptr, nullptr);
-    const int tile_bytes = carve_tile(cfg->dev, ops, nullptr, nullptr);
+    const int tile_bytes = tile_bytes_for(cfg, ops);
     fused_fn fn = fused_for(cfg, mode);
     int device = 0;
     cudaError_t e = cudaGetDevice(&device);
@@ -1233,8 +1332,9 @@ static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, lo
     // makes 8 warps the optimum of the 10x10 boards; with 128 registers per thread (no spills) the 8x8 board peaks at
     // 12 warps (272 M env-steps/s; 16 warps 256 M) and the 6x6 board at the 16 warps that fit (372 M).
     const int small_board = std::max(8, std::min(32, (232 * 1024 + tile_bytes / 2) / std::max(1, tile_bytes)));
-    const int preferred = tile_bytes <= 8 * 1024 ? 32 : tile_bytes <= 32 * 1024 ? (cfg->dev.N >= 100 ? 8 : small_board)
-                          : tile_bytes <= 64 * 1024 ? 6 : 10;  // 15x15 (74 KB per game): 4 warps 39 M, 6: 55 M, 8: 69 M, 10: 75 M env-steps/s
+    int preferred = tile_bytes <= 8 * 1024 ? 32 : tile_bytes <= 32 * 1024 ? (cfg->dev.N >= 100 ? 8 : small_board)
+                    : tile_bytes <= 64 * 1024 ? 6 : 10;  // 15x15 (74 KB per game): 4 warps 39 M, 6: 55 M, 8: 69 M, 10: 75 M env-steps/s
+    if (cfg->obs_elem_bytes == 2 && (ops & (OP_PO | OP_FO))) preferred = shape16(cfg->dev, ops).warps;
     int warps = std::min(max_warps, std::max(1, env_int("SX_WARPS", std::min(max_warps, cfg->tune_warps > 0 ? cfg->tune_warps : preferred))));
     const int games = cfg->games_per_warp;  // each game of a warp has its own slice
     while (warps > 1 && tile_bytes + warps * games * warp_bytes > max_smem_optin) --warps;
@@ -1282,16 +1382,22 @@ static bool toy_eligible(const sx_config *cfg, const KernelArgs &a, int mode)
 }
 
 typedef void (*toy_fn)(const KernelArgs);
-static toy_fn toy_for_mode(int mode)
+static toy_fn toy_for_mode(int mode, int obs_elem_bytes)
 {
+    if (obs_elem_bytes == 2 && mode != MODE_STEP_LEAN)
+        return mode == MODE_STEP_PO_MASK ? sx_toy_kernel<MODE_STEP_PO_MASK, uint16_t> : sx_toy_kernel<MODE_STEP_PO_FO_MASK, uint16_t>;
     return mode == MODE_STEP_PO_MASK ? sx_toy_kernel<MODE_STEP_PO_MASK>
          : mode == MODE_STEP_PO_FO_MASK ? sx_toy_kernel<MODE_STEP_PO_FO_MASK> : sx_toy_kernel<MODE_STEP_LEAN>;
 }
 
-static int toy_warp_bytes(const DevConfig &d, uint32_t ops)
+// host mirror of the shared-memory slice of one warp of sx_toy_kernel
+static int toy_warp_bytes(const sx_config *cfg, uint32_t ops)
 {
+    const DevConfig &d = cfg->dev;
+    const int eb = cfg->obs_elem_bytes;
     const int mask_img = (ops & OP_MASK) ? round16(toy::GAMES * d.mask_bytes + 16) : 0;
-    const int tile = ((ops & OP_PO) ? d.po_floats * 4 : 0) + ((ops & OP_FO) ? d.fo_floats * 4 : 0);
+    const int po = (ops & OP_PO) ? d.po_floats * eb : 0, fo = (ops & OP_FO) ? d.fo_floats * eb : 0;
+    const int tile = eb == 2 ? toy::tile_slot(po) + toy::tile_slot(fo) : po + fo;
     return toy::GAMES * toy::STAGE_BYTES + mask_img + SX_TOY_TILES * tile;
 }
 
@@ -1305,8 +1411,8 @@ static int plan_toy(const sx_config *cfg, uint32_t ops, ToyPlan *plan)
     if (e != cudaSuccess) return cuda_fail("cudaGetDevice", e);
     cudaDeviceGetAttribute(&plan->num_sms, cudaDevAttrMultiProcessorCount, device);
     cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
-    plan->tile_bytes = carve_tile(cfg->dev, ops, nullptr, nullptr);
-    plan->warp_bytes = toy_warp_bytes(cfg->dev, ops);
+    plan->tile_bytes = tile_bytes_for(cfg, ops);
+    plan->warp_bytes = toy_warp_bytes(cfg, ops);
     // 12 warps per SM (or as many as shared memory holds): Micro 8 warps 1.10 G, 10: 1.35 G, 11: 1.42 G, 12: 1.49 G,
     // 13-16: 1.40-1.43 G env-steps/s; Tiny 8: 1.02 G, 10-13: 1.08 G
     // (Tiny 4x4 peaks at 11 warps: 1 113 M vs 1 072 M at 12, measured twice, profiles/r2o_*, r2t_*.  A warp sync between a
@@ -1324,7 +1430,7 @@ static int launch_toy(const sx_config *cfg, KernelArgs &args, int mode, cudaStre
     const uint32_t ops = mode_ops(mode);
     ToyPlan plan;
     if (int rc = plan_toy(cfg, ops, &plan)) return rc;
-    toy_fn fn = toy_for_mode(mode);
+    toy_fn fn = toy_for_mode(mode, cfg->obs_elem_bytes);
     static std::mutex attr_mutex;
     {
         std::lock_guard<std::mutex> lock(attr_mutex);
@@ -1340,6 +1446,32 @@ static int launch_toy(const sx_config *cfg, KernelArgs &args, int mode, cudaStre
     fn<<<grid, plan.warps * 32, plan.smem, stream>>>(args);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : cuda_fail("sx toy kernel launch", e);
+}
+
+// `elems` observation elements of the configuration's type past p
+static float *obs_at(const sx_config *cfg, float *p, int64_t elems)
+{
+    return p ? reinterpret_cast<float *>(reinterpret_cast<uint8_t *>(p) + elems * cfg->obs_elem_bytes) : nullptr;
+}
+
+// the outputs of the games from `lo` on
+static sx_outputs offset_outputs(const sx_config *cfg, const sx_outputs &o, int64_t lo)
+{
+    const DevConfig &d = cfg->dev;
+    sx_outputs r = o;
+    r.partial_obs = obs_at(cfg, r.partial_obs, lo * d.po_floats);
+    r.full_obs = obs_at(cfg, r.full_obs, lo * d.fo_floats);
+    if (r.valid_mask) r.valid_mask += lo * d.mask_bytes;
+    if (r.reward) r.reward += lo;
+    if (r.done) r.done += lo;
+    if (r.winner) r.winner += lo;
+    if (r.ending_invalid) r.ending_invalid += lo;
+    if (r.illegal) r.illegal += lo;
+    if (r.player) r.player += lo;
+    if (r.next_action) r.next_action += lo;
+    r.terminal_partial_obs = obs_at(cfg, r.terminal_partial_obs, lo * 2 * d.po_floats);
+    r.terminal_full_obs = obs_at(cfg, r.terminal_full_obs, lo * 2 * d.fo_floats);
+    return r;
 }
 
 static int launch_fused(const sx_config *cfg, KernelArgs &args, cudaStream_t stream)
@@ -1363,19 +1495,7 @@ static int launch_fused(const sx_config *cfg, KernelArgs &args, cudaStream_t str
         args.actions += whole;
         args.env_base += whole;
         args.num_envs = rest;
-        sx_outputs &o = args.out;
-        if (o.partial_obs) o.partial_obs += whole * cfg->dev.po_floats;
-        if (o.full_obs) o.full_obs += whole * cfg->dev.fo_floats;
-        if (o.valid_mask) o.valid_mask += whole * cfg->dev.mask_bytes;
-        if (o.reward) o.reward += whole;
-        if (o.done) o.done += whole;
-        if (o.winner) o.winner += whole;
-        if (o.ending_invalid) o.ending_invalid += whole;
-        if (o.illegal) o.illegal += whole;
-        if (o.player) o.player += whole;
-        if (o.next_action) o.next_action += whole;
-        if (o.terminal_partial_obs) o.terminal_partial_obs += whole * 2 * cfg->dev.po_floats;
-        if (o.terminal_full_obs) o.terminal_full_obs += whole * 2 * cfg->dev.fo_floats;
+        args.out = offset_outputs(cfg, args.out, whole);
     }
     if (int rc = plan_launch(cfg, args.ops, mode, args.num_envs, &plan)) return rc;
     args.cfg = cfg->dev;
@@ -1556,11 +1676,15 @@ extern "C" int sx_step_all(const sx_config *cfg, sx_state st, int64_t num_envs, 
     // boards up to 10x10 with one observation issue the copy after the outcome (shipped-library sweeps, profiles/
     // r3o_shipped_tuning_sweep.txt, r3y_small_boards_tuning.txt: 8x8 +2.1 %, 6x6 +3.5 %, 5x5 +3.8 % over a late issue); both
     // observations and the 15x15 board issue late (15x15: 79.8 M late, 76.8 M after the outcome)
-    const int tune = env_int("SX_DEBUG", cfg->tune_issue >= 0 ? cfg->tune_issue << 4 : (n <= 128 && one_obs) ? 16 : 0);
+    const uint32_t ops = step_all_ops(out, flags);
+    const int issue = cfg->tune_issue >= 0 ? cfg->tune_issue
+                    : (cfg->obs_elem_bytes == 2 && (ops & (OP_PO | OP_FO))) ? shape16(cfg->dev, ops).issue
+                    : (n <= 128 && one_obs) ? 1 : 0;
+    const int tune = env_int("SX_DEBUG", issue << 4);
     a.flags = (flags & 0xffffu) | (uint32_t(tune) << 16);
     if ((tune & 0x30) == 0 && !ten_by_ten) a.flags |= SX_TUNE_COMMIT_GAP;  // late issue, not the 10x10 board
     a.out = out;
-    a.ops = step_all_ops(out, flags);
+    a.ops = ops;
     a.setups = setups_d; a.n_setups = n_setups;
     a.key = make_key(seed);
     a.stats = reinterpret_cast<long long *>(stats_d);
@@ -1610,7 +1734,7 @@ extern "C" int sx_step_all_launch_info(const sx_config *cfg, uint32_t obs_mask, 
         ToyPlan tp;
         if (int rc = plan_toy(cfg, ops, &tp)) return rc;
         cudaFuncAttributes attr;
-        cudaError_t e = cudaFuncGetAttributes(&attr, toy_for_mode(mode_for(cfg, probe)));
+        cudaError_t e = cudaFuncGetAttributes(&attr, toy_for_mode(mode_for(cfg, probe), cfg->obs_elem_bytes));
         if (e != cudaSuccess) return cuda_fail("cudaFuncGetAttributes", e);
         out->warps_per_block = tp.warps; out->blocks_per_sm = 1; out->smem_bytes_per_block = tp.smem;
         out->num_sms = tp.num_sms; out->grid_blocks = tp.grid_max; out->regs_per_thread = attr.numRegs;
@@ -1676,8 +1800,9 @@ extern "C" int sx_host_env_create(const sx_config *cfg, int64_t num_envs, int64_
     ok(dev_alloc(&h->st.board, B * d.board_stride));
     ok(dev_alloc(&h->st.aux, B * 8));
     ok(dev_alloc(&h->st.captured, B * d.cap_stride));
-    if (obs_mask & 1) ok(dev_alloc(&h->dev.partial_obs, B * d.po_floats));
-    if (obs_mask & 2) ok(dev_alloc(&h->dev.full_obs, B * d.fo_floats));
+    const size_t eb = size_t(cfg->obs_elem_bytes);
+    if (obs_mask & 1) ok(dev_alloc(reinterpret_cast<uint8_t **>(&h->dev.partial_obs), B * d.po_floats * eb));
+    if (obs_mask & 2) ok(dev_alloc(reinterpret_cast<uint8_t **>(&h->dev.full_obs), B * d.fo_floats * eb));
     if (obs_mask & 4) ok(dev_alloc(&h->dev.valid_mask, B * d.mask_bytes));
     ok(dev_alloc(&h->dev.reward, B)); ok(dev_alloc(&h->dev.done, B)); ok(dev_alloc(&h->dev.winner, B));
     ok(dev_alloc(&h->dev.ending_invalid, B)); ok(dev_alloc(&h->dev.illegal, B)); ok(dev_alloc(&h->dev.player, B));
@@ -1710,24 +1835,6 @@ static sx_state offset_state(const sx_host_env *h, int64_t lo)
     return sx_state{h->st.board + lo * d.board_stride, h->st.aux + lo * 8, h->st.captured + lo * d.cap_stride};
 }
 
-static sx_outputs offset_outputs(const DevConfig &d, const sx_outputs &o, int64_t lo)
-{
-    sx_outputs r = o;
-    if (r.partial_obs) r.partial_obs += lo * d.po_floats;
-    if (r.full_obs) r.full_obs += lo * d.fo_floats;
-    if (r.valid_mask) r.valid_mask += lo * d.mask_bytes;
-    if (r.reward) r.reward += lo;
-    if (r.done) r.done += lo;
-    if (r.winner) r.winner += lo;
-    if (r.ending_invalid) r.ending_invalid += lo;
-    if (r.illegal) r.illegal += lo;
-    if (r.player) r.player += lo;
-    if (r.next_action) r.next_action += lo;
-    if (r.terminal_partial_obs) r.terminal_partial_obs += lo * 2 * d.po_floats;
-    if (r.terminal_full_obs) r.terminal_full_obs += lo * 2 * d.fo_floats;
-    return r;
-}
-
 template <typename T>
 static cudaError_t d2h(T *host, const T *dev, size_t count, cudaStream_t s)
 {
@@ -1738,11 +1845,13 @@ static cudaError_t d2h(T *host, const T *dev, size_t count, cudaStream_t s)
 static int copy_outputs(const sx_host_env *h, const sx_outputs &host, int64_t lo, int64_t n, cudaStream_t s)
 {
     const DevConfig &d = h->cfg->dev;
-    const sx_outputs dv = offset_outputs(d, h->dev, lo), hv = offset_outputs(d, host, lo);
+    const size_t eb = size_t(h->cfg->obs_elem_bytes);
+    const sx_outputs dv = offset_outputs(h->cfg, h->dev, lo), hv = offset_outputs(h->cfg, host, lo);
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-    ok(d2h(hv.partial_obs, dv.partial_obs, size_t(n) * d.po_floats, s));
-    ok(d2h(hv.full_obs, dv.full_obs, size_t(n) * d.fo_floats, s));
+    auto bytes = [](float *p) { return reinterpret_cast<uint8_t *>(p); };
+    ok(d2h(bytes(hv.partial_obs), bytes(dv.partial_obs), size_t(n) * d.po_floats * eb, s));
+    ok(d2h(bytes(hv.full_obs), bytes(dv.full_obs), size_t(n) * d.fo_floats * eb, s));
     ok(d2h(hv.valid_mask, dv.valid_mask, size_t(n) * d.mask_bytes, s));
     ok(d2h(hv.reward, dv.reward, size_t(n), s));
     ok(d2h(hv.done, dv.done, size_t(n), s));
@@ -1781,7 +1890,7 @@ extern "C" int sx_host_env_reset(sx_host_env *h, sx_outputs host_out)
         if (int rc = sx_reset(h->cfg, offset_state(h, lo), hi - lo, h->env_base + lo, nullptr, h->setups_d, h->n_setups, nullptr,
                               h->seed, h->flags & (SX_RESET_RANDOM_SHUFFLE | SX_SAME_SETUP | SX_REPEAT_OTHER_SIDE), s))
             return rc;
-        sx_outputs o = offset_outputs(h->cfg->dev, h->dev, lo);
+        sx_outputs o = offset_outputs(h->cfg, h->dev, lo);
         KernelArgs a;
         base_args(a, offset_state(h, lo), hi - lo, h->env_base + lo);
         a.out = o;
@@ -1808,7 +1917,7 @@ static int host_env_step_impl(sx_host_env *h, const int32_t *actions_host, const
             if (e != cudaSuccess) return cuda_fail("sx_host_env H2D", e);
         }
         if (int rc = sx_step_all(h->cfg, offset_state(h, lo), hi - lo, h->env_base + lo, acts, action_format, step_flags,
-                                 h->setups_d, h->n_setups, h->seed, offset_outputs(h->cfg->dev, h->dev, lo), h->stats_d, s))
+                                 h->setups_d, h->n_setups, h->seed, offset_outputs(h->cfg, h->dev, lo), h->stats_d, s))
             return rc;
         if (host_out)
             if (int rc = copy_outputs(h, *host_out, lo, hi - lo, s)) return rc;

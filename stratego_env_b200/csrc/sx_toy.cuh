@@ -488,27 +488,34 @@ __device__ __forceinline__ void mark_row(const DevConfig &cfg, const MoveSets &m
 // float offset, UNDO_NONE = nothing.
 constexpr uint32_t UNDO_NONE = 0xffffffffu;
 
-__device__ __forceinline__ void restore_tile(const DevConfig &cfg, float *tile, const ObsMap om, int lane, uint32_t undo)
+// Bytes of shared memory a 16-bit observation tile of `bytes` bytes takes: room to start it at the residue mod 16 its
+// game's row has in the output tensor (0 or 8: rows are a multiple of 8 bytes, cells a multiple of 4).
+__host__ __device__ inline int tile_slot(int bytes) { return bytes ? round16(bytes) + 16 : 0; }
+
+// T: observation element, float or uint16_t (obs_value)
+template <class T = float>
+__device__ __forceinline__ void restore_tile(const DevConfig &cfg, T *tile, const ObsMap om, int lane, uint32_t undo)
 {
     if (lane < cfg.N) {  // four unconditional stores: "no entry" is recorded as channel 0, whose background is zero too
-        float *cell = tile + lane * om.channels;
-        const float zero = cfg.unit_lut[0];
+        T *cell = tile + lane * om.channels;
+        const T zero = obs_value<T>(cfg.unit_lut[0]);
 #pragma unroll
         for (int k = 0; k < 4; ++k) cell[(undo >> (8 * k)) & 0xffu] = zero;
     } else if (lane >= 16 && undo != UNDO_NONE) {
-        tile[undo & 0xffffu] = lane < 20 ? cfg.recent_lut[3] : cfg.cap_lut[((undo >> 16) & 15u) * 9];
+        tile[undo & 0xffffu] = obs_value<T>(lane < 20 ? cfg.recent_lut[3] : cfg.cap_lut[((undo >> 16) & 15u) * 9]);
     }
 }
 
-__device__ __forceinline__ uint32_t patch_tile(const DevConfig &cfg, const uint8_t *stage, float *tile, const ObsMap om, int lane)
+template <class T = float>
+__device__ __forceinline__ uint32_t patch_tile(const DevConfig &cfg, const uint8_t *stage, T *tile, const ObsMap om, int lane)
 {
     const uint32_t info0 = *reinterpret_cast<const uint32_t *>(stage + 32), info1 = *reinterpret_cast<const uint32_t *>(stage + 36);
     const int me = (info1 >> 16) & 1, flip = me, CH = om.channels, N = cfg.N;
-    const float one = cfg.unit_lut[1];
+    const T one = obs_value<T>(cfg.unit_lut[1]);
     uint32_t undo = UNDO_NONE;
     if (lane < N) {
         const uint32_t b = stage[view(lane, flip, N)];
-        float *cell = tile + lane * CH;
+        T *cell = tile + lane * CH;
         uint32_t c0 = 0xff, c1 = 0xff, c2 = 0xff, c3 = 0xff;
         if (b & CELL_OBST) c0 = om.obstacle;
         const int rank = b & CELL_RANK;
@@ -534,7 +541,7 @@ __device__ __forceinline__ uint32_t patch_tile(const DevConfig &cfg, const uint8
         const int code = (l & 1) ? -rcode : 1;
         if (cell_abs != NO_CELL) {
             const uint32_t off = uint32_t(view(cell_abs, flip, N) * CH + (l < 2 ? om.own_recent : om.enemy_recent));
-            tile[off] = cfg.recent_lut[code + 3];
+            tile[off] = obs_value<T>(cfg.recent_lut[code + 3]);
             undo = 0x80000000u | off;
         }
     } else if (lane >= 20 && lane < 28) {
@@ -543,7 +550,7 @@ __device__ __forceinline__ uint32_t patch_tile(const DevConfig &cfg, const uint8
             const uint32_t ent = reinterpret_cast<const uint16_t *>(stage + 16)[e];
             const int cell_abs = ent & 0xff, owner = (ent >> 8) & 1, type0 = (ent >> 9) & 15, count = int(ent >> 13) + 1;
             const uint32_t off = uint32_t(view(cell_abs, flip, N) * CH + (owner == me ? om.own_cap : om.enemy_cap) + type0);
-            tile[off] = cfg.cap_lut[type0 * 9 + count];
+            tile[off] = obs_value<T>(cfg.cap_lut[type0 * 9 + count]);
             undo = 0x80000000u | (uint32_t(type0) << 16) | off;
         }
     }

@@ -48,6 +48,18 @@ class DeviceState:
         return DeviceState(self.board[lo:hi], self.aux[lo:hi], self.captured[lo:hi])
 
 
+# observation element types (sx_config_desc::obs_dtype)
+OBS_DTYPES = {torch.float32: _lib.SX_DTYPE_F32, torch.bfloat16: _lib.SX_DTYPE_BF16, torch.float16: _lib.SX_DTYPE_F16}
+
+
+def obs_dtype_code(obs_dtype) -> int:
+    """the sx_config_desc::obs_dtype value of a torch dtype; ValueError for anything but float32 / bfloat16 / float16"""
+    code = OBS_DTYPES.get(obs_dtype) if isinstance(obs_dtype, torch.dtype) else None
+    if code is None:
+        raise ValueError("obs_dtype must be torch.float32, torch.bfloat16 or torch.float16, not %r" % (obs_dtype,))
+    return code
+
+
 def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else t.data_ptr()
 
@@ -58,12 +70,16 @@ def _stream():
 
 class StrategoEngine:
     def __init__(self, game_version_config: dict, device=None, p2_rot180: bool = True, normalize: bool = True,
-                 capture_capacity: int = 0, obs_channel_mode: str = 'extended'):
+                 capture_capacity: int = 0, obs_channel_mode: str = 'extended', obs_dtype=torch.float32):
         """normalize=False: observations carry the raw channel values of the procedural layer (penv:157-173)
         instead of the env-level [-1, 1] normalisation (maenv:499-508).  obs_channel_mode='original' selects the
-        deprecated 32 / 33-channel observations (maenv:370-375, impl:1048-1197)."""
+        deprecated 32 / 33-channel observations (maenv:370-375, impl:1048-1197).  obs_dtype: element type of every
+        observation output, torch.float32, torch.bfloat16 or torch.float16; a 16-bit observation equals the float32 one
+        cast with ``.to(obs_dtype)`` (round to nearest even), at half the bytes written."""
         if obs_channel_mode not in ('extended', 'original'):
             raise ValueError("obs_channel_mode must be 'extended' or 'original'")
+        desc_obs_dtype = obs_dtype_code(obs_dtype)
+        self.obs_dtype = obs_dtype
         self.obs_channel_mode = obs_channel_mode
         original = obs_channel_mode == 'original'
         if not torch.cuda.is_available():
@@ -104,6 +120,7 @@ class StrategoEngine:
         desc.unit_lut = self._unit_lut.ctypes.data
         desc.p2_rot180 = 1 if p2_rot180 else 0
         desc.capture_capacity = int(capture_capacity)
+        desc.obs_dtype = desc_obs_dtype
         handle = C.c_void_p()
         _lib.check(self.lib.sx_config_create(C.byref(desc), C.byref(handle)), "sx_config_create")
         self._cfg = handle
@@ -176,26 +193,29 @@ class StrategoEngine:
             "player": torch.zeros(num_envs, dtype=torch.int8, device=d),
         }
         if partial:
-            out["partial_obs"] = torch.empty((num_envs, R, Cc, self.po_channels), dtype=torch.float32, device=d)
+            out["partial_obs"] = torch.empty((num_envs, R, Cc, self.po_channels), dtype=self.obs_dtype, device=d)
         if full:
-            out["full_obs"] = torch.empty((num_envs, R, Cc, self.fo_channels), dtype=torch.float32, device=d)
+            out["full_obs"] = torch.empty((num_envs, R, Cc, self.fo_channels), dtype=self.obs_dtype, device=d)
         if mask:
             out["valid_mask"] = torch.empty((num_envs, R, Cc, self.spatial_channels), dtype=torch.uint8, device=d)
         if sample:
             out["next_action"] = torch.zeros(num_envs, dtype=torch.int32, device=d)
         if terminal and partial:
-            out["terminal_partial_obs"] = torch.zeros((num_envs, 2, R, Cc, self.po_channels), dtype=torch.float32, device=d)
+            out["terminal_partial_obs"] = torch.zeros((num_envs, 2, R, Cc, self.po_channels), dtype=self.obs_dtype, device=d)
         if terminal and full:
-            out["terminal_full_obs"] = torch.zeros((num_envs, 2, R, Cc, self.fo_channels), dtype=torch.float32, device=d)
+            out["terminal_full_obs"] = torch.zeros((num_envs, 2, R, Cc, self.fo_channels), dtype=self.obs_dtype, device=d)
         return out
 
-    @staticmethod
-    def _outputs_struct(out: dict) -> _lib.SxOutputs:
+    _OBS_OUTPUTS = ("partial_obs", "full_obs", "terminal_partial_obs", "terminal_full_obs")
+
+    def _outputs_struct(self, out: dict) -> _lib.SxOutputs:
         s = _lib.SxOutputs()
         for name, _ in _lib.SxOutputs._fields_:
             t = out.get(name)
             if t is not None:
                 assert t.is_cuda and t.is_contiguous(), name
+                if name in self._OBS_OUTPUTS and t.dtype != self.obs_dtype:
+                    raise ValueError("%s is %s; this engine writes %s observations" % (name, t.dtype, self.obs_dtype))
                 setattr(s, name, t.data_ptr())
         return s
 

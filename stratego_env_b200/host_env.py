@@ -2,8 +2,9 @@
 
 Thin wrapper of the C ABI's ``sx_host_env_*`` object (include/stratego_b200.h): the library owns the device
 state and output buffers and, per step, pipelines H2D(actions) -> fused kernel -> D2H(outputs) in chunks over
-internal streams.  Pass pinned tensors; this path is PCIe-bound (~30.5 KB of outputs per 10x10 game and step)
-and is what ``bench.py`` reports as ``e2e``.
+internal streams.  Pass pinned tensors; this path is PCIe-bound (~30.5 KB of outputs per 10x10 game and step, ~17 KB
+with an engine built with ``obs_dtype=torch.bfloat16``: the observation buffers follow the engine's dtype) and is what
+``bench.py`` reports as ``e2e``.
 """
 import ctypes as C
 from typing import Optional
@@ -43,9 +44,9 @@ class HostBufferEnv:
                      "next_action": pinned((B,), torch.int32)}
         if copy_obs:  # copy_obs=False: observations and mask stay on the device (scalars only cross PCIe)
             if partial:
-                self.host["partial_obs"] = pinned((B, R, Cc, engine.po_channels), torch.float32)
+                self.host["partial_obs"] = pinned((B, R, Cc, engine.po_channels), engine.obs_dtype)
             if full:
-                self.host["full_obs"] = pinned((B, R, Cc, engine.fo_channels), torch.float32)
+                self.host["full_obs"] = pinned((B, R, Cc, engine.fo_channels), engine.obs_dtype)
             if mask:
                 self.host["valid_mask"] = pinned((B, R, Cc, A), torch.uint8)
         self._out = _lib.SxOutputs()
