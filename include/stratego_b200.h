@@ -223,7 +223,8 @@ int sx_sample_valid(const uint8_t *mask_d, int64_t num_envs, int32_t mask_len, i
  * Draws actions_d[b] ~ softmax(logits[b] / temperature) restricted to mask[b] != 0 (Gumbel-max, Philox4x32-10
  * keyed by (seed, env_base + b, step, entry)); invalid entries have probability exactly 0.  logits_d is
  * [num_envs][n_actions] of logits_dtype; logprob_d (optional) receives log p(action).  actions_d[b] = -1 when a
- * mask row has no valid entry. */
+ * mask row has no valid entry.  A valid logit of -inf has probability 0; when every valid logit is -inf the action is
+ * the lowest valid index and the log-probability NaN.  temperature must be > 0 with a finite reciprocal. */
 int sx_sample_logits(const void *logits_d, int32_t logits_dtype, const uint8_t *mask_d, int64_t num_envs,
                      int32_t n_actions, int64_t env_base, uint64_t seed, uint32_t step, float temperature,
                      int32_t *actions_d, float *logprob_d, void *stream);

@@ -38,6 +38,59 @@ __host__ __device__ __forceinline__ float uniform_open01(uint32_t bits)
     return (float(bits >> 9) + 0.5f) * (1.0f / 8388608.0f);
 }
 
+// Gumbel-perturbed score z + G of one valid entry, G = -log(-log(u)) from the entry's Philox word.  The inner log needs
+// relative accuracy: near u = 1, -log(u) is as small as 6e-8 while __logf promises only 3.6e-7 absolute there, and on
+// the B200 it made G wrong by 1e-4 for u > 1 - 2^-10 and by 2.0 at the largest u, exactly the draws in which a low
+// logit wins.  logf is accurate to a few ulp relative (G within 3e-6 for every u, tests/test_sampler_reference_gpu.py);
+// the outer __logf's absolute error of 3.6e-7 is harmless.
+__device__ __forceinline__ float gumbel_score(float z, uint32_t bits)
+{
+    return z - __logf(-logf(uniform_open01(bits)));
+}
+
+// One lane's share of a draw, the same in both samplers: the running argmax of the Gumbel-perturbed scores (a lane
+// visits its entries in ascending index order, so `>` keeps the lowest index on ties) and, when LSE is set, the online
+// log-sum-exp of z over the visited entries.  A z of -inf adds nothing to the sum and is skipped: in a lane that has
+// not seen a finite z yet, exp(z - run_max) would be exp(-inf - -inf) = NaN and poison the whole warp's sum.
+template <bool LSE>
+struct GumbelMaxLane {
+    float best = -INFINITY, best_logit = 0.0f;  // Gumbel-perturbed score of the running argmax and its scaled logit
+    int best_i = -1;
+    float run_max = -INFINITY, run_sum = 0.0f;
+
+    __device__ __forceinline__ void visit(int i, float z, uint64_t gid, uint32_t step, uint2 key)
+    {
+        const uint4 r = philox4x32_10(make_uint4(uint32_t(gid), uint32_t(gid >> 32), RNG_POLICY ^ step, uint32_t(i)), key);
+        const float score = gumbel_score(z, r.x);
+        if (score > best || best_i < 0) { best = score; best_i = i; best_logit = z; }
+        if (LSE) {
+            if (z > run_max) { run_sum = run_sum * __expf(run_max - z) + 1.0f; run_max = z; }
+            else if (z > -INFINITY) run_sum += __expf(z - run_max);
+        }
+    }
+
+    // warp argmax (ties: lowest index, so the result is independent of the lane assignment) and log-sum-exp
+    __device__ __forceinline__ void reduce_warp()
+    {
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            const float ob = __shfl_xor_sync(FULL, best, off), ol = __shfl_xor_sync(FULL, best_logit, off);
+            const int oi = __shfl_xor_sync(FULL, best_i, off);
+            const bool take = oi >= 0 && (best_i < 0 || ob > best || (ob == best && oi < best_i));
+            if (take) { best = ob; best_i = oi; best_logit = ol; }
+            if (LSE) {
+                const float om = __shfl_xor_sync(FULL, run_max, off), os = __shfl_xor_sync(FULL, run_sum, off);
+                const float nm = fmaxf(run_max, om);
+                if (nm > -INFINITY) run_sum = run_sum * __expf(run_max - nm) + os * __expf(om - nm);
+                run_max = nm;
+            }
+        }
+    }
+
+    // log p(best_i); NaN when every valid z is -inf (as torch.log_softmax)
+    __device__ __forceinline__ float logprob() const { return best_logit - (run_max + __logf(run_sum)); }
+};
+
 template <typename T>
 __global__ void __launch_bounds__(256) sx_sample_logits_kernel(const T *logits, const uint8_t *mask, long long num_envs,
                                                                int n_actions, long long env_base, uint2 key, uint32_t step,
@@ -50,19 +103,8 @@ __global__ void __launch_bounds__(256) sx_sample_logits_kernel(const T *logits, 
     const T *lrow = logits + env * n_actions;
     const uint64_t gid = uint64_t(env_base + env);
 
-    float best = -INFINITY, best_logit = 0.0f;  // Gumbel-perturbed score of the running argmax and its scaled logit
-    int best_i = -1;
-    float run_max = -INFINITY, run_sum = 0.0f;  // online log-sum-exp over the valid entries (for the log-prob)
-
-    auto visit = [&](int i) {
-        const float z = load_logit<T>(lrow + i) * inv_temperature;
-        const uint4 r = philox4x32_10(make_uint4(uint32_t(gid), uint32_t(gid >> 32), RNG_POLICY ^ step, uint32_t(i)), key);
-        const float u = uniform_open01(r.x);
-        const float score = z - __logf(-__logf(u));
-        if (score > best || best_i < 0) { best = score; best_i = i; best_logit = z; }
-        if (z > run_max) { run_sum = run_sum * __expf(run_max - z) + 1.0f; run_max = z; }
-        else run_sum += __expf(z - run_max);
-    };
+    GumbelMaxLane<true> g;
+    auto visit = [&](int i) { g.visit(i, load_logit<T>(lrow + i) * inv_temperature, gid, step, key); };
 
     // the mask row starts at env * n_actions: 4-byte aligned for every board (R*C*A is even x even or handled below)
     const int head = int((4 - (reinterpret_cast<uintptr_t>(mrow) & 3)) & 3);
@@ -92,21 +134,10 @@ __global__ void __launch_bounds__(256) sx_sample_logits_kernel(const T *logits, 
     for (int i = head + (words << 2) + lane; i < n_actions; i += 32)
         if (mrow[i]) visit(i);
 
-    // warp argmax (ties: lowest index, so the result is independent of the lane assignment)
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        const float ob = __shfl_xor_sync(FULL, best, off), ol = __shfl_xor_sync(FULL, best_logit, off);
-        const int oi = __shfl_xor_sync(FULL, best_i, off);
-        const bool take = oi >= 0 && (best_i < 0 || ob > best || (ob == best && oi < best_i));
-        if (take) { best = ob; best_i = oi; best_logit = ol; }
-        const float om = __shfl_xor_sync(FULL, run_max, off), os = __shfl_xor_sync(FULL, run_sum, off);
-        const float nm = fmaxf(run_max, om);
-        if (nm > -INFINITY) run_sum = run_sum * __expf(run_max - nm) + os * __expf(om - nm);
-        run_max = nm;
-    }
+    g.reduce_warp();
     if (lane == 0) {
-        actions[env] = best_i;  // -1: the mask had no valid entry
-        if (logprob) logprob[env] = best_i >= 0 ? best_logit - (run_max + __logf(run_sum)) : 0.0f;
+        actions[env] = g.best_i;  // -1: the mask had no valid entry
+        if (logprob) logprob[env] = g.best_i >= 0 ? g.logprob() : 0.0f;
     }
 }
 
@@ -202,8 +233,7 @@ __global__ void __launch_bounds__(256) sx_sample_policy_kernel(const __grid_cons
 
     const T *lrow = logits + env * (long long)(cfg.N * cfg.A);
     const uint64_t gid = uint64_t(env_base + env);
-    float best = -INFINITY, best_logit = 0.0f, run_max = -INFINITY, run_sum = 0.0f;
-    int best_i = -1;
+    GumbelMaxLane<LOGPROB> g;
     for (int t = lane; t < total; t += 32) {  // ascending flat index within a lane, so `>` keeps the lowest index on ties
         int lo = 0, hi = cfg.N;               // last cell p with before[p] <= t: the cell that holds move t
         while (hi - lo > 1) {
@@ -213,33 +243,17 @@ __global__ void __launch_bounds__(256) sx_sample_policy_kernel(const __grid_cons
         const uint2 bits = m.moves[lo];
         const int ch = nth_set_bit64(bits, t - int(before[lo]));
         const int i = lo * cfg.A + ch;
-        const float z = load_logit<T>(lrow + i) * inv_temperature;
-        const uint4 rnd = philox4x32_10(make_uint4(uint32_t(gid), uint32_t(gid >> 32), RNG_POLICY ^ step, uint32_t(i)), key);
-        const float score = z - __logf(-__logf(uniform_open01(rnd.x)));
-        if (score > best || best_i < 0) { best = score; best_i = i; best_logit = z; }
-        if (LOGPROB) {  // online log-sum-exp over the valid entries, only when the log-probability is asked for
-            if (z > run_max) { run_sum = run_sum * __expf(run_max - z) + 1.0f; run_max = z; }
-            else run_sum += __expf(z - run_max);
-        }
+        g.visit(i, load_logit<T>(lrow + i) * inv_temperature, gid, step, key);
     }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        const float ob = __shfl_xor_sync(FULL, best, off), ol = __shfl_xor_sync(FULL, best_logit, off);
-        const int oi = __shfl_xor_sync(FULL, best_i, off);
-        const bool take = oi >= 0 && (best_i < 0 || ob > best || (ob == best && oi < best_i));
-        if (take) { best = ob; best_i = oi; best_logit = ol; }
-        if (LOGPROB) {
-            const float om = __shfl_xor_sync(FULL, run_max, off), os = __shfl_xor_sync(FULL, run_sum, off);
-            const float nm = fmaxf(run_max, om);
-            if (nm > -INFINITY) run_sum = run_sum * __expf(run_max - nm) + os * __expf(om - nm);
-            run_max = nm;
-        }
-    }
+    g.reduce_warp();
     if (lane == 0) {
-        actions[env] = best_i;
-        if (LOGPROB) logprob[env] = best_logit - (run_max + __logf(run_sum));
+        actions[env] = g.best_i;
+        if (LOGPROB) logprob[env] = g.logprob();
     }
 }
+
+// z = logit * (1 / T): a subnormal T makes 1 / T infinite and every 0-valued logit NaN
+static bool valid_temperature(float temperature) { return temperature > 0.0f && 1.0f / temperature < INFINITY; }
 
 }  // namespace sx
 
@@ -249,7 +263,8 @@ extern "C" int sx_sample_logits(const void *logits_d, int32_t logits_dtype, cons
 {
     using namespace sx;
     if (!logits_d || !mask_d || !actions_d) return sx_set_error("sx_sample_logits: null argument");
-    if (!(temperature > 0.0f)) return sx_set_error("sx_sample_logits: temperature must be > 0");
+    if (!valid_temperature(temperature))
+        return sx_set_error("sx_sample_logits: temperature must be > 0 with a finite reciprocal");
     if (n_actions < 1) return sx_set_error("sx_sample_logits: n_actions must be >= 1");
     if (num_envs <= 0) return 0;
     const int wpb = 8;
@@ -306,7 +321,8 @@ extern "C" int sx_sample_policy(const sx_config *cfg, sx_state st, int64_t num_e
                                 float *logprob_d, void *stream)
 {
     if (!cfg || !st.board || !st.aux || !logits_d || !actions_d) return sx_set_error("sx_sample_policy: null argument");
-    if (!(temperature > 0.0f)) return sx_set_error("sx_sample_policy: temperature must be > 0");
+    if (!sx::valid_temperature(temperature))
+        return sx_set_error("sx_sample_policy:temperature must be > 0 with a finite reciprocal");
     if (num_envs <= 0) return 0;
     const uint2 key = make_uint2(uint32_t(seed), uint32_t(seed >> 32));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
