@@ -11,8 +11,9 @@
  *
  * Conventions
  *   - Every `*_d` / sx_state pointer is a DEVICE pointer owned by the caller (torch tensors in the
- *     Python host layer).  The library never allocates or frees caller-visible memory, except for
- *     the sx_host_env convenience object at the bottom, which owns its own device buffers.
+ *     Python host layer).  The library never allocates or frees caller-visible memory, except through
+ *     sx_device_alloc / sx_device_free and in the sx_host_env convenience object at the bottom, which
+ *     owns its own device buffers.
  *   - Every call enqueues work on `stream` (a cudaStream_t passed as void*) and returns without
  *     synchronising.  Return value: 0 = ok, negative = error (sx_last_error() has the text).
  *   - Games are independent: `num_envs` games, game b uses row b of every tensor.
@@ -252,10 +253,29 @@ typedef struct {
     int32_t background_bytes; /* shared-memory background images of a block (DESIGN.md "Rendering") */
     int32_t thread_per_game;  /* 1: the variant steps through sx_toy_kernel (one thread per game, boards of <= 16 cells) */
 } sx_launch_info;
-int sx_step_all_launch_info(const sx_config *cfg, uint32_t obs_mask /*1 po, 2 fo, 4 mask*/, sx_launch_info *out);
+/* obs_mask bit 8: the launch shape used when the observation / mask outputs lie in compressible memory (sx_device_alloc) */
+int sx_step_all_launch_info(const sx_config *cfg, uint32_t obs_mask /*1 po, 2 fo, 4 mask, 8 compressible*/, sx_launch_info *out);
+
+/* ---- device memory ------------------------------------------------------------------------------
+ * sx_device_alloc allocates `bytes` (0 counts as 1) of device memory on CUDA device `device`.  With
+ * SX_ALLOC_COMPRESSIBLE it asks for memory with the generic data compression of the memory system
+ * (cuMemCreate, CU_MEM_ALLOCATION_COMP_GENERIC): lines between L2 and DRAM are compressed, invisibly to kernels,
+ * copy engines and torch, so an almost constant output image costs fewer DRAM bytes to write.  The size is rounded
+ * up to the granularity of such memory (2 MB on B200).  When the device does not support it or the driver does
+ * not grant it, the memory comes from cudaMalloc instead; *granted_flags (optional) tells which: SX_ALLOC_COMPRESSIBLE
+ * or 0.  Any other flag bit is an error.  The contents are uninitialised.
+ * sx_device_free releases such an allocation (NULL is a no-op; any other pointer is an error).  A compressible
+ * allocation is unmapped only after the device has finished its work (cudaDeviceSynchronize), as cudaFree would.
+ * sx_device_alloc_info reports an allocation's requested size and granted flags and, optionally, how many
+ * allocations of the library are live (ptr may be NULL for the count alone). */
+#define SX_ALLOC_COMPRESSIBLE 1u
+int sx_device_alloc(int32_t device, uint64_t bytes, uint32_t flags, void **ptr, uint32_t *granted_flags);
+int sx_device_free(void *ptr);
+int sx_device_alloc_info(const void *ptr, uint64_t *bytes, uint32_t *granted_flags, int64_t *live_allocations);
 
 /* ---- host-buffer convenience object (the e2e path: host actions in, host tensors out) ------------
- * Owns device state + output buffers for num_envs games on the current device and pipelines
+ * Owns device state + output buffers for num_envs games on the current device (the observation and mask buffers
+ * compressible where the device grants it, see sx_device_alloc) and pipelines
  * H2D(actions) -> sx_step_all -> D2H(outputs) in chunks over internal streams. */
 typedef struct sx_host_env sx_host_env;
 int sx_host_env_create(const sx_config *cfg, int64_t num_envs, int64_t env_base, uint32_t obs_mask, uint32_t flags,

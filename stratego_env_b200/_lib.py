@@ -16,6 +16,7 @@ SX_SAME_SETUP, SX_REPEAT_OTHER_SIDE = 32, 64
 OBS_PO, OBS_FO, OBS_MASK = 1, 2, 4
 SX_CHANNELS_EXTENDED, SX_CHANNELS_ORIGINAL = 0, 1
 SX_DTYPE_F32, SX_DTYPE_BF16, SX_DTYPE_F16 = 0, 1, 2
+SX_ALLOC_COMPRESSIBLE = 1
 
 
 class SxConfigDesc(C.Structure):
@@ -69,6 +70,9 @@ SYMBOLS = {
     "sx_sample_policy": (C.c_int, [_vp, SxState, _i64, _i64, _vp, _i32, _u64, _u32, C.c_float, _vp, _vp, _vp]),
     "sx_heuristic_rewards": (C.c_int, [_vp, SxState, _i64, _vp, _i32, _vp, _vp, _vp]),
     "sx_step_all_launch_info": (C.c_int, [_vp, _u32, C.POINTER(SxLaunchInfo)]),
+    "sx_device_alloc": (C.c_int, [_i32, _u64, _u32, C.POINTER(_vp), C.POINTER(_u32)]),
+    "sx_device_free": (C.c_int, [_vp]),
+    "sx_device_alloc_info": (C.c_int, [_vp, C.POINTER(_u64), C.POINTER(_u32), C.POINTER(_i64)]),
     "sx_host_env_create": (C.c_int, [_vp, _i64, _i64, _u32, _u32, _vp, _i32, _u64, _i32, C.POINTER(_vp)]),
     "sx_host_env_destroy": (None, [_vp]),
     "sx_host_env_reset": (C.c_int, [_vp, SxOutputs]),

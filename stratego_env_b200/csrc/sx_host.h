@@ -34,3 +34,5 @@ struct sx_config {
 };
 
 int sx_set_error(const std::string &msg);  // records the text sx_last_error() returns; always returns -1
+// true when p lies inside a live compressible allocation of sx_device_alloc (sx_alloc.cu)
+bool sx_in_compressible_allocation(const void *p);

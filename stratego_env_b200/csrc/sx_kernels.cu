@@ -1276,20 +1276,50 @@ static Shape16 shape16(const DevConfig &d, uint32_t ops)
 
 // Block shape: one block per SM with as many warps as the register file allows (SX_WARPS overrides; a
 // tuning aid); the block's shared memory is the background images plus one small slice per warp.
-static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan);
+static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan,
+                                int compressed_warps);
 
-static int plan_launch(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan)
+// Launch shape of a 10x10 float32 step whose observation / mask planes all lie in compressible memory (sx_device_alloc),
+// 0 for any other launch.  The memory system then writes fewer DRAM bytes, DRAM stops limiting the write stream, and
+// more copies in flight pay off (tools/sweep_tuning.py on compressible outputs, profiles/r4c_compressed_shape_sweep.txt;
+// env-steps/s at the plain shape -> here): one observation + mask 12 warps with the copy issued late, Barrage 188.4 M ->
+// 217.3 M, Standard 179.2 M -> 196.7 M; both observations 7 warps, late, 91.1 M -> 99.1 M.  Every shape gives the same
+// results (tests/test_tuning_gpu.py).
+static int compressed_shape_warps(const sx_config *cfg, uint32_t ops)
+{
+    if (cfg->obs_elem_bytes != 4 || !(ops & OP_STEP) || !(ops & (OP_PO | OP_FO)) || cfg->dev.N < 100 || cfg->dev.N > 128)
+        return 0;
+    return (ops & OP_PO) && (ops & OP_FO) ? 7 : 12;
+}
+
+static bool outputs_compressible(const sx_outputs &out)
+{
+    for (const void *p : {static_cast<const void *>(out.partial_obs), static_cast<const void *>(out.full_obs),
+                          static_cast<const void *>(out.valid_mask)})
+        if (p && !sx_in_compressible_allocation(p)) return false;
+    return true;
+}
+
+static int compressed_warps_for(const sx_config *cfg, const sx_outputs &out, uint32_t ops)
+{
+    const int w = compressed_shape_warps(cfg, ops);
+    return w && outputs_compressible(out) ? w : 0;
+}
+
+static int plan_launch(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan,
+                       int compressed_warps = 0)
 {
     int device = 0;
     cudaError_t e = cudaGetDevice(&device);
     if (e != cudaSuccess) return cuda_fail("cudaGetDevice", e);
-    const uint64_t key = (uint64_t(uint32_t(device)) << 40) | (uint64_t(ops) << 8) | uint64_t(mode);
+    const uint64_t key = (uint64_t(uint32_t(device)) << 40) | (uint64_t(compressed_warps) << 24) | (uint64_t(ops) << 8) |
+                         uint64_t(mode);
     {
         std::lock_guard<std::mutex> lock(cfg->plan_mutex);
         auto it = cfg->plans.find(key);
         if (it == cfg->plans.end()) {
             LaunchPlan full;
-            if (int rc = plan_launch_uncached(cfg, ops, mode, 1LL << 40, &full)) return rc;
+            if (int rc = plan_launch_uncached(cfg, ops, mode, 1LL << 40, &full, compressed_warps)) return rc;
             it = cfg->plans.emplace(key, full).first;
         }
         *plan = it->second;
@@ -1305,7 +1335,8 @@ static int tile_bytes_for(const sx_config *cfg, uint32_t ops)
     return cfg->obs_elem_bytes == 2 ? carve_tile<2>(cfg->dev, ops, nullptr, nullptr) : carve_tile<4>(cfg->dev, ops, nullptr, nullptr);
 }
 
-static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan)
+static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan,
+                                int compressed_warps)
 {
     const int warp_bytes = carve_warp(cfg->dev, nullptr, nullptr);
     const int tile_bytes = tile_bytes_for(cfg, ops);
@@ -1335,6 +1366,7 @@ static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, lo
     int preferred = tile_bytes <= 8 * 1024 ? 32 : tile_bytes <= 32 * 1024 ? (cfg->dev.N >= 100 ? 8 : small_board)
                     : tile_bytes <= 64 * 1024 ? 6 : 10;  // 15x15 (74 KB per game): 4 warps 39 M, 6: 55 M, 8: 69 M, 10: 75 M env-steps/s
     if (cfg->obs_elem_bytes == 2 && (ops & (OP_PO | OP_FO))) preferred = shape16(cfg->dev, ops).warps;
+    if (compressed_warps) preferred = compressed_warps;
     int warps = std::min(max_warps, std::max(1, env_int("SX_WARPS", std::min(max_warps, cfg->tune_warps > 0 ? cfg->tune_warps : preferred))));
     const int games = cfg->games_per_warp;  // each game of a warp has its own slice
     while (warps > 1 && tile_bytes + warps * games * warp_bytes > max_smem_optin) --warps;
@@ -1497,7 +1529,7 @@ static int launch_fused(const sx_config *cfg, KernelArgs &args, cudaStream_t str
         args.num_envs = rest;
         args.out = offset_outputs(cfg, args.out, whole);
     }
-    if (int rc = plan_launch(cfg, args.ops, mode, args.num_envs, &plan)) return rc;
+    if (int rc = plan_launch(cfg, args.ops, mode, args.num_envs, &plan, compressed_warps_for(cfg, args.out, args.ops))) return rc;
     args.cfg = cfg->dev;
     args.warp_bytes = plan.warp_bytes;
     args.tile_bytes = plan.tile_bytes;
@@ -1678,6 +1710,7 @@ extern "C" int sx_step_all(const sx_config *cfg, sx_state st, int64_t num_envs, 
     // observations and the 15x15 board issue late (15x15: 79.8 M late, 76.8 M after the outcome)
     const uint32_t ops = step_all_ops(out, flags);
     const int issue = cfg->tune_issue >= 0 ? cfg->tune_issue
+                    : compressed_warps_for(cfg, out, ops) ? 0
                     : (cfg->obs_elem_bytes == 2 && (ops & (OP_PO | OP_FO))) ? shape16(cfg->dev, ops).issue
                     : (n <= 128 && one_obs) ? 1 : 0;
     const int tune = env_int("SX_DEBUG", issue << 4);
@@ -1742,7 +1775,8 @@ extern "C" int sx_step_all_launch_info(const sx_config *cfg, uint32_t obs_mask, 
         out->thread_per_game = 1;
         return 0;
     }
-    if (int rc = plan_launch(cfg, ops, mode_for(cfg, probe), 1LL << 40, &plan)) return rc;
+    const int cw = (obs_mask & 8) ? compressed_shape_warps(cfg, ops) : 0;
+    if (int rc = plan_launch(cfg, ops, mode_for(cfg, probe), 1LL << 40, &plan, cw)) return rc;
     out->warps_per_block = plan.warps_per_block; out->blocks_per_sm = plan.blocks_per_sm;
     out->smem_bytes_per_block = plan.smem_per_block; out->num_sms = plan.num_sms; out->grid_blocks = plan.grid;
     out->regs_per_thread = plan.regs;
@@ -1766,18 +1800,34 @@ struct sx_host_env {
     std::vector<cudaStream_t> streams;
 };
 
+// every device buffer of the object comes from sx_device_alloc: the observation and mask planes compressible where the
+// device grants it (they are written every step and are almost constant), the rest plain.  Below one 2 MB granule of
+// compressible memory, compression would round up more than it saves (StrategoEngine applies the same bound).
 template <typename T>
-static cudaError_t dev_alloc(T **p, size_t count) { return cudaMalloc(reinterpret_cast<void **>(p), std::max<size_t>(count, 1) * sizeof(T)); }
+static cudaError_t dev_alloc(T **p, size_t count, uint32_t flags = 0)
+{
+    int device = 0;
+    cudaError_t e = cudaGetDevice(&device);
+    if (e != cudaSuccess) return e;
+    void *q = nullptr;
+    if (count * sizeof(T) < (size_t(2) << 20)) flags &= ~uint32_t(SX_ALLOC_COMPRESSIBLE);
+    if (sx_device_alloc(device, count * sizeof(T), flags, &q, nullptr)) return cudaErrorMemoryAllocation;
+    *p = static_cast<T *>(q);
+    return cudaSuccess;
+}
 
 extern "C" void sx_host_env_destroy(sx_host_env *env)
 {
     if (!env) return;
     for (cudaStream_t s : env->streams) cudaStreamDestroy(s);
-    cudaFree(env->st.board); cudaFree(env->st.aux); cudaFree(env->st.captured);
-    cudaFree(env->dev.partial_obs); cudaFree(env->dev.full_obs); cudaFree(env->dev.valid_mask);
-    cudaFree(env->dev.reward); cudaFree(env->dev.done); cudaFree(env->dev.winner); cudaFree(env->dev.ending_invalid);
-    cudaFree(env->dev.illegal); cudaFree(env->dev.player); cudaFree(env->dev.next_action);
-    cudaFree(env->actions_d); cudaFree(env->setups_d); cudaFree(env->stats_d);
+    for (void *p : {static_cast<void *>(env->st.board), static_cast<void *>(env->st.aux), static_cast<void *>(env->st.captured),
+                    static_cast<void *>(env->dev.partial_obs), static_cast<void *>(env->dev.full_obs),
+                    static_cast<void *>(env->dev.valid_mask), static_cast<void *>(env->dev.reward),
+                    static_cast<void *>(env->dev.done), static_cast<void *>(env->dev.winner),
+                    static_cast<void *>(env->dev.ending_invalid), static_cast<void *>(env->dev.illegal),
+                    static_cast<void *>(env->dev.player), static_cast<void *>(env->dev.next_action),
+                    static_cast<void *>(env->actions_d), static_cast<void *>(env->setups_d), static_cast<void *>(env->stats_d)})
+        sx_device_free(p);
     delete env;
 }
 
@@ -1801,9 +1851,9 @@ extern "C" int sx_host_env_create(const sx_config *cfg, int64_t num_envs, int64_
     ok(dev_alloc(&h->st.aux, B * 8));
     ok(dev_alloc(&h->st.captured, B * d.cap_stride));
     const size_t eb = size_t(cfg->obs_elem_bytes);
-    if (obs_mask & 1) ok(dev_alloc(reinterpret_cast<uint8_t **>(&h->dev.partial_obs), B * d.po_floats * eb));
-    if (obs_mask & 2) ok(dev_alloc(reinterpret_cast<uint8_t **>(&h->dev.full_obs), B * d.fo_floats * eb));
-    if (obs_mask & 4) ok(dev_alloc(&h->dev.valid_mask, B * d.mask_bytes));
+    if (obs_mask & 1) ok(dev_alloc(reinterpret_cast<uint8_t **>(&h->dev.partial_obs), B * d.po_floats * eb, SX_ALLOC_COMPRESSIBLE));
+    if (obs_mask & 2) ok(dev_alloc(reinterpret_cast<uint8_t **>(&h->dev.full_obs), B * d.fo_floats * eb, SX_ALLOC_COMPRESSIBLE));
+    if (obs_mask & 4) ok(dev_alloc(&h->dev.valid_mask, B * d.mask_bytes, SX_ALLOC_COMPRESSIBLE));
     ok(dev_alloc(&h->dev.reward, B)); ok(dev_alloc(&h->dev.done, B)); ok(dev_alloc(&h->dev.winner, B));
     ok(dev_alloc(&h->dev.ending_invalid, B)); ok(dev_alloc(&h->dev.illegal, B)); ok(dev_alloc(&h->dev.player, B));
     ok(dev_alloc(&h->dev.next_action, B));

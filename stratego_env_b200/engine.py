@@ -68,16 +68,50 @@ def _stream():
     return torch.cuda.current_stream().cuda_stream
 
 
+class DeviceAllocation:
+    """One device allocation of the library (sx_device_alloc): ``nbytes`` bytes on ``device``, compressible
+    (``compressed``) when asked for and granted.  It exposes itself as a uint8 [nbytes] array through
+    ``__cuda_array_interface__``; tensors made from it with ``torch.as_tensor`` hold a reference to it, so the memory is
+    freed (sx_device_free) once, when the last of them is gone."""
+
+    def __init__(self, device, nbytes: int, compressible: bool = True):
+        lib = _lib.load()
+        ptr, granted = C.c_void_p(), C.c_uint32()
+        device = torch.device(device)
+        index = device.index if device.index is not None else torch.cuda.current_device()
+        _lib.check(lib.sx_device_alloc(index, int(nbytes), _lib.SX_ALLOC_COMPRESSIBLE if compressible else 0,
+                                       C.byref(ptr), C.byref(granted)), "sx_device_alloc")
+        self._lib, self.ptr, self.nbytes = lib, ptr.value, int(nbytes)
+        self.compressed = bool(granted.value & _lib.SX_ALLOC_COMPRESSIBLE)
+        self.__cuda_array_interface__ = {"shape": (self.nbytes,), "typestr": "|u1", "data": (self.ptr, False),
+                                         "strides": None, "version": 3}
+
+    def __del__(self):
+        ptr, self.ptr = getattr(self, "ptr", None), None
+        if ptr:
+            self._lib.sx_device_free(ptr)
+
+
 class StrategoEngine:
     def __init__(self, game_version_config: dict, device=None, p2_rot180: bool = True, normalize: bool = True,
-                 capture_capacity: int = 0, obs_channel_mode: str = 'extended', obs_dtype=torch.float32):
+                 capture_capacity: int = 0, obs_channel_mode: str = 'extended', obs_dtype=torch.float32,
+                 compressible_outputs: Optional[bool] = None):
         """normalize=False: observations carry the raw channel values of the procedural layer (penv:157-173)
         instead of the env-level [-1, 1] normalisation (maenv:499-508).  obs_channel_mode='original' selects the
         deprecated 32 / 33-channel observations (maenv:370-375, impl:1048-1197).  obs_dtype: element type of every
         observation output, torch.float32, torch.bfloat16 or torch.float16; a 16-bit observation equals the float32 one
-        cast with ``.to(obs_dtype)`` (round to nearest even), at half the bytes written."""
+        cast with ``.to(obs_dtype)`` (round to nearest even), at half the bytes written.
+        compressible_outputs: where ``alloc_outputs`` puts the observation and mask planes.  None (default): in one
+        allocation of the library with the device's generic data compression when the device grants it (the planes are
+        an almost constant image, so the DRAM write stream that bounds the fused kernel shrinks; results are the same
+        bytes), plain device memory otherwise; True: the same, but an error when compression is not granted; False:
+        ``torch.empty`` as before.  ``outputs_compressed`` tells what the last ``alloc_outputs`` got."""
         if obs_channel_mode not in ('extended', 'original'):
             raise ValueError("obs_channel_mode must be 'extended' or 'original'")
+        if compressible_outputs is not None and not isinstance(compressible_outputs, bool):
+            raise ValueError("compressible_outputs must be None, True or False, not %r" % (compressible_outputs,))
+        self.compressible_outputs = compressible_outputs
+        self.outputs_compressed = False
         desc_obs_dtype = obs_dtype_code(obs_dtype)
         self.obs_dtype = obs_dtype
         self.obs_channel_mode = obs_channel_mode
@@ -192,19 +226,55 @@ class StrategoEngine:
             "illegal": torch.zeros(num_envs, dtype=torch.uint8, device=d),
             "player": torch.zeros(num_envs, dtype=torch.int8, device=d),
         }
+        planes = []  # (name, shape, dtype, zero-filled)
         if partial:
-            out["partial_obs"] = torch.empty((num_envs, R, Cc, self.po_channels), dtype=self.obs_dtype, device=d)
+            planes.append(("partial_obs", (num_envs, R, Cc, self.po_channels), self.obs_dtype, False))
         if full:
-            out["full_obs"] = torch.empty((num_envs, R, Cc, self.fo_channels), dtype=self.obs_dtype, device=d)
+            planes.append(("full_obs", (num_envs, R, Cc, self.fo_channels), self.obs_dtype, False))
         if mask:
-            out["valid_mask"] = torch.empty((num_envs, R, Cc, self.spatial_channels), dtype=torch.uint8, device=d)
+            planes.append(("valid_mask", (num_envs, R, Cc, self.spatial_channels), torch.uint8, False))
+        if terminal and partial:
+            planes.append(("terminal_partial_obs", (num_envs, 2, R, Cc, self.po_channels), self.obs_dtype, True))
+        if terminal and full:
+            planes.append(("terminal_full_obs", (num_envs, 2, R, Cc, self.fo_channels), self.obs_dtype, True))
+        out.update(self._alloc_planes(planes))
         if sample:
             out["next_action"] = torch.zeros(num_envs, dtype=torch.int32, device=d)
-        if terminal and partial:
-            out["terminal_partial_obs"] = torch.zeros((num_envs, 2, R, Cc, self.po_channels), dtype=self.obs_dtype, device=d)
-        if terminal and full:
-            out["terminal_full_obs"] = torch.zeros((num_envs, 2, R, Cc, self.fo_channels), dtype=self.obs_dtype, device=d)
         return out
+
+    # Below one granule of compressible memory (2 MB on B200) compression rounds up more than it can save, and the
+    # allocation and its synchronising free would dominate the small per-call buffers of the one-game API.
+    _COMPRESSIBLE_MIN_BYTES = 2 << 20
+
+    def _alloc_planes(self, planes) -> dict:
+        """the observation / mask planes: torch tensors, or views of ONE library allocation (compressible where the
+        device grants it) that the views keep alive"""
+        size = lambda shape, dtype: int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()  # noqa: E731
+        pad = lambda n: (n + 255) // 256 * 256  # noqa: E731
+        total = sum(pad(size(shape, dtype)) for _, shape, dtype, _ in planes)
+        if self.compressible_outputs is False or total < self._COMPRESSIBLE_MIN_BYTES:
+            if planes:
+                self.outputs_compressed = False
+            return {name: (torch.zeros if zero else torch.empty)(shape, dtype=dtype, device=self.device)
+                    for name, shape, dtype, zero in planes}
+        alloc = DeviceAllocation(self.device, total, compressible=self._alloc_compressible)
+        if self.compressible_outputs and not alloc.compressed:
+            raise _lib.StrategoB200Error("compressible_outputs=True: device %s did not grant compressible memory"
+                                         % self.device)
+        self.outputs_compressed = alloc.compressed
+        with torch.cuda.device(self.device):
+            buf = torch.as_tensor(alloc, device=self.device)
+        out, off = {}, 0
+        for name, shape, dtype, zero in planes:
+            n = size(shape, dtype)
+            out[name] = buf[off:off + n].view(dtype).view(shape)
+            if zero:
+                out[name].zero_()
+            off += pad(n)
+        return out
+
+    # False: the library's plain-memory path, the one a device without compression takes (the tests force it so)
+    _alloc_compressible = True
 
     _OBS_OUTPUTS = ("partial_obs", "full_obs", "terminal_partial_obs", "terminal_full_obs")
 
@@ -403,8 +473,9 @@ class StrategoEngine:
         return rewards
 
     def launch_info(self, partial=True, full=False, mask=True) -> dict:
+        """launch shape of sx_step_all for these outputs, in compressible memory when the last ``alloc_outputs`` got it"""
         info = _lib.SxLaunchInfo()
-        obs = (1 if partial else 0) | (2 if full else 0) | (4 if mask else 0)
+        obs = (1 if partial else 0) | (2 if full else 0) | (4 if mask else 0) | (8 if self.outputs_compressed else 0)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.sx_step_all_launch_info(self._cfg, obs, C.byref(info)), "sx_step_all_launch_info")
         return {n: getattr(info, n) for n, _ in _lib.SxLaunchInfo._fields_}
