@@ -247,6 +247,35 @@ int sx_sample_policy(const sx_config *cfg, sx_state st, int64_t num_envs, int64_
 int sx_heuristic_rewards(const sx_config *cfg, sx_state st, int64_t num_envs, const int32_t *actions_d,
                          int32_t action_format, const float *reward_matrix_d, float *rewards_d, void *stream);
 
+/* Determinization: n_samples complete game states per game that agree with what one player knows (for PIMC,
+ * information-set MCTS, determinized rollouts, belief-model training).
+ * The viewer of game b is viewer_d[b] (1 = player +1, anything else = player -1, as player_override of the step) or,
+ * with viewer_d NULL, the player to move.  The HIDDEN cells of a game are the cells that hold a piece of the viewer's
+ * opponent that is not CELL_REVEALED, on no obstacle; their HIDDEN MULTISET is the multiset of the true codes there (on
+ * a reachable state: piece_amounts - captured - revealed alive, for the opponent: what the viewer can infer).
+ * IMMOVABLE codes are FLAG (11) and BOMB (12).  S = hidden cells with CELL_STILL (never moved), I = immovable and
+ * M = movable pieces of the hidden multiset.  A sample is a copy of the game in which the hidden multiset is placed on
+ * the hidden cells uniformly at random among all placements that put no immovable piece on a cell without CELL_STILL.
+ * Everything else stays byte for byte: aux, the capture list, every other cell byte, and the owner / revealed / still /
+ * obstacle bits of the hidden cells; only their CELL_RANK nibble may differ.  A game without hidden cells is copied
+ * unchanged; finished games are sampled like any other.  If I > S no placement exists (play never produces such a
+ * state; sx_import_ref_state of a state in which a bomb or flag has moved can): the rows are copied unchanged and
+ * status_d[b] = 1 (optional output; 0 otherwise).
+ * Draws (exact, so a host reference can reproduce them): each hidden cell c (absolute index, < 256) of sample k of game
+ * b gets one Philox4x32-10 block, key (seed lo, seed hi), counter (gid lo, gid hi, RNG_HIDDEN ^ draw, (k << 8) | c)
+ * with gid = env_base + b and RNG_HIDDEN = 0x48494444; its words x and y are sort keys.  1. The still hidden cells are
+ * ordered by (x, c) ascending; rank j < I receives the j-th immovable code in ascending order (flags before bombs).
+ * 2. Every hidden cell not filled in step 1 is ordered by (y, c) ascending; rank j receives the j-th movable code in
+ * ascending order.  Ranking by i.i.d. keys is a uniform permutation, so every consistent placement comes from exactly
+ * one equally likely pair of (immovable, movable) placements; breaking key ties by the cell index biases this by less
+ * than n^2 / 2^33 for n hidden cells.  Sample k of a game depends on (seed, draw, gid, k) only, not on n_samples, the
+ * batch split or where env_base puts the game.
+ * out has num_envs * n_samples rows (same strides as st); row b * n_samples + k is sample k of game b.  Refused:
+ * n_samples < 1 or >= 2^24, a row count that overflows, out.board == st.board. */
+int sx_sample_hidden_states(const sx_config *cfg, sx_state st, int64_t num_envs, int64_t env_base,
+                            const int8_t *viewer_d, int32_t n_samples, uint64_t seed, uint32_t draw,
+                            sx_state out, uint8_t *status_d, void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

@@ -233,6 +233,17 @@ class BatchedStrategoEnv:
             d[OC.FULL_OBSERVATION.value] = o["full_obs"]
         return d
 
+    def sample_hidden_states(self, n_samples: int = 1, viewer: Optional[torch.Tensor] = None) -> DeviceState:
+        """Determinized copies of the current games (StrategoEngine.sample_hidden_states): ``n_samples`` states per game
+        in which the pieces the viewer has not seen are re-placed uniformly at random, consistently with what the viewer
+        knows.  viewer: None (the player to move) or an integer tensor [num_envs] of INTERNAL player ids (+1 / -1), the
+        ids ``observe`` takes -- not the agent ids of ``random_player_assignment`` or curriculum starts.  Uses the env's
+        seed and env_base and a draw counter that advances per call, so repeated calls give fresh samples.  Returns a
+        DeviceState of num_envs * n_samples rows (row b * n_samples + k = sample k of game b) for ``self.engine``."""
+        self._hidden_draw = getattr(self, "_hidden_draw", 0) + 1
+        return self.engine.sample_hidden_states(self.state, n_samples=n_samples, viewer=viewer, seed=self.seed,
+                                                draw=self._hidden_draw, env_base=self.env_base)
+
     # ---- checkpoint / interop in the reference's dense layout ---------------------------------------------
     def export_states(self):
         """(int64 [B, 34, R, C], int8 [B] player to move) -- the reference's state layout (impl:16-60)"""

@@ -331,6 +331,42 @@ class StrategoEngine:
                              % bad)
         return state
 
+    # torch integer dtypes a viewer tensor may have (bool is not one)
+    _VIEWER_DTYPES = (torch.int8, torch.int16, torch.int32, torch.int64, torch.uint8)
+
+    def sample_hidden_states(self, state: DeviceState, n_samples: int = 1, viewer: Optional[torch.Tensor] = None,
+                             seed: int = 0, draw: int = 0, env_base: int = 0, check: bool = True) -> DeviceState:
+        """Determinization (sx_sample_hidden_states): ``n_samples`` complete game states per game that agree with what
+        the viewer knows.  The opponent's unrevealed pieces are re-placed uniformly at random among the placements that
+        keep the multiset of their codes and put no flag or bomb on a piece that has moved; everything else is copied.
+        viewer: None (the player to move) or an integer tensor [B], 1 = player +1, anything else = player -1.
+        Returns a new DeviceState of B * n_samples rows in this engine's strides, row b * n_samples + k = sample k of
+        game b, ready for observe / step / step_all / export_ref_state.  Sample k of a game depends only on (seed, draw,
+        env_base + b, k).  check=True: a game in which more flags and bombs are hidden than unmoved hidden pieces exist
+        (no placement; only an imported state can be so) raises ValueError naming the games; with check=False its rows
+        are plain copies."""
+        if isinstance(n_samples, bool) or not isinstance(n_samples, (int, np.integer)) or not 1 <= n_samples < 1 << 24:
+            raise ValueError("n_samples must be an integer in [1, 2^24), not %r" % (n_samples,))
+        B = state.num_envs
+        if viewer is not None:
+            if not isinstance(viewer, torch.Tensor) or viewer.dtype not in self._VIEWER_DTYPES or tuple(viewer.shape) != (B,):
+                raise ValueError("viewer must be None or an integer tensor of shape (%d,), not %s" % (
+                    B, "%s %s" % (viewer.dtype, tuple(viewer.shape)) if isinstance(viewer, torch.Tensor) else type(viewer).__name__))
+            viewer = viewer.to(self.device, dtype=torch.int8).contiguous()
+        n_samples = int(n_samples)
+        out = self.alloc_state(B * n_samples)
+        status = torch.zeros(B, dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sx_sample_hidden_states(self._cfg, state.as_struct(), B, int(env_base), _ptr(viewer),
+                                                        n_samples, seed & (2 ** 64 - 1), int(draw) & 0xffffffff,
+                                                        out.as_struct(), status.data_ptr(), _stream()),
+                       "sx_sample_hidden_states")
+        if check and bool(status.any().item()):
+            bad = torch.nonzero(status).flatten().tolist()[:8]
+            raise ValueError("game(s) %s hide more flags and bombs than unmoved pieces: no consistent placement exists "
+                             "(not reachable by play)" % bad)
+        return out
+
     def export_ref_state(self, state: DeviceState):
         B = state.num_envs
         dense = torch.empty((B, NUM_STATE_LAYERS, self.rows, self.columns), dtype=torch.int64, device=self.device)
