@@ -276,6 +276,25 @@ int sx_sample_hidden_states(const sx_config *cfg, sx_state st, int64_t num_envs,
                             const int8_t *viewer_d, int32_t n_samples, uint64_t seed, uint32_t draw,
                             sx_state out, uint8_t *status_d, void *stream);
 
+/* The children of a node, for search (PIMC, information-set MCTS, tree expansion).  The CHILDREN of game b are one per
+ * legal move of its player to move: exactly the non-zero entries of sx_valid_mask(b) in the spatial format without the
+ * noop channel A-1, each identified by its flat spatial index in that player's frame (what sx_step_all,
+ * sx_sample_policy and a policy head use), in ascending index order.  A game with no legal move (a finished game, or an
+ * imported state whose player to move is stuck) has zero children.  Nothing is random.
+ * sx_count_moves: counts_d[b] (int32) = the number of children of game b.
+ * sx_expand_moves: offsets_d is int64 [num_envs + 1], normally the exclusive prefix sum of the counts; child t of game b
+ * is row offsets_d[b] + t of out (same strides as st), actions_d (int32) and the scalars of out_scalars.  The row holds,
+ * byte for byte, what sx_step (SX_ACTION_SPATIAL, flags 0) makes of a copy of game b with action actions_d[row]: board
+ * (padding included), aux, capture list, and reward, done, winner, ending_invalid, illegal (0, or 2 when the capture
+ * list overflows) and player (any of them may be NULL).  st is never written.  offsets_d is not checked on the host: no
+ * row outside [0, n_children) is written, a slot [offsets_d[b], offsets_d[b+1]) shorter than the count receives the
+ * game's first children in order, and rows of a slot beyond the count are left untouched.  Refused: a null config,
+ * state, out, actions_d or offsets_d, out.board == st.board, n_children < 0, and a non-null observation, mask,
+ * next_action or terminal pointer in out_scalars.  num_envs <= 0 or n_children == 0: nothing to do. */
+int sx_count_moves(const sx_config *cfg, sx_state st, int64_t num_envs, int32_t *counts_d, void *stream);
+int sx_expand_moves(const sx_config *cfg, sx_state st, int64_t num_envs, const int64_t *offsets_d, int64_t n_children,
+                    sx_state out, int32_t *actions_d, sx_outputs out_scalars, void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

@@ -28,7 +28,7 @@ import torch
 
 from . import sharding
 from .config import HUMAN_INIT_TABLE, VERSION_CONFIGS, as_version
-from .engine import DeviceState, StrategoEngine, load_setup_table, obs_dtype_code
+from .engine import DeviceState, Expansion, StrategoEngine, load_setup_table, obs_dtype_code
 from .enums import GameVersions, ObservationComponents, ObservationModes
 from .stratego_multiagent_env import DEFAULT_CONFIG, with_base_config
 
@@ -243,6 +243,12 @@ class BatchedStrategoEnv:
         self._hidden_draw = getattr(self, "_hidden_draw", 0) + 1
         return self.engine.sample_hidden_states(self.state, n_samples=n_samples, viewer=viewer, seed=self.seed,
                                                 draw=self._hidden_draw, env_base=self.env_base)
+
+    def expand_moves(self) -> Expansion:
+        """The children of the current games (StrategoEngine.expand_moves): one per legal move of the player to move, in
+        ascending flat spatial index, each with the state and step outputs that move leads to.  Player ids in the result
+        (``player``) are INTERNAL (+1 / -1), as for ``sample_hidden_states``.  One host synchronisation per call."""
+        return self.engine.expand_moves(self.state)
 
     # ---- checkpoint / interop in the reference's dense layout ---------------------------------------------
     def export_states(self):

@@ -1031,6 +1031,22 @@ __device__ __forceinline__ void patch_obs(const DevConfig &cfg, const WarpMem &m
     }
 }
 
+// position of the n-th (0-based) set bit of a 64-bit set that has more than n bits: six popcount-guided halvings
+// (one __fns per 32-bit half costs about twice as many instructions)
+__device__ __forceinline__ int nth_set_bit64(uint2 bits, int n)
+{
+    int pos = 0;
+    uint32_t x = bits.x;
+    const int c0 = __popc(bits.x);
+    if (n >= c0) { n -= c0; x = bits.y; pos = 32; }
+#pragma unroll
+    for (int w = 16; w >= 1; w >>= 1) {
+        const int c = __popc(x & ((1u << w) - 1u));
+        if (n >= c) { n -= c; x >>= w; pos += w; }
+    }
+    return pos;
+}
+
 // ---- uniform draw over the generated moves (replaces maenv:830-834) ----------------------------------
 // Order = ascending flat spatial index (cell, then channel).
 template <int K, class GT>

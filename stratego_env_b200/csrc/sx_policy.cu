@@ -147,21 +147,6 @@ __global__ void __launch_bounds__(256) sx_sample_logits_kernel(const T *logits, 
 // with the engine's own move generator (gen_moves: occupancy bit-lines), spreads the valid entries evenly over the lanes
 // and runs the identical Gumbel-max / log-sum-exp per entry.  Same Philox key per (game, step, entry)
 // and the same tie rule as the mask kernel, so both return the SAME action for the same key.
-// position of the n-th (0-based) set bit of a 64-bit set that has more than n bits: six popcount-guided halvings
-// (one __fns per 32-bit half costs about twice as many instructions)
-__device__ __forceinline__ int nth_set_bit64(uint2 bits, int n)
-{
-    int pos = 0;
-    uint32_t x = bits.x;
-    const int c0 = __popc(bits.x);
-    if (n >= c0) { n -= c0; x = bits.y; pos = 32; }
-#pragma unroll
-    for (int w = 16; w >= 1; w >>= 1) {
-        const int c = __popc(x & ((1u << w) - 1u));
-        if (n >= c) { n -= c; x >>= w; pos += w; }
-    }
-    return pos;
-}
 
 template <typename T, int K, bool LOGPROB, bool CM = false>
 __global__ void __launch_bounds__(256) sx_sample_policy_kernel(const __grid_constant__ DevConfig cfg, const uint8_t *board,

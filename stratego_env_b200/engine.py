@@ -48,6 +48,22 @@ class DeviceState:
         return DeviceState(self.board[lo:hi], self.aux[lo:hi], self.captured[lo:hi])
 
 
+@dataclass
+class Expansion:
+    """The children of a batch of games (StrategoEngine.expand_moves), T rows in all; game b's children are rows
+    offsets[b] .. offsets[b + 1] - 1 of every field."""
+    states: DeviceState           # T children, in the engine's strides
+    actions: torch.Tensor         # int32 [T] flat spatial index of the move, in the parent's player-to-move frame
+    parent: torch.Tensor          # int64 [T] game each child comes from
+    offsets: torch.Tensor         # int64 [B + 1] exclusive prefix sum of the number of children per game
+    reward: torch.Tensor          # float32 [T] as step returns them for that move
+    done: torch.Tensor            # uint8 [T]
+    winner: torch.Tensor          # int8 [T]
+    ending_invalid: torch.Tensor  # uint8 [T]
+    illegal: torch.Tensor         # uint8 [T] 0, or 2 when the capture list overflowed
+    player: torch.Tensor          # int8 [T] player to move in the child (+1 / -1)
+
+
 # observation element types (sx_config_desc::obs_dtype)
 OBS_DTYPES = {torch.float32: _lib.SX_DTYPE_F32, torch.bfloat16: _lib.SX_DTYPE_BF16, torch.float16: _lib.SX_DTYPE_F16}
 
@@ -366,6 +382,42 @@ class StrategoEngine:
             raise ValueError("game(s) %s hide more flags and bombs than unmoved pieces: no consistent placement exists "
                              "(not reachable by play)" % bad)
         return out
+
+    def expand_moves(self, state: DeviceState) -> "Expansion":
+        """The children of every game (sx_count_moves + sx_expand_moves): one per legal move of the player to move, in
+        ascending flat spatial index (that player's frame, the index step / step_all / sample_policy take).  Child j of
+        game b is row offsets[b] + j of every field and equals, byte for byte, what ``step`` (spatial actions, no flags)
+        makes of a copy of game b with action actions[row]: state rows and the reward, done, winner, ending_invalid,
+        illegal and player it returns.  A finished game or a stuck player has no children.  ``state`` is not written.
+        Reading the number of children back to size the outputs is ONE host synchronisation per call."""
+        lay = self.layout
+        if not isinstance(state, DeviceState):
+            raise ValueError("state must be a DeviceState, not %s" % type(state).__name__)
+        B = state.num_envs
+        for name, t, dtype, width in (("board", state.board, torch.uint8, lay.board_stride),
+                                      ("aux", state.aux, torch.int16, lay.aux_stride),
+                                      ("captured", state.captured, torch.int16, lay.captured_stride)):
+            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != (B, width)
+                    or not t.is_contiguous() or t.device != self.device):
+                raise ValueError("state.%s must be a contiguous %s tensor of shape (%d, %d) on %s, not %s" % (
+                    name, dtype, B, width, self.device,
+                    "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor) else type(t).__name__))
+        d = self.device
+        counts = torch.empty(B, dtype=torch.int32, device=d)
+        offsets = torch.zeros(B + 1, dtype=torch.int64, device=d)
+        with torch.cuda.device(d):
+            _lib.check(self.lib.sx_count_moves(self._cfg, state.as_struct(), B, counts.data_ptr(), _stream()),
+                       "sx_count_moves")
+            torch.cumsum(counts, 0, dtype=torch.int64, out=offsets[1:])
+            T = int(offsets[-1].item())  # the host synchronisation
+            out = self.alloc_state(T)
+            scalars = self.alloc_outputs(T, partial=False, full=False, mask=False)
+            actions = torch.empty(T, dtype=torch.int32, device=d)
+            _lib.check(self.lib.sx_expand_moves(self._cfg, state.as_struct(), B, offsets.data_ptr(), T, out.as_struct(),
+                                                actions.data_ptr(), self._outputs_struct(scalars), _stream()),
+                       "sx_expand_moves")
+            parent = torch.repeat_interleave(torch.arange(B, device=d), counts, output_size=T)
+        return Expansion(states=out, actions=actions, parent=parent, offsets=offsets, **scalars)
 
     def export_ref_state(self, state: DeviceState):
         B = state.num_envs
