@@ -148,7 +148,7 @@ int sx_config_create(const sx_config_desc *desc, sx_config **out);
 void sx_config_destroy(sx_config *cfg);
 int sx_config_layout(const sx_config *cfg, sx_layout *out);
 
-/* Launch tuning of the warp-level kernel; a development aid (tools/sweep_fused.py times the shipped library with it).
+/* Launch tuning of the warp-level kernel; a development aid (tools/sweep_tuning.py times the library with it).
  * Every setting gives bit-identical results -- only the speed changes.  -1 keeps the built-in choice.
  *   warps_per_block  resident warps per SM (0 = built-in again)
  *   issue_point      where a game's background copy is handed to the TMA engine: 0 right before the sparse entries,

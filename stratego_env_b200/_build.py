@@ -45,16 +45,5 @@ def build_extension(force: bool = False, verbose: bool = False) -> str:
     return LIB_PATH
 
 
-def build_experiments(tag: str = "exp", defines=()) -> str:
-    """A SEPARATE copy of the library with the tuning / experiment switches compiled in (-DSX_EXPERIMENTS: environment
-    knobs SX_WARPS, SX_RING_WARPS, SX_RING_SLOTS, SX_DEBUG ...; some of them produce wrong results by design).  Only the
-    sweep tools load it, through SX_LIB; the shipped library never reads the environment."""
-    path = os.path.join(CSRC, "libstratego_b200_%s.so" % tag)
-    cmd = [_nvcc(), *NVCC_FLAGS, "-DSX_EXPERIMENTS", *["-D%s" % d for d in defines], "-o", path,
-           *[os.path.join(CSRC, s) for s in SOURCES]]
-    subprocess.run(cmd, check=True, cwd=CSRC)
-    return path
-
-
 if __name__ == "__main__":
     print(build_extension(force=True, verbose=True))

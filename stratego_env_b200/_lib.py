@@ -102,7 +102,8 @@ def load(build_if_missing: bool = True):
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("SX_LIB") or _build.LIB_PATH  # SX_LIB: tuning aid (alternative builds)
+    # SX_LIB: load another build of the library instead, e.g. to time two builds against each other
+    path = os.environ.get("SX_LIB") or _build.LIB_PATH
     if build_if_missing and path == _build.LIB_PATH and _build.is_stale():
         try:
             _build.build_extension()

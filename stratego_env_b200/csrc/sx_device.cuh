@@ -12,30 +12,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-// L2 cache-hint use per access class (1 = hinted instruction form).  Measured on B200: keeping the state
-// evict_last and streaming the outputs evict_first changes Barrage by < 2 % and costs Standard 10 %, so
-// the hints are compiled out by default; the switches stay for future tuning.
-#ifndef SX_HINT_ST
-#define SX_HINT_ST 0
-#endif
-#ifndef SX_HINT_ST8
-#define SX_HINT_ST8 0
-#endif
-#ifndef SX_HINT_TMA
-#define SX_HINT_TMA 0
-#endif
-#ifndef SX_HINT_CPASYNC
-#define SX_HINT_CPASYNC 0  /* cp.async + L2::cache_hint raises "illegal instruction" on sm_100a (CUDA 12.9) */
-#endif
-
-// K-loops of the hot functions: 1 keeps the fused loop small enough for the instruction cache
-#ifndef SX_UNROLL_K
-#define SX_UNROLL_K 1
-#endif
+// The per-lane cell loops (k < K) of the hot functions stay rolled (`#pragma unroll 1`): that keeps the fused loop small
+// enough for the instruction cache; unrolling them cost 9 % on Barrage / Standard (profiles/r2n_register_budget_sweep.txt).
 
 namespace sx {
-
-constexpr int UNROLL_K = SX_UNROLL_K;
 
 // ---- piece codes (impl:145-163) -----------------------------------------------------------------
 constexpr int SP_SPY = 1, SP_SCOUT = 2, SP_MINER = 3, SP_MARSHAL = 10, SP_FLAG = 11, SP_BOMB = 12, SP_UNKNOWN = 13;
@@ -210,57 +190,13 @@ __device__ __forceinline__ int fast_div(int x, uint32_t magic) { return int(__um
 // flat cell index in `me`'s frame <-> absolute frame: a 180-degree rotation is index reversal
 __device__ __forceinline__ int view(int cell, int flip, int N) { return flip ? N - 1 - cell : cell; }
 
-// ---- L2 residency hints ------------------------------------------------------------------------------
-// The ~0.3 KB/game state is re-read every step and fits in the 126 MB L2 for hundreds of thousands of games;
-// the ~30 KB/game outputs are written once and stream to HBM.  Marking the former evict_last and the latter
-// evict_first keeps the state resident, so the write stream is not interrupted by DRAM reads.
-__device__ __forceinline__ uint64_t l2_policy(int kind)  // 0 normal, 1 evict_last (keep), 2 evict_first (stream)
-{
-    uint64_t p;
-    if (kind == 1) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    else if (kind == 2) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    else asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void st_hint(float *p, float v, uint64_t pol)
-{
-    if (!SX_HINT_ST) { *p = v; return; }
-    asm volatile("st.global.L2::cache_hint.f32 [%0], %1, %2;" ::"l"(p), "f"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void st_hint(uint8_t *p, uint32_t v, uint64_t pol)
-{
-    if (!SX_HINT_ST8) { *p = uint8_t(v); return; }
-    asm volatile("st.global.L2::cache_hint.u8 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void st_hint(uint32_t *p, uint32_t v, uint64_t pol)
-{
-    if (!SX_HINT_ST) { *p = v; return; }
-    asm volatile("st.global.L2::cache_hint.b32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void st_hint(uint16_t *p, uint16_t v, uint64_t pol)
-{
-    if (!SX_HINT_ST) { *p = v; return; }
-    asm volatile("st.global.L2::cache_hint.b16 [%0], %1, %2;" ::"l"(p), "h"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void st_hint(uint4 *p, uint4 v, uint64_t pol)
-{
-    if (!SX_HINT_ST) { *p = v; return; }
-    asm volatile("st.global.L2::cache_hint.v4.b32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z),
-                 "r"(v.w), "l"(pol)
-                 : "memory");
-}
-
 // ---- TMA bulk copy shared -> global (SASS: UBLKCP), tracked by the issuing thread's bulk group -----
-__device__ __forceinline__ void bulk_store(void *gdst, const void *ssrc, uint32_t bytes, uint64_t pol)
+// Stores and copies carry no L2 cache hint: state evict_last + outputs evict_first measured < 2 % on Barrage and -10 % on
+// Standard, the reverse policy -2 to -5 % (DESIGN.md §3.1).
+__device__ __forceinline__ void bulk_store(void *gdst, const void *ssrc, uint32_t bytes)
 {
     const uint32_t saddr = static_cast<uint32_t>(__cvta_generic_to_shared(ssrc));
-    if (!SX_HINT_TMA) {
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(saddr), "r"(bytes) : "memory");
-        return;
-    }
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst), "r"(saddr),
-                 "r"(bytes), "l"(pol)
-                 : "memory");
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(saddr), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
@@ -273,7 +209,7 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 // <16-byte head and tail as plain word stores; otherwise (odd-sized variants such as 5x5 and 15x15,
 // whose per-env byte counts are not multiples of 16) the tile is copied with plain stores.
 template <class GT>
-static __device__ __noinline__ void emit_tile(uint8_t *gdst, const uint8_t *ssrc, int bytes, uint64_t pol)
+static __device__ __noinline__ void emit_tile(uint8_t *gdst, const uint8_t *ssrc, int bytes)
 {
     const int lane = GT::lane();
     const uintptr_t g = reinterpret_cast<uintptr_t>(gdst);
@@ -296,7 +232,7 @@ static __device__ __noinline__ void emit_tile(uint8_t *gdst, const uint8_t *ssrc
         const int off = head + body + ((lane - 4) << 2);
         *reinterpret_cast<uint32_t *>(gdst + off) = *reinterpret_cast<const uint32_t *>(ssrc + off);
     }
-    if (body > 0 && lane == 0) bulk_store(gdst + head, ssrc + head, uint32_t(body), pol);
+    if (body > 0 && lane == 0) bulk_store(gdst + head, ssrc + head, uint32_t(body));
 }
 
 // emit_tile for 16-bit observations: src, dst and bytes are even, and the callers pick a source congruent to the
@@ -304,7 +240,7 @@ static __device__ __noinline__ void emit_tile(uint8_t *gdst, const uint8_t *ssrc
 // go out as one half-word store per lane and the body as one TMA bulk copy.  A destination no image row can match (a
 // caller's buffer that starts inside a 64-byte cell of the 32-channel mode) is copied with half-word stores.
 template <class GT>
-static __device__ __noinline__ void emit_tile16(uint8_t *gdst, const uint8_t *ssrc, int bytes, uint64_t pol)
+static __device__ __noinline__ void emit_tile16(uint8_t *gdst, const uint8_t *ssrc, int bytes)
 {
     const int lane = GT::lane();
     const uintptr_t g = reinterpret_cast<uintptr_t>(gdst);
@@ -321,7 +257,7 @@ static __device__ __noinline__ void emit_tile16(uint8_t *gdst, const uint8_t *ss
     const int tail_at = (head + body) >> 1;
     if (lane < (head >> 1)) gd[lane] = sd[lane];
     if (lane < ((bytes - head - body) >> 1)) gd[tail_at + lane] = sd[tail_at + lane];
-    if (body > 0 && lane == 0) bulk_store(gdst + head, ssrc + head, uint32_t(body), pol);
+    if (body > 0 && lane == 0) bulk_store(gdst + head, ssrc + head, uint32_t(body));
 }
 
 // ---- occupancy bit-lines in `me`'s frame ------------------------------------------------------------
@@ -406,7 +342,7 @@ __device__ __forceinline__ bool gen_moves(const DevConfig &cfg, const WarpMem &m
 {
     const int lane = GT::lane();
     if (a.over) {  // impl:414
-#pragma unroll UNROLL_K
+#pragma unroll 1
         for (int k = 0; k < K; ++k) {
             const int p = lane * K + k;
             if (p < cfg.N) m.moves[p] = make_uint2(0, 0);
@@ -472,7 +408,7 @@ __device__ __forceinline__ bool gen_moves(const DevConfig &cfg, const WarpMem &m
             m.moves[p] = make_uint2(uint32_t(bits), uint32_t(bits >> 32));
         }
     } else {
-#pragma unroll UNROLL_K
+#pragma unroll 1
         for (int k = 0; k < K; ++k) {
             const int p = lane * K + k;
             if (p < cfg.N) {
@@ -494,19 +430,19 @@ __device__ __forceinline__ bool gen_moves(const DevConfig &cfg, const WarpMem &m
 // Expands m.moves into the spatial mask [cell][channel]: stores a 1 at every move on top of the zero
 // background at `image` (global memory).
 template <int K, class GT>
-__device__ __forceinline__ void mark_spatial(const DevConfig &cfg, const WarpMem &m, uint8_t *image, uint64_t pol)
+__device__ __forceinline__ void mark_spatial(const DevConfig &cfg, const WarpMem &m, uint8_t *image)
 {
     const int lane = GT::lane();
-#pragma unroll UNROLL_K
+#pragma unroll 1
     for (int k = 0; k < K; ++k) {
         const int p = lane * K + k;
         const uint2 bits = p < cfg.N ? m.moves[p] : make_uint2(0, 0);
         if ((bits.x | bits.y) != 0) {
             uint8_t *cell = image + p * cfg.A;
 #pragma unroll 1
-            for (uint32_t w = bits.x; w != 0; w &= w - 1) st_hint(cell + __ffs(w) - 1, 1u, pol);
+            for (uint32_t w = bits.x; w != 0; w &= w - 1) *(cell + __ffs(w) - 1) = 1;
 #pragma unroll 1
-            for (uint32_t w = bits.y; w != 0; w &= w - 1) st_hint(cell + 31 + __ffs(w), 1u, pol);
+            for (uint32_t w = bits.y; w != 0; w &= w - 1) *(cell + 31 + __ffs(w)) = 1;
         }
     }
 }
@@ -972,10 +908,10 @@ static __device__ __noinline__ void fill_background(const DevConfig &cfg, T *til
 // One game's background copy of a 16-bit observation of `elems` elements to `g`: the image row that makes the copy's
 // source congruent to g mod 16 is chosen, so the body leaves as one TMA bulk copy.
 template <class GT>
-__device__ __forceinline__ void emit_obs16(uint16_t *g, const uint16_t *bg, int channels, int elems, uint64_t pol)
+__device__ __forceinline__ void emit_obs16(uint16_t *g, const uint16_t *bg, int channels, int elems)
 {
     const int k = align_cells16(channels, int((reinterpret_cast<uintptr_t>(g) >> 1) & 7));
-    emit_tile16<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg + k * channels), elems * 2, pol);
+    emit_tile16<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg + k * channels), elems * 2);
 }
 
 // Writes the sparse, state-dependent entries of observer `me`'s observation on top of the background
@@ -983,34 +919,34 @@ __device__ __forceinline__ void emit_obs16(uint16_t *g, const uint16_t *bg, int 
 // ORIG = the deprecated 'original' channel mode: rank planes carry the normalised rank instead of one-hot groups.
 template <int K, class GT, bool ORIG = false, class T = float>
 __device__ __forceinline__ void patch_obs(const DevConfig &cfg, const WarpMem &m, const Aux &a, T *tile,
-                                          const ObsMap om, int me, uint64_t pol)
+                                          const ObsMap om, int me)
 {
     const int lane = GT::lane(), flip = me, CH = om.channels;
     const T one = obs_value<T>(cfg.unit_lut[1]);
-#pragma unroll UNROLL_K
+#pragma unroll 1
     for (int k = 0; k < K; ++k) {
         const int p = lane * K + k;
         if (p < cfg.N) {
             const uint32_t b = m.board[view(p, flip, cfg.N)];
             T *cell = tile + p * CH;
-            if (b & CELL_OBST) st_hint(cell + om.obstacle, one, pol);
+            if (b & CELL_OBST) *(cell + om.obstacle) = one;
             const int rank = b & CELL_RANK;
             if (rank) {
                 const int po = (b & CELL_REVEALED) ? rank : SP_UNKNOWN;
                 const bool own = int((b >> 4) & 1) == me;
                 if (ORIG) {  // impl:1178-1195 / impl:1102-1121 + maenv:499-508
                     if (own || om.enemy_true >= 0)
-                        st_hint(cell + (own ? om.own_true : om.enemy_true), obs_value<T>(cfg.rank_lut[rank]), pol);
-                    st_hint(cell + (own ? om.own_po : om.enemy_po), obs_value<T>(cfg.po_rank_lut[po]), pol);
-                    if (b & CELL_STILL) st_hint(cell + (own ? om.own_still : om.enemy_still), one, pol);
+                        *(cell + (own ? om.own_true : om.enemy_true)) = obs_value<T>(cfg.rank_lut[rank]);
+                    *(cell + (own ? om.own_po : om.enemy_po)) = obs_value<T>(cfg.po_rank_lut[po]);
+                    if (b & CELL_STILL) *(cell + (own ? om.own_still : om.enemy_still)) = one;
                 } else if (own) {
-                    st_hint(cell + om.own_true + rank - 1, one, pol);
-                    st_hint(cell + om.own_po + po - 1, one, pol);
-                    if (b & CELL_STILL) st_hint(cell + om.own_still, one, pol);
+                    *(cell + om.own_true + rank - 1) = one;
+                    *(cell + om.own_po + po - 1) = one;
+                    if (b & CELL_STILL) *(cell + om.own_still) = one;
                 } else {
-                    if (om.enemy_true >= 0) st_hint(cell + om.enemy_true + rank - 1, one, pol);
-                    st_hint(cell + om.enemy_po + po - 1, one, pol);
-                    if (b & CELL_STILL) st_hint(cell + om.enemy_still, one, pol);
+                    if (om.enemy_true >= 0) *(cell + om.enemy_true + rank - 1) = one;
+                    *(cell + om.enemy_po + po - 1) = one;
+                    if (b & CELL_STILL) *(cell + om.enemy_still) = one;
                 }
             }
         }
@@ -1020,14 +956,14 @@ __device__ __forceinline__ void patch_obs(const DevConfig &cfg, const WarpMem &m
         const int cell_abs = (lane & 1) ? a.rto[who] : a.rfrom[who];
         const int code = (lane & 1) ? -a.rcode[who] : 1;
         if (cell_abs != NO_CELL)
-            st_hint(tile + view(cell_abs, flip, cfg.N) * CH + (lane < 2 ? om.own_recent : om.enemy_recent),
-                    obs_value<T>(cfg.recent_lut[code + 3]), pol);
+            *(tile + view(cell_abs, flip, cfg.N) * CH + (lane < 2 ? om.own_recent : om.enemy_recent)) =
+                obs_value<T>(cfg.recent_lut[code + 3]);
     }
     for (int e = lane; e < a.ncap; e += GT::L) {
         const uint32_t ent = m.cap[e];
         const int cell_abs = ent & 0xff, owner = (ent >> 8) & 1, type0 = (ent >> 9) & 15, count = int(ent >> 13) + 1;
-        st_hint(tile + view(cell_abs, flip, cfg.N) * CH + (owner == me ? om.own_cap : om.enemy_cap) + type0,
-                obs_value<T>(cfg.cap_lut[type0 * 9 + count]), pol);
+        *(tile + view(cell_abs, flip, cfg.N) * CH + (owner == me ? om.own_cap : om.enemy_cap) + type0) =
+            obs_value<T>(cfg.cap_lut[type0 * 9 + count]);
     }
 }
 
@@ -1055,7 +991,7 @@ __device__ __forceinline__ int sample_move(const DevConfig &cfg, const WarpMem &
     if (!any_moves) return cfg.A - 1;  // the noop entry [0,0,A-1]
     const int lane = GT::lane();
     int mine = 0;
-#pragma unroll UNROLL_K
+#pragma unroll 1
     for (int k = 0; k < K; ++k) {
         const int p = lane * K + k;
         if (p < cfg.N) {

@@ -12,7 +12,6 @@
 
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -47,7 +46,7 @@ struct KernelArgs {
     const int32_t *actions;
     int action_format;
     const int8_t *player_override;
-    uint32_t flags, ops;  // flags: SX_* of the header in the low 16 bits, tuning / experiment switches above (sx_step_all)
+    uint32_t flags, ops;  // flags: SX_* of the header in the low 16 bits, result-preserving tuning bits above (sx_step_all)
     sx_outputs out;
     uint8_t *mask1d;
     const uint8_t *setups;
@@ -56,14 +55,12 @@ struct KernelArgs {
     const uint8_t *reset_mask;
     uint2 key;
     long long *stats;
-    int chunk_log2;  // log2 of the run of consecutive games a warp takes before it jumps ahead (0 = interleaved)
     const uint8_t *start_board;  // curriculum table (sx_config_set_start_states), n_start == 0: setups
     const int16_t *start_aux;
     const uint16_t *start_cap;
     uint32_t n_start;
     int32_t *start_index;  // [global env id - start_index_base], may be null
     long long start_index_base, start_index_len;
-    int exp_nap, exp_stagger;  // experiments builds only: ns to sleep before the copy wait / per warp index at the start
     int warp_bytes;  // shared-memory slice of one game (state + move sets + scratch)
     int tile_bytes;  // the block's background images (0 = this launch renders nothing)
 };
@@ -122,23 +119,22 @@ static __device__ __noinline__ void render_terminal(const KernelArgs *args, cons
     Aux a;
     aux_unpack(w, a);
     const ObsMap pom = original ? po_map_original() : po_map(), fom = original ? fo_map_original() : fo_map();
-    const uint64_t pol = l2_policy(0);
     T *tpo = reinterpret_cast<T *>(args->out.terminal_partial_obs), *tfo = reinterpret_cast<T *>(args->out.terminal_full_obs);
 #pragma unroll 1
     for (int side = 0; side < 2; ++side) {
         T *gpo = tpo ? tpo + (env * 2 + side) * cfg.po_floats : nullptr;
         T *gfo = tfo ? tfo + (env * 2 + side) * cfg.fo_floats : nullptr;
         if constexpr (sizeof(T) == 2) {
-            if (gpo) emit_obs16<GT>(gpo, bg_po, pom.channels, cfg.po_floats, pol);
-            if (gfo) emit_obs16<GT>(gfo, bg_fo, fom.channels, cfg.fo_floats, pol);
+            if (gpo) emit_obs16<GT>(gpo, bg_po, pom.channels, cfg.po_floats);
+            if (gfo) emit_obs16<GT>(gfo, bg_fo, fom.channels, cfg.fo_floats);
         } else {
             if (gpo) {
                 const int k = align_rows(pom.channels, int((reinterpret_cast<uintptr_t>(gpo) >> 2) & 3));
-                emit_tile<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<const uint8_t *>(bg_po + k * pom.channels), cfg.po_floats * 4, pol);
+                emit_tile<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<const uint8_t *>(bg_po + k * pom.channels), cfg.po_floats * 4);
             }
             if (gfo) {
                 const int k = align_rows(fom.channels, int((reinterpret_cast<uintptr_t>(gfo) >> 2) & 3));
-                emit_tile<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<const uint8_t *>(bg_fo + k * fom.channels), cfg.fo_floats * 4, pol);
+                emit_tile<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<const uint8_t *>(bg_fo + k * fom.channels), cfg.fo_floats * 4);
             }
         }
         if (GT::lane() == 0) bulk_commit();
@@ -146,11 +142,11 @@ static __device__ __noinline__ void render_terminal(const KernelArgs *args, cons
         if (GT::lane() == 0) bulk_wait_all();
         GT::sync();
         if (original) {
-            if (gpo) patch_obs<K, GT, true, T>(cfg, m, a, gpo, pom, side, pol);
-            if (gfo) patch_obs<K, GT, true, T>(cfg, m, a, gfo, fom, side, pol);
+            if (gpo) patch_obs<K, GT, true, T>(cfg, m, a, gpo, pom, side);
+            if (gfo) patch_obs<K, GT, true, T>(cfg, m, a, gfo, fom, side);
         } else {
-            if (gpo) patch_obs<K, GT, false, T>(cfg, m, a, gpo, pom, side, pol);
-            if (gfo) patch_obs<K, GT, false, T>(cfg, m, a, gfo, fom, side, pol);
+            if (gpo) patch_obs<K, GT, false, T>(cfg, m, a, gpo, pom, side);
+            if (gfo) patch_obs<K, GT, false, T>(cfg, m, a, gfo, fom, side);
         }
         GT::sync();
     }
@@ -221,25 +217,12 @@ __device__ __forceinline__ uint8_t illegal_code(StepStatus status, const Aux &a)
 }
 constexpr int MAX_REDRAWS = 8;  // re-draws of an unplayable setup (first player without a move) per reset
 
-#ifndef SX_MAX_THREADS
-#define SX_MAX_THREADS 512
-#endif
-// Experiment switches (flag bits 16-19 and 22-23 of KernelArgs::flags, and the SX_DEBUG / SX_WARPS / SX_BLOCKS /
-// SX_TOY / SX_TOY_WARPS / SX_GAMES_PER_WARP environment variables) exist only in builds made with -DSX_EXPERIMENTS
-// (tools/sweep_fused.py builds its own copy of the library): several of them produce WRONG results by design (skip
-// the copies, skip the sparse stores, no state write-back), so the shipped library neither reads the environment nor
-// contains those branches.  Bits 20-21 (where a game's background copy is issued) are result-preserving and stay.
-#ifdef SX_EXPERIMENTS
-#define SX_EXP(flags, bit) (((flags) & (bit)) != 0)
-#else
-#define SX_EXP(flags, bit) false
-#endif
 // Result-preserving tuning bits the host sets per variant (sx_step_all): bits 20-21 = where a game's background copy is
 // issued, bit 24 = SX_TUNE_COMMIT_GAP.
 // SX_TUNE_COMMIT_GAP: on the boards that issue the copy LATE, `cp.async.bulk.commit_group` is directly followed by
 // `cp.async.bulk.wait_group 0` (SASS: UTMACMDFLUSH; DEPBAR.LE SB0, 0 back to back), and that pair is slow on B200: ANY
-// instruction between the two -- a warp sync, `nanosleep 0`, or the never-taken experiment branches of a
-// -DSX_EXPERIMENTS build, which is how it was found -- makes the 15x15 board 37 % faster (55 -> 75 M env-steps/s), 5x5
+// instruction between the two -- a warp sync, `nanosleep 0`, or the never-taken branches of the experiments build it
+// was found with -- makes the 15x15 board 37 % faster (55 -> 75 M env-steps/s), 5x5
 // 12 %, 6x6 6 %, 8x8 2 % (profiles/r2q_experiment_branch_layout_sweep.txt, r2r_commit_wait_gap.txt).  The 10x10 board
 // with both observations is the one late-issue variant that does not gain (-1 %), so the host leaves the bit clear there.
 constexpr uint32_t SX_TUNE_COMMIT_GAP = 0x1000000u;
@@ -248,14 +231,9 @@ constexpr uint32_t SX_TUNE_COMMIT_GAP = 0x1000000u;
 // per warp gets 512 threads = 128 registers: with the 1 024-thread bound of round 1 the 6x6 / 8x8 kernels were held to
 // 64 registers and spilled ~230 bytes per thread -- measured (profiles/r2l_small_board_launch_bound_sweep.txt) 8x8:
 // 222 M env-steps/s at 1 024 threads / 16 warps, 242 M at 768 / 16, 272 M at 512 / 12; 6x6: 307 M / 337 M / 372 M.
-// Several games per warp (3x4 ... 5x5; SX_KG_THREADS) likewise: 5x5 385 M at 1 024 threads / 32 warps, 456 M at
-// 768 / 24, 492 M at 512 / 16 (profiles/r2m_small_board_sweep.txt).
-#ifndef SX_K2_THREADS
-#define SX_K2_THREADS 512
-#endif
-#ifndef SX_KG_THREADS
-#define SX_KG_THREADS 512
-#endif
+// Several games per warp (3x4 ... 5x5) likewise: 5x5 385 M at 1 024 threads / 32 warps, 456 M at 768 / 24, 492 M at
+// 512 / 16 (profiles/r2m_small_board_sweep.txt).
+constexpr int FUSED_THREADS = 512;
 // where the table entry a game is started from is recorded (sx_config_set_start_states); null = not recorded
 __device__ __forceinline__ int32_t *start_index_slot(const KernelArgs &args, long long env)
 {
@@ -266,7 +244,7 @@ __device__ __forceinline__ int32_t *start_index_slot(const KernelArgs &args, lon
 // CM: gen_moves hands movers to lanes (dense 10x10 boards).  T: observation element, float or uint16_t (bfloat16 /
 // float16 bit patterns); the 16-bit instantiations exist only for the modes that render observations.
 template <int K, int MODE, int G, bool CM = false, class T = float>
-__global__ void __launch_bounds__(K > 2 ? SX_MAX_THREADS : G == 1 ? SX_K2_THREADS : SX_KG_THREADS, 1)
+__global__ void __launch_bounds__(FUSED_THREADS, 1)
 sx_fused_kernel(const __grid_constant__ KernelArgs args)
 {
     using GT = Grp<G>;
@@ -305,9 +283,6 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
         fence_async_smem();  // generic-proxy writes above -> visible to the TMA engine (async proxy)
     }
     __syncthreads();
-    const bool hints = !SX_EXP(flags, 0x40000u);
-    const uint64_t pol_keep = l2_policy(hints ? 1 : 0), pol_stream = l2_policy(hints ? 2 : 0);
-    const uint64_t pol_bg = pol_stream;
 
     // ---- software pipeline -----------------------------------------------------------------------------
     // While game i runs, (1) game i+1's state / action loads are in flight in registers and (2) game i+1's
@@ -330,27 +305,26 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
         pf.action = do_step ? args.actions[e] : 0;
     };
     auto issue_background = [&](long long e) {
-        if (SX_EXP(flags, 0x10000u)) return;  // experiment: no background copies
         // the small mask copy goes first (measured: +3 % over observation-first at 10 warps per SM)
         if (do_mask) {
             uint8_t *gmask = args.out.valid_mask + e * cfg.mask_bytes;
-            emit_tile<GT>(gmask, bg.mask + (reinterpret_cast<uintptr_t>(gmask) & 15), cfg.mask_bytes, pol_bg);
+            emit_tile<GT>(gmask, bg.mask + (reinterpret_cast<uintptr_t>(gmask) & 15), cfg.mask_bytes);
         }
         if constexpr (sizeof(T) == 2) {
-            if (do_po) emit_obs16<GT>(reinterpret_cast<T *>(args.out.partial_obs) + e * cfg.po_floats, reinterpret_cast<const T *>(bg.po), pom.channels, cfg.po_floats, pol_bg);
-            if (do_fo) emit_obs16<GT>(reinterpret_cast<T *>(args.out.full_obs) + e * cfg.fo_floats, reinterpret_cast<const T *>(bg.fo), fom.channels, cfg.fo_floats, pol_bg);
+            if (do_po) emit_obs16<GT>(reinterpret_cast<T *>(args.out.partial_obs) + e * cfg.po_floats, reinterpret_cast<const T *>(bg.po), pom.channels, cfg.po_floats);
+            if (do_fo) emit_obs16<GT>(reinterpret_cast<T *>(args.out.full_obs) + e * cfg.fo_floats, reinterpret_cast<const T *>(bg.fo), fom.channels, cfg.fo_floats);
         } else {
             if (do_po) {
                 float *g = args.out.partial_obs + e * cfg.po_floats;
                 const int k = align_rows(pom.channels, int((reinterpret_cast<uintptr_t>(g) >> 2) & 3));
                 emit_tile<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg.po + k * pom.channels),
-                              cfg.po_floats * 4, pol_bg);
+                              cfg.po_floats * 4);
             }
             if (do_fo) {
                 float *g = args.out.full_obs + e * cfg.fo_floats;
                 const int k = align_rows(fom.channels, int((reinterpret_cast<uintptr_t>(g) >> 2) & 3));
                 emit_tile<GT>(reinterpret_cast<uint8_t *>(g), reinterpret_cast<const uint8_t *>(bg.fo + k * fom.channels),
-                              cfg.fo_floats * 4, pol_bg);
+                              cfg.fo_floats * 4);
             }
         }
         if (lane == 0) bulk_commit();
@@ -360,29 +334,20 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
     // one atomic each); attacks and the step count stay in registers / are derived, and are published once per launch.
     // (Eight live counters cost the 64-register kernels of the small boards 30 % more spill traffic.)
     uint32_t n_attacks = 0, n_steps = 0;
-    // Which games a warp takes: chunks of 2^chunk_log2 consecutive games, chunk c to game slot c mod (slots in the grid).
-    // chunk_log2 = 0 is the plain interleaving (game g to slot g mod slots).  Games are independent, so any order gives
-    // the same results; the order decides which addresses are written at the same time.
-    const long long total_warps = (long long)gridDim.x * warps_per_block;
-    const int chunk_lg = args.chunk_log2;
-    const long long chunk_mask = (1LL << chunk_lg) - 1;
-    auto next_game = [&](long long e) -> long long {
-        return (e & chunk_mask) != chunk_mask ? e + 1 : (((e >> chunk_lg) + total_warps) << chunk_lg);
-    };
-    long long env = ((long long)blockIdx.x * warps_per_block + warp) << chunk_lg;
-#ifdef SX_EXPERIMENTS
-    if (args.exp_stagger > 0) __nanosleep(args.exp_stagger * warp);
-#endif
+    // Game g goes to game slot g mod (slots in the grid).  (Runs of 8 or 32 consecutive games per slot measured -1 to
+    // -3 %, profiles/r2u_chunk_mapping_sweep.txt.)
+    const int total_warps = gridDim.x * warps_per_block;  // (a 64-bit stride made the ptxas allocation spill more)
+    long long env = (long long)blockIdx.x * warps_per_block + warp;
     Prefetched pf;
     // Where a game's background copy is issued.  The sparse entries must reach L2 while the background lines are
     // still resident there (otherwise every 4-byte store becomes a DRAM read-modify-write; measured: storing them one
     // whole game later costs 10-25 %), and the warp should have work to do while its copy drains.  0 = late, right
     // before the wait; 1 = after the outcome, before state write-back and sampling (best for a 10x10 board with one
     // observation: ~400 instructions overlap the drain); 2 = top of the game.  sx_step_all picks per variant
-    // (SX_DEBUG bits 4-5 override).
+    // (sx_config_set_tuning overrides).
     const int issue_at = (flags >> 20) & 3;
     if (env < args.num_envs) load_state(env, pf);
-    for (; env < args.num_envs; env = next_game(env)) {
+    for (; env < args.num_envs; env += total_warps) {
         const uint64_t gid = uint64_t(args.env_base + env);
         // ---- this game's state has arrived in registers: move it to the working slice, request the next ----
         GT::sync();
@@ -399,16 +364,10 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
             aux_unpack(w, a);
         }
         GT::sync();
-        const long long next_env = next_game(env);
+        const long long next_env = env + total_warps;
         const bool has_next = next_env < args.num_envs;
         if (has_next) load_state(next_env, pf);
         if (do_tile && issue_at == 2) issue_background(env);
-        if (SX_EXP(flags, 0x800000u)) {  // experiment: output skeleton only (no rules): background copy + wait
-            if (do_tile && issue_at != 2) issue_background(env);
-            if (lane == 0) bulk_wait_all();
-            GT::sync();
-            continue;
-        }
 
         bool dirty = false;
         // out-of-line helpers take and return everything by value so that `a` never has to live in local memory
@@ -521,17 +480,15 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
             if (!any && lane == 0) row[cfg.action_size - 1] = 1;  // impl:639-640
         }
 
-        if ((ops & OP_WRITE_STATE) && dirty && !SX_EXP(flags, 0x400000u)) {  // (0x400000: experiment, no state write-back)
+        if ((ops & OP_WRITE_STATE) && dirty) {
             uint32_t *gb = reinterpret_cast<uint32_t *>(args.board + env * cfg.board_stride);
-            for (int i = lane; i < (cfg.board_stride >> 2); i += GT::L)
-                st_hint(gb + i, reinterpret_cast<const uint32_t *>(m.board)[i], pol_keep);
+            for (int i = lane; i < (cfg.board_stride >> 2); i += GT::L) gb[i] = reinterpret_cast<const uint32_t *>(m.board)[i];
             uint32_t *gc = reinterpret_cast<uint32_t *>(args.cap + env * cfg.cap_stride);
-            for (int i = lane; i < (cfg.cap_stride >> 1); i += GT::L)
-                st_hint(gc + i, reinterpret_cast<const uint32_t *>(m.cap)[i], pol_keep);
+            for (int i = lane; i < (cfg.cap_stride >> 1); i += GT::L) gc[i] = reinterpret_cast<const uint32_t *>(m.cap)[i];
             if (lane == 0) {
                 uint32_t w[4];
                 aux_pack(a, w);
-                st_hint(reinterpret_cast<uint4 *>(args.aux + env * 8), make_uint4(w[0], w[1], w[2], w[3]), pol_keep);
+                *reinterpret_cast<uint4 *>(args.aux + env * 8) = make_uint4(w[0], w[1], w[2], w[3]);
             }
         }
 
@@ -546,24 +503,20 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
             issue_background(env);
             if (flags & SX_TUNE_COMMIT_GAP) GT::sync();  // keeps commit_group and wait_group apart (see SX_TUNE_COMMIT_GAP)
         }
-        if (do_tile && !SX_EXP(flags, 0x20000u)) {
-#ifdef SX_EXPERIMENTS
-            if (args.exp_nap > 0) __nanosleep(args.exp_nap);
-#endif
+        if (do_tile) {
             if (lane == 0) bulk_wait_all();  // this game's background is in global memory
             GT::sync();
-            if (SX_EXP(flags, 0x80000u)) continue;  // experiment: wait but skip the sparse stores
             if (original) {
-                if (do_po) patch_obs<K, GT, true, T>(cfg, m, a, reinterpret_cast<T *>(args.out.partial_obs) + env * cfg.po_floats, pom, viewer, pol_stream);
-                if (do_fo) patch_obs<K, GT, true, T>(cfg, m, a, reinterpret_cast<T *>(args.out.full_obs) + env * cfg.fo_floats, fom, viewer, pol_stream);
+                if (do_po) patch_obs<K, GT, true, T>(cfg, m, a, reinterpret_cast<T *>(args.out.partial_obs) + env * cfg.po_floats, pom, viewer);
+                if (do_fo) patch_obs<K, GT, true, T>(cfg, m, a, reinterpret_cast<T *>(args.out.full_obs) + env * cfg.fo_floats, fom, viewer);
             } else {
-                if (do_po) patch_obs<K, GT, false, T>(cfg, m, a, reinterpret_cast<T *>(args.out.partial_obs) + env * cfg.po_floats, pom, viewer, pol_stream);
-                if (do_fo) patch_obs<K, GT, false, T>(cfg, m, a, reinterpret_cast<T *>(args.out.full_obs) + env * cfg.fo_floats, fom, viewer, pol_stream);
+                if (do_po) patch_obs<K, GT, false, T>(cfg, m, a, reinterpret_cast<T *>(args.out.partial_obs) + env * cfg.po_floats, pom, viewer);
+                if (do_fo) patch_obs<K, GT, false, T>(cfg, m, a, reinterpret_cast<T *>(args.out.full_obs) + env * cfg.fo_floats, fom, viewer);
             }
             if (do_mask) {
                 uint8_t *gmask = args.out.valid_mask + env * cfg.mask_bytes;
-                mark_spatial<K, GT>(cfg, m, gmask, pol_stream);
-                if (!any && lane == 0) st_hint(gmask + cfg.A - 1, 1u, pol_stream);  // [0,0,A-1], impl:514-515
+                mark_spatial<K, GT>(cfg, m, gmask);
+                if (!any && lane == 0) *(gmask + cfg.A - 1) = 1;  // [0,0,A-1], impl:514-515
             }
         }
         GT::sync();
@@ -583,15 +536,11 @@ sx_fused_kernel(const __grid_constant__ KernelArgs args)
 // as many warps as shared memory holds.
 // compiled for the 12 warps it runs with: 144 registers instead of the 120 a 512-thread bound leaves (Micro +1 %, Tiny
 // +4 %, profiles/r2o_toy_register_budget_sweep.txt)
-#ifndef SX_TOY_TILES
-#define SX_TOY_TILES 2  /* observation tiles per warp: one is rendered while the copy of the other is read; divides 32 */
-#endif
-#ifndef SX_TOY_THREADS
-#define SX_TOY_THREADS 384
-#endif
+constexpr int TOY_TILES = 2;  // observation tiles per warp: one is rendered while the copy of the other is read; divides 32
+constexpr int TOY_THREADS = 384;
 // T: observation element, float or uint16_t (bfloat16 / float16 bit patterns)
 template <int MODE, class T = float>
-__global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_constant__ KernelArgs args)
+__global__ void __launch_bounds__(TOY_THREADS, 1) sx_toy_kernel(const __grid_constant__ KernelArgs args)
 {
     using GT = Grp<1>;
     extern __shared__ __align__(16) uint8_t smem[];
@@ -605,7 +554,6 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
     const bool do_sample = (flags & SX_SAMPLE_NEXT) && args.out.next_action != nullptr;
     const bool allow_osc = flags & SX_ALLOW_OSCILLATION;
     const ObsMap pom = po_map(), fom = fo_map();
-    const uint64_t pol = l2_policy(0);
 
     Tile bg;
     carve_tile<sizeof(T)>(cfg, ops, smem, &bg);
@@ -631,7 +579,7 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
     // copy (1 234 M / 914 M), two games rendered per pass by the half-warps (1 360 M).  Every one of them needs more
     // shared memory per warp, and the block's shared memory comes out of the SM's 256 KB L1: this kernel keeps ~100 bytes
     // of per-thread arrays in local memory, so it wants the L1 that 150 KB of shared memory leaves.
-    constexpr int NT = SX_TOY_TILES;
+    constexpr int NT = TOY_TILES;
     uint32_t undo_po[NT], undo_fo[NT];
 #pragma unroll
     for (int h = 0; h < NT; ++h) undo_po[h] = undo_fo[h] = lane < 16 ? 0u : toy::UNDO_NONE;  // cell lanes: "channel 0" four times
@@ -675,7 +623,7 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
             // the mask image is about to be rewritten: its copy is the OLDEST group of the previous 32 games, so it is
             // enough that all but the newest T - 1 groups (the last observation tiles, which the render loop below waits
             // for tile by tile) have been read; draining everything here stalled the warp once per 32 games (Micro +1 %)
-            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(SX_TOY_TILES - 1) : "memory");
+            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(TOY_TILES - 1) : "memory");
             __syncwarp();
             if (do_mask)
                 for (int i = lane; i < (mask_img_bytes >> 4); i += 32) reinterpret_cast<uint4 *>(mask_img)[i] = make_uint4(0, 0, 0, 0);
@@ -785,7 +733,7 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
         fence_async_smem();
         __syncwarp();
         if (do_mask) {  // the 32 mask rows are contiguous in the output tensor: one bulk copy (+ unaligned head / tail words)
-            emit_tile<GT>(gmask, mask_rows, mask_total, pol);
+            emit_tile<GT>(gmask, mask_rows, mask_total);
             if (lane == 0) bulk_commit();
         }
         if (do_po || do_fo) {
@@ -808,8 +756,8 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
                         if (do_fo) undo_fo[h] = toy::patch_tile(cfg, st, tfo, fom, lane);
                         fence_async_smem();
                         __syncwarp();
-                        if (do_po) emit_tile16<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<uint8_t *>(tpo), po_bytes, pol);
-                        if (do_fo) emit_tile16<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<uint8_t *>(tfo), fo_bytes, pol);
+                        if (do_po) emit_tile16<GT>(reinterpret_cast<uint8_t *>(gpo), reinterpret_cast<uint8_t *>(tpo), po_bytes);
+                        if (do_fo) emit_tile16<GT>(reinterpret_cast<uint8_t *>(gfo), reinterpret_cast<uint8_t *>(tfo), fo_bytes);
                         if (lane == 0) bulk_commit();
                     } else {
                         if (do_po) toy::restore_tile(cfg, reinterpret_cast<float *>(tile), pom, lane, undo_po[h]);
@@ -821,8 +769,8 @@ __global__ void __launch_bounds__(SX_TOY_THREADS, 1) sx_toy_kernel(const __grid_
                         fence_async_smem();
                         __syncwarp();
                         if (lane == 0) {
-                            if (do_po) bulk_store(gpo, tile, uint32_t(po_bytes), pol);
-                            if (do_fo) bulk_store(gfo, tile + po_bytes, uint32_t(fo_bytes), pol);
+                            if (do_po) bulk_store(gpo, tile, uint32_t(po_bytes));
+                            if (do_fo) bulk_store(gfo, tile + po_bytes, uint32_t(fo_bytes));
                             bulk_commit();
                         }
                     }
@@ -1048,18 +996,6 @@ static int fail(const std::string &msg)
 int sx_set_error(const std::string &msg) { return fail(msg); }  // for the other translation units of the library
 static int cuda_fail(const char *what, cudaError_t e) { return fail(std::string(what) + ": " + cudaGetErrorString(e)); }
 
-// tuning knobs: read from the environment only in -DSX_EXPERIMENTS builds (see SX_EXP above)
-static int env_int(const char *name, int fallback)
-{
-#ifdef SX_EXPERIMENTS
-    const char *v = std::getenv(name);
-    return (v && *v) ? std::atoi(v) : fallback;
-#else
-    (void)name;
-    return fallback;
-#endif
-}
-
 extern "C" const char *sx_last_error(void) { return g_error.c_str(); }
 extern "C" int sx_version(void) { return 1; }
 
@@ -1138,14 +1074,12 @@ extern "C" int sx_config_create(const sx_config_desc *desc, sx_config **out)
     // games per warp: small boards share a warp (each game needs max(R, C) <= lanes / 2 and N <= 2 * lanes)
     const int side = std::max(d.R, d.C);
     c->games_per_warp = (side <= 4 && d.N <= 16) ? 4 : (side <= 8 && d.N <= 32) ? 2 : 1;
-    if (env_int("SX_GAMES_PER_WARP", 0) == 1) c->games_per_warp = 1;  // tuning / A-B switch
     const int lanes = 32 / c->games_per_warp;
     const int k = (d.N + lanes - 1) / lanes;
     c->cells_per_lane = k <= 2 ? 2 : k <= 4 ? 4 : 8;
     // dense boards of the 10x10 class: movers are handed to lanes (measured: Standard, 40 pieces a side, +4 %; Barrage, 8
     // pieces, -3 %; profiles/r3g_all_boards.txt)
     c->compact_movers = c->cells_per_lane == 4 && c->games_per_warp == 1 && pieces > 16;
-    if (const int cm = env_int("SX_COMPACT", -1); cm >= 0) c->compact_movers = cm != 0 && c->cells_per_lane == 4 && c->games_per_warp == 1;
     sx_layout &l = c->layout;
     l.rows = d.R; l.cols = d.C; l.cells = d.N; l.spatial_channels = d.A; l.spatial_actions = d.mask_bytes;
     l.action_size = d.action_size; l.board_stride = d.board_stride; l.aux_stride = 8; l.captured_stride = d.cap_stride;
@@ -1174,7 +1108,7 @@ extern "C" int sx_config_set_start_states(sx_config *cfg, sx_state table, int64_
     return 0;
 }
 
-// Result-preserving launch tuning (include/stratego_b200.h): lets tools/sweep_fused.py time the SHIPPED library under
+// Result-preserving launch tuning (include/stratego_b200.h): lets tools/sweep_tuning.py time the shipped library under
 // other launch shapes than the built-in ones.  None of the three settings changes a result.
 extern "C" int sx_config_set_tuning(sx_config *cfg, int32_t warps_per_block, int32_t issue_point, int32_t compact_movers)
 {
@@ -1274,8 +1208,8 @@ static Shape16 shape16(const DevConfig &d, uint32_t ops)
     return {16, 1};                              // 8x8, 6x6, 5x5 and the warp-level path of the toy boards
 }
 
-// Block shape: one block per SM with as many warps as the register file allows (SX_WARPS overrides; a
-// tuning aid); the block's shared memory is the background images plus one small slice per warp.
+// Block shape: one block per SM with as many warps as the register file allows
+// (sx_config_set_tuning overrides); the block's shared memory is the background images plus one small slice per warp.
 static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, long long num_envs, LaunchPlan *plan,
                                 int compressed_warps);
 
@@ -1367,7 +1301,7 @@ static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, lo
                     : tile_bytes <= 64 * 1024 ? 6 : 10;  // 15x15 (74 KB per game): 4 warps 39 M, 6: 55 M, 8: 69 M, 10: 75 M env-steps/s
     if (cfg->obs_elem_bytes == 2 && (ops & (OP_PO | OP_FO))) preferred = shape16(cfg->dev, ops).warps;
     if (compressed_warps) preferred = compressed_warps;
-    int warps = std::min(max_warps, std::max(1, env_int("SX_WARPS", std::min(max_warps, cfg->tune_warps > 0 ? cfg->tune_warps : preferred))));
+    int warps = std::min(max_warps, std::max(1, cfg->tune_warps > 0 ? cfg->tune_warps : preferred));
     const int games = cfg->games_per_warp;  // each game of a warp has its own slice
     while (warps > 1 && tile_bytes + warps * games * warp_bytes > max_smem_optin) --warps;
     const int smem = tile_bytes + warps * games * warp_bytes;
@@ -1376,7 +1310,7 @@ static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, lo
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, fn, warps * 32, size_t(smem));
     if (e != cudaSuccess) return cuda_fail("cudaOccupancyMaxActiveBlocksPerMultiprocessor", e);
     if (blocks < 1) return fail("fused kernel cannot be resident on this device");
-    blocks = std::max(1, std::min(blocks, env_int("SX_BLOCKS", tile_bytes > 8 * 1024 ? 1 : blocks)));
+    if (tile_bytes > 8 * 1024) blocks = 1;
     plan->warps_per_block = warps;
     plan->blocks_per_sm = blocks;
     plan->smem_per_block = smem;
@@ -1397,7 +1331,7 @@ static int plan_launch_uncached(const sx_config *cfg, uint32_t ops, int mode, lo
 static bool toy_eligible(const sx_config *cfg, const KernelArgs &a, int mode)
 {
     const DevConfig &d = cfg->dev;
-    if (env_int("SX_TOY", 1) == 0 || (a.flags & (SX_KERNEL_BASELINE | SX_REPEAT_OTHER_SIDE))) return false;
+    if (a.flags & (SX_KERNEL_BASELINE | SX_REPEAT_OTHER_SIDE)) return false;
     if (a.out.terminal_partial_obs || a.out.terminal_full_obs) return false;
     if (cfg->n_start_states > 0) return false;  // curriculum starts are a warp-level kernel feature
     if (mode != MODE_STEP_PO_MASK && mode != MODE_STEP_PO_FO_MASK && mode != MODE_STEP_LEAN) return false;
@@ -1430,7 +1364,7 @@ static int toy_warp_bytes(const sx_config *cfg, uint32_t ops)
     const int mask_img = (ops & OP_MASK) ? round16(toy::GAMES * d.mask_bytes + 16) : 0;
     const int po = (ops & OP_PO) ? d.po_floats * eb : 0, fo = (ops & OP_FO) ? d.fo_floats * eb : 0;
     const int tile = eb == 2 ? toy::tile_slot(po) + toy::tile_slot(fo) : po + fo;
-    return toy::GAMES * toy::STAGE_BYTES + mask_img + SX_TOY_TILES * tile;
+    return toy::GAMES * toy::STAGE_BYTES + mask_img + TOY_TILES * tile;
 }
 
 struct ToyPlan {
@@ -1449,7 +1383,7 @@ static int plan_toy(const sx_config *cfg, uint32_t ops, ToyPlan *plan)
     // 13-16: 1.40-1.43 G env-steps/s; Tiny 8: 1.02 G, 10-13: 1.08 G
     // (Tiny 4x4 peaks at 11 warps: 1 113 M vs 1 072 M at 12, measured twice, profiles/r2o_*, r2t_*.  A warp sync between a
     // pass's commit_group and the next pass's wait_group.read changes nothing here: that wait is for an older group.)
-    plan->warps = std::max(1, std::min(SX_TOY_THREADS / 32, env_int("SX_TOY_WARPS", cfg->dev.N <= 12 ? 12 : 11)));
+    plan->warps = std::min(TOY_THREADS / 32, cfg->dev.N <= 12 ? 12 : 11);
     while (plan->warps > 1 && plan->tile_bytes + plan->warps * plan->warp_bytes > max_smem) --plan->warps;
     plan->smem = plan->tile_bytes + plan->warps * plan->warp_bytes;
     if (plan->smem > max_smem) return fail("toy kernel does not fit in shared memory");
@@ -1535,10 +1469,6 @@ static int launch_fused(const sx_config *cfg, KernelArgs &args, cudaStream_t str
     args.tile_bytes = plan.tile_bytes;
     // launches without a step (sx_observe, sx_valid_mask, the observe pass of a reset) issue their copies late
     if (!(args.ops & OP_STEP)) args.flags |= SX_TUNE_COMMIT_GAP;
-    args.chunk_log2 = std::max(0, std::min(10, env_int("SX_CHUNK_LOG2", 0)));
-    args.exp_nap = env_int("SX_NAP", 0);
-    args.exp_stagger = env_int("SX_STAGGER", 0);
-    if (const int gap = env_int("SX_GAP", -1); gap >= 0) args.flags = gap ? (args.flags | SX_TUNE_COMMIT_GAP) : (args.flags & ~SX_TUNE_COMMIT_GAP);
     // (Tried and removed: marking the state range as persisting in L2 with an access-policy window.  A pure store
     // stream loses ~8 % when the ~0.2 KB/game state reads come from DRAM (tools/probes/probe_write.cu), but any L2
     // set-aside large enough to hold the state takes capacity from the output lines that wait for their sparse
@@ -1672,13 +1602,12 @@ extern "C" int sx_step(const sx_config *cfg, sx_state st, int64_t num_envs, cons
     return launch_fused(cfg, a, static_cast<cudaStream_t>(stream));
 }
 
-static uint32_t step_all_ops(const sx_outputs &out, uint32_t flags)
+static uint32_t step_all_ops(const sx_outputs &out)
 {
     uint32_t ops = OP_STEP | OP_WRITE_STATE | OP_NEED_MOVES;
     if (out.valid_mask) ops |= OP_MASK;
     if (out.partial_obs) ops |= OP_PO;
     if (out.full_obs) ops |= OP_FO;
-    (void)flags;
     return ops;
 }
 
@@ -1696,26 +1625,22 @@ extern "C" int sx_step_all(const sx_config *cfg, sx_state st, int64_t num_envs, 
     KernelArgs a;
     base_args(a, st, num_envs, env_base);
     a.actions = actions_d; a.action_format = action_format;
-    // bits 16+: tuning / experiment switches (SX_DEBUG overrides; they exist for tools/sweep_fused.py, results are WRONG
-    // with 1, 2, 8, 64 or 128): 1 skip TMA, 2 skip wait + sparse stores, 4 plain L2 policy, 8 skip sparse stores, 16 / 32
-    // background issue point (after the outcome / top of the game; default late), 64 no state write-back, 128 output
-    // skeleton only.
-    // B200 sweeps (tools/sweep_fused.py, profiles/r1k_sweep*.txt): a 10x10 board with ONE observation is fastest with the
-    // copy issued after the outcome (16) at 8 warps per SM; both observations and the smaller boards issue late (0).
+    // flag bits 20-21: where a game's background copy is issued (0 late, 1 after the outcome, 2 top of the game).
+    // B200 sweeps (profiles/r1k_sweeps.txt): a 10x10 board with ONE observation is fastest with the copy issued after the
+    // outcome at 8 warps per SM; both observations and the smaller boards issue late.
     const bool one_obs = (out.partial_obs != nullptr) != (out.full_obs != nullptr);
     const int n = cfg->dev.N;
     const bool ten_by_ten = n >= 100 && n <= 128;
     // boards up to 10x10 with one observation issue the copy after the outcome (shipped-library sweeps, profiles/
     // r3o_shipped_tuning_sweep.txt, r3y_small_boards_tuning.txt: 8x8 +2.1 %, 6x6 +3.5 %, 5x5 +3.8 % over a late issue); both
     // observations and the 15x15 board issue late (15x15: 79.8 M late, 76.8 M after the outcome)
-    const uint32_t ops = step_all_ops(out, flags);
+    const uint32_t ops = step_all_ops(out);
     const int issue = cfg->tune_issue >= 0 ? cfg->tune_issue
                     : compressed_warps_for(cfg, out, ops) ? 0
                     : (cfg->obs_elem_bytes == 2 && (ops & (OP_PO | OP_FO))) ? shape16(cfg->dev, ops).issue
                     : (n <= 128 && one_obs) ? 1 : 0;
-    const int tune = env_int("SX_DEBUG", issue << 4);
-    a.flags = (flags & 0xffffu) | (uint32_t(tune) << 16);
-    if ((tune & 0x30) == 0 && !ten_by_ten) a.flags |= SX_TUNE_COMMIT_GAP;  // late issue, not the 10x10 board
+    a.flags = (flags & 0xffffu) | (uint32_t(issue) << 20);
+    if (issue == 0 && !ten_by_ten) a.flags |= SX_TUNE_COMMIT_GAP;  // late issue, not the 10x10 board
     a.out = out;
     a.ops = ops;
     a.setups = setups_d; a.n_setups = n_setups;

@@ -1,7 +1,6 @@
 """Launch-shape sweep of the SHIPPED library through sx_config_set_tuning (result-preserving knobs only): one process,
 one de-phased state, many (warps per SM, issue point, compact movers) settings; `-` keeps the built-in choice.
-    python tools/sweep_tuning.py <workload> "<warps>:<issue 0|1|2>:<compact 0|1>,..." [envs]
-(tools/sweep_fused.py does the same for an EXPERIMENTS build and its result-changing switches.)"""
+    python tools/sweep_tuning.py <workload> "<warps>:<issue 0|1|2>:<compact 0|1>,..." [envs]"""
 import sys
 
 import torch
