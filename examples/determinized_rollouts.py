@@ -3,7 +3,7 @@ pieces.
 
 1. Play a batch of Barrage games a few random moves in.
 2. Draw K complete game states per game that agree with what the player to move knows (sample_hidden_states).
-3. Play every sampled world to its end with uniformly random moves (step_all(..., sample_next=True, auto_reset=False)).
+3. Play every sampled world to its end with uniformly random moves (playout: one launch, no host loop).
 4. Average the outcome per original game, from the point of view of its player to move.
 
     python examples/determinized_rollouts.py [--games 1024] [--worlds 32] [--max-plies 3000]
@@ -11,8 +11,6 @@ pieces.
 import argparse
 import os
 import sys
-
-import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from stratego_env_b200.batched_env import BatchedStrategoEnv  # noqa: E402
@@ -33,23 +31,11 @@ def main():
     me = obs["player"].clone()  # the player to move in each original game
 
     worlds = env.sample_hidden_states(n_samples=K)  # row b * K + k: world k of game b
-    eng = env.engine
-    out = eng.alloc_outputs(B * K, partial=False, full=False, mask=True, sample=True)
-    eng.observe(worlds, out=out, partial=False, full=False, mask=True)
-    actions = eng.sample_valid(out["valid_mask"], seed=2)
-    winner = torch.zeros(B * K, dtype=torch.int8, device=env.device)
-    finished = torch.zeros(B * K, dtype=torch.bool, device=env.device)
-    for ply in range(args.max_plies):
-        eng.step_all(worlds, actions, out, auto_reset=False, sample_next=True, seed=2)
-        ended = out["done"] != 0
-        winner = torch.where(ended, out["winner"], winner)
-        finished |= ended
-        actions = out["next_action"].clone()
-        if ply % 100 == 99 and bool(finished.all()):
-            break
+    res = env.engine.playout(worlds, max_plies=args.max_plies, seed=2)
+    winner, finished = res.winner, res.done == 1
     value = (winner.view(B, K).float() * me.view(B, 1).float()).mean(1)  # +1 win, -1 loss, 0 draw or unfinished
-    print("%d games x %d worlds, %d plies, %.1f %% of the worlds finished" % (B, K, ply + 1,
-                                                                             100 * finished.float().mean().item()))
+    print("%d games x %d worlds, longest playout %d plies, %.1f %% of the worlds finished" % (
+        B, K, int(res.plies.max().item()), 100 * finished.float().mean().item()))
     print("value for the player to move: mean %+.3f, min %+.3f, max %+.3f" % (value.mean().item(), value.min().item(),
                                                                              value.max().item()))
     print("first games:", " ".join("%+.2f" % v for v in value[:8].tolist()))

@@ -3,15 +3,15 @@
 At each of its turns the searcher, for every game in the batch at once:
 1. draws K complete worlds that agree with what it knows (sample_hidden_states, viewer = the player to move);
 2. expands every world (expand_moves): one child per legal move, the same action list in every world;
-3. plays every child on with uniformly random moves (step_all(..., sample_next=True, auto_reset=False)) for at most
-   --rollout-plies plies, scoring a win +1, a loss -1 and an unfinished rollout or a turn-limit ending 0;
+3. plays every child on with uniformly random moves (playout) for at most --rollout-plies plies, scoring a win +1, a
+   loss -1 and an unfinished rollout or a turn-limit ending 0;
 4. averages the score per (game, position in the action list) over the K worlds and plays the argmax.
 The random player moves uniformly among its legal moves.  The searcher is player +1 and moves first.
 
     python examples/pimc_one_ply.py [--games 256] [--worlds 16] [--rollout-plies 200]
 
-With the defaults the searcher won 225 and lost 31 of 256 games, in 7.0 s on a B200 at 1 000 W
-(profiles/r7a_expand_moves.txt).
+With the defaults the searcher won 228 and lost 28 of 256 games, in 1.4 s on a B200 at 1 000 W
+(profiles/r7c_examples.txt).
 """
 import argparse
 import os
@@ -33,18 +33,8 @@ def search(e, st, games, K, plies, seed, draw):
     ex = e.expand_moves(worlds)
     T = ex.states.num_envs
     mover = -ex.player.float()  # the player who made the move (the child's player to move is the other one)
-    score = torch.where(ex.done == 1, ex.winner.float() * mover, torch.zeros_like(mover))
-    finished = ex.done == 1
-    kids = ex.states
-    out = e.alloc_outputs(T, partial=False, full=False, mask=True, sample=True)
-    e.observe(kids, out=out, partial=False, full=False, mask=True)
-    actions = e.sample_valid(out["valid_mask"], seed=seed, step=draw)
-    for _ in range(plies):
-        e.step_all(kids, actions, out, auto_reset=False, sample_next=True, seed=seed ^ draw)
-        ended = (out["done"] == 1) & ~finished
-        score = torch.where(ended, out["winner"].float() * mover, score)
-        finished |= ended
-        actions = out["next_action"].clone()
+    rollout = e.playout(ex.states, max_plies=plies, seed=seed ^ draw)  # a child that is already over plays nothing
+    score = torch.where(rollout.done == 1, rollout.winner.float() * mover, torch.zeros_like(mover))
     # child row -> (game, position j in the action list); the K worlds of a game share one action list
     game = ex.parent // K
     j = torch.arange(T, device=e.device) - ex.offsets[ex.parent]

@@ -295,6 +295,32 @@ int sx_count_moves(const sx_config *cfg, sx_state st, int64_t num_envs, int32_t 
 int sx_expand_moves(const sx_config *cfg, sx_state st, int64_t num_envs, const int64_t *offsets_d, int64_t n_children,
                     sx_state out, int32_t *actions_d, sx_outputs out_scalars, void *stream);
 
+/* Random playouts, for scoring search leaves: every game of the batch is played on with uniformly random legal moves
+ * until it ends or max_plies plies have been played, whichever comes first.  st is updated in place, like sx_step_all.
+ * The move of each ply is the SX_SAMPLE_NEXT draw of sx_step_all for the state before that ply: Philox4x32-10 with key
+ * (seed lo, seed hi) and counter (gid lo, gid hi, RNG_SAMPLE ^ (turn & 0xffff), episode), gid = env_base + b, first
+ * output word w; the move is number __umulhi(w, n_moves) of the player to move's moves in ascending flat spatial index
+ * (that player's frame).  So a playout of n plies equals, byte for byte (board with padding, aux, capture list and the
+ * scalars below), this chain: a = that draw on the initial state; repeat { sx_step_all(a, SX_ACTION_SPATIAL,
+ * SX_SAMPLE_NEXT, no auto-reset, same seed and env_base); a = next_action } until a step reports done or n steps have
+ * run.  A playout therefore continues the chain a caller's last sx_step_all with that seed started (its first move is
+ * the next_action that step returned), playout(a) then playout(b) equals playout(a + b), and the result depends on
+ * (seed, gid, state) only, not on the batch split.  Two cases differ from that chain:
+ *  - a game that is over at entry plays 0 plies and its rows are not written (a step of a finished game flips player);
+ *  - a player to move with no legal move (only an imported state can be so) draws the noop entry A-1 and loses by it,
+ *    as sx_step_all does with the 1D noop action (SX_ACTION_1D, action_size - 1); the spatial noop entry would be
+ *    rejected as illegal, and the chain would never end.
+ * Every game that is not over ends within max_turns - turn + 1 plies (turn limit), so max_plies = INT32_MAX plays every
+ * game to its end.
+ * Outputs per game, each optional (NULL): plies_d (int32) the plies played in this call; in out_scalars, as the step
+ * that ended the game reported them (or, for a game over at entry, computed the same way from its aux): done (1 if the
+ * game is over at the end of the call), winner, ending_invalid, reward; illegal (0, or 2 once the capture list has
+ * overflowed: sticky, as in the step); player (to move at the end).  Refused: a null config or state tensor,
+ * max_plies < 0, and a non-null observation, mask, next_action or terminal pointer in out_scalars.  num_envs <= 0:
+ * nothing to do. */
+int sx_playout(const sx_config *cfg, sx_state st, int64_t num_envs, int64_t env_base, int32_t max_plies,
+               uint64_t seed, int32_t *plies_d, sx_outputs out_scalars, void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

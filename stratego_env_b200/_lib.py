@@ -72,6 +72,7 @@ SYMBOLS = {
     "sx_sample_hidden_states": (C.c_int, [_vp, SxState, _i64, _i64, _vp, _i32, _u64, _u32, SxState, _vp, _vp]),
     "sx_count_moves": (C.c_int, [_vp, SxState, _i64, _vp, _vp]),
     "sx_expand_moves": (C.c_int, [_vp, SxState, _i64, _vp, _i64, SxState, _vp, SxOutputs, _vp]),
+    "sx_playout": (C.c_int, [_vp, SxState, _i64, _i64, _i32, _u64, _vp, SxOutputs, _vp]),
     "sx_step_all_launch_info": (C.c_int, [_vp, _u32, C.POINTER(SxLaunchInfo)]),
     "sx_device_alloc": (C.c_int, [_i32, _u64, _u32, C.POINTER(_vp), C.POINTER(_u32)]),
     "sx_device_free": (C.c_int, [_vp]),

@@ -685,6 +685,40 @@ __device__ __forceinline__ StepStatus apply_move(const DevConfig &cfg, const War
     return STEP_MOVED;
 }
 
+// impl:1029-1043, the rest of a step after apply_move returned STEP_MOVED for `mover`: the next player's move sets in
+// m.moves, the opponent-stuck win and the turn limit.  Returns whether the next player has a move.  Used by the search
+// kernels (sx_expand.cu, sx_playout.cu); the fused kernel keeps its own copy, which also serves viewers other than the
+// player to move and the terminal re-generation of its outputs.
+template <int K, class GT, bool CM>
+__device__ __forceinline__ bool after_move(const DevConfig &cfg, const WarpMem &m, Aux &a, int mover)
+{
+    const bool any = gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
+    if (!any && !a.over) { a.over = 1; a.winner = mover == 0 ? 1 : -1; }  // impl:1031-1036
+    if (a.turn >= a.max_turns && !a.over) { a.over = 1; a.invalid = 1; }  // impl:1040-1043
+    return any;
+}
+
+// stages game b's board (padding included) and, with scap non-null, its capture list in shared memory (one warp);
+// returns its packed aux words
+__device__ __forceinline__ uint4 load_game(const DevConfig &cfg, const uint8_t *board, const int16_t *aux, const uint16_t *cap,
+                                           long long b, uint8_t *sboard, uint16_t *scap)
+{
+    const int lane = threadIdx.x & 31;
+    const uint32_t *gb = reinterpret_cast<const uint32_t *>(board + b * cfg.board_stride);
+    for (int w = lane; w < (cfg.board_stride >> 2); w += 32) reinterpret_cast<uint32_t *>(sboard)[w] = gb[w];
+    if (scap) {
+        const uint32_t *gc = reinterpret_cast<const uint32_t *>(cap + b * cfg.cap_stride);
+        for (int w = lane; w < (cfg.cap_stride >> 1); w += 32) reinterpret_cast<uint32_t *>(scap)[w] = gc[w];
+    }
+    return *reinterpret_cast<const uint4 *>(aux + b * 8);
+}
+
+__device__ __forceinline__ void unpack(uint4 aw, Aux &a)
+{
+    const uint32_t w[4] = {aw.x, aw.y, aw.z, aw.w};
+    aux_unpack(w, a);
+}
+
 // ---- setups / reset (impl:213-249, util:13-53, util:241-319) ---------------------------------------
 // own_map[i], i < setup_len: piece code at own-frame cell i (row-major over the usable rows).
 template <class GT>

@@ -17,7 +17,6 @@
 // working copy of the parent staged in shared memory: apply_move, the next player's gen_moves, the outcome, the child row.
 #include <cuda_runtime.h>
 
-#include <algorithm>
 #include <cstdint>
 #include <string>
 
@@ -28,26 +27,6 @@
 namespace sx {
 
 constexpr int EXPAND_WARPS = 8;  // warps per block of both kernels
-
-// stages game b's board (padding included) and capture list in the warp's slice; returns its packed aux words
-__device__ __forceinline__ uint4 load_game(const DevConfig &cfg, const uint8_t *board, const int16_t *aux, const uint16_t *cap,
-                                           long long b, uint8_t *sboard, uint16_t *scap)
-{
-    const int lane = threadIdx.x & 31;
-    const uint32_t *gb = reinterpret_cast<const uint32_t *>(board + b * cfg.board_stride);
-    for (int w = lane; w < (cfg.board_stride >> 2); w += 32) reinterpret_cast<uint32_t *>(sboard)[w] = gb[w];
-    if (scap) {
-        const uint32_t *gc = reinterpret_cast<const uint32_t *>(cap + b * cfg.cap_stride);
-        for (int w = lane; w < (cfg.cap_stride >> 1); w += 32) reinterpret_cast<uint32_t *>(scap)[w] = gc[w];
-    }
-    return *reinterpret_cast<const uint4 *>(aux + b * 8);
-}
-
-__device__ __forceinline__ void unpack(uint4 aw, Aux &a)
-{
-    const uint32_t w[4] = {aw.x, aw.y, aw.z, aw.w};
-    aux_unpack(w, a);
-}
 
 // moves of the player to move in m.moves (all zero for a finished game or a stuck player); returns their number
 template <int K, bool CM>
@@ -180,11 +159,7 @@ __global__ void __launch_bounds__(EXPAND_WARPS * 32, 3) sx_expand_moves_kernel(
                 const Move mv = decode_spatial(cfg, action, mover);
                 int attack;
                 const StepStatus status = apply_move<GT>(cfg, m, a, mv, false, attack);
-                if (status == STEP_MOVED) {
-                    const bool any = gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
-                    if (!any && !a.over) { a.over = 1; a.winner = mover == 0 ? 1 : -1; }  // impl:1031-1036
-                    if (a.turn >= a.max_turns && !a.over) { a.over = 1; a.invalid = 1; }  // impl:1040-1043
-                }
+                if (status == STEP_MOVED) after_move<K, GT, CM>(cfg, m, a, mover);
                 const bool done = status != STEP_ILLEGAL && a.over;
                 uint32_t w4[4];
                 aux_pack(a, w4);
@@ -215,16 +190,6 @@ __global__ void __launch_bounds__(EXPAND_WARPS * 32, 3) sx_expand_moves_kernel(
 typedef void (*count_fn)(DevConfig, const uint8_t *, const int16_t *, long long, int32_t *, int);
 typedef void (*expand_fn)(DevConfig, const uint8_t *, const int16_t *, const uint16_t *, long long, const int64_t *, long long,
                           uint8_t *, int16_t *, uint16_t *, int32_t *, sx_outputs, int);
-
-// the instantiation launch_policy (sx_policy.cu) picks: cells per lane by board size, compact movers where configured
-template <class F>
-static F pick(const sx_config *cfg, F k2, F k4, F k4cm, F k8)
-{
-    const int n = cfg->dev.N;
-    return n <= 64 ? k2 : n <= 128 ? (cfg->compact_movers ? k4cm : k4) : k8;
-}
-
-static int fail(const char *who, cudaError_t e) { return sx_set_error(std::string(who) + ": " + cudaGetErrorString(e)); }
 
 }  // namespace sx
 
@@ -269,13 +234,9 @@ extern "C" int sx_expand_moves(const sx_config *cfg, sx_state st, int64_t num_en
     const expand_fn k = pick<expand_fn>(cfg, sx_expand_moves_kernel<2, false>, sx_expand_moves_kernel<4, false>,
                                         sx_expand_moves_kernel<4, true>, sx_expand_moves_kernel<8, false>);
     // as many blocks as are resident at once: every warp loops over many parents, which evens out their move counts
-    int device = 0, sms = 0, per_sm = 0;
-    cudaError_t e = cudaGetDevice(&device);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, EXPAND_WARPS * 32, smem);
+    unsigned grid = 0;
+    cudaError_t e = resident_grid(k, EXPAND_WARPS * 32, smem, (num_envs + EXPAND_WARPS - 1) / EXPAND_WARPS, grid);
     if (e != cudaSuccess) return fail("sx_expand_moves", e);
-    const long long blocks = (num_envs + EXPAND_WARPS - 1) / EXPAND_WARPS;
-    const unsigned grid = unsigned(std::max(1LL, std::min(blocks, (long long)std::max(1, per_sm) * sms)));
     k<<<grid, EXPAND_WARPS * 32, smem, static_cast<cudaStream_t>(stream)>>>(d, st.board, st.aux, st.captured, num_envs, offsets_d,
                                                                           n_children, out.board, out.aux, out.captured,
                                                                           actions_d, o, warp_bytes);

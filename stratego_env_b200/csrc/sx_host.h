@@ -36,3 +36,32 @@ struct sx_config {
 int sx_set_error(const std::string &msg);  // records the text sx_last_error() returns; always returns -1
 // true when p lies inside a live compressible allocation of sx_device_alloc (sx_alloc.cu)
 bool sx_in_compressible_allocation(const void *p);
+
+namespace sx {
+
+// the instantiation of a one-warp-per-game search kernel (sx_expand.cu, sx_playout.cu), as launch_policy
+// (sx_policy.cu) picks it: cells per lane by board size, compact movers where configured
+template <class F>
+inline F pick(const sx_config *cfg, F k2, F k4, F k4cm, F k8)
+{
+    const int n = cfg->dev.N;
+    return n <= 64 ? k2 : n <= 128 ? (cfg->compact_movers ? k4cm : k4) : k8;
+}
+
+inline int fail(const char *who, cudaError_t e) { return sx_set_error(std::string(who) + ": " + cudaGetErrorString(e)); }
+
+// the blocks of `threads` threads and `smem` bytes of shared memory that the current device holds at once, at most
+// `wanted`, at least 1
+template <class F>
+inline cudaError_t resident_grid(F kernel, int threads, size_t smem, long long wanted, unsigned &grid)
+{
+    int device = 0, sms = 0, per_sm = 0;
+    cudaError_t e = cudaGetDevice(&device);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
+    const long long most = (long long)(per_sm > 1 ? per_sm : 1) * sms;
+    grid = unsigned(wanted < 1 ? 1 : wanted < most ? wanted : most);
+    return e;
+}
+
+}  // namespace sx

@@ -64,6 +64,18 @@ class Expansion:
     player: torch.Tensor          # int8 [T] player to move in the child (+1 / -1)
 
 
+@dataclass
+class Playout:
+    """What StrategoEngine.playout reports per game of the batch (B rows each)."""
+    plies: torch.Tensor           # int32 [B] plies played in this call
+    reward: torch.Tensor          # float32 [B] player +1's reward if the game is over at the end, else 0
+    done: torch.Tensor            # uint8 [B] the game is over at the end of the call
+    winner: torch.Tensor          # int8 [B] +1 / -1, 0 for a draw by the turn limit or a game still running
+    ending_invalid: torch.Tensor  # uint8 [B] the game ended by the turn limit
+    illegal: torch.Tensor         # uint8 [B] 0, or 2 once the capture list has overflowed
+    player: torch.Tensor          # int8 [B] player to move at the end (+1 / -1)
+
+
 # observation element types (sx_config_desc::obs_dtype)
 OBS_DTYPES = {torch.float32: _lib.SX_DTYPE_F32, torch.bfloat16: _lib.SX_DTYPE_BF16, torch.float16: _lib.SX_DTYPE_F16}
 
@@ -383,13 +395,9 @@ class StrategoEngine:
                              "(not reachable by play)" % bad)
         return out
 
-    def expand_moves(self, state: DeviceState) -> "Expansion":
-        """The children of every game (sx_count_moves + sx_expand_moves): one per legal move of the player to move, in
-        ascending flat spatial index (that player's frame, the index step / step_all / sample_policy take).  Child j of
-        game b is row offsets[b] + j of every field and equals, byte for byte, what ``step`` (spatial actions, no flags)
-        makes of a copy of game b with action actions[row]: state rows and the reward, done, winner, ending_invalid,
-        illegal and player it returns.  A finished game or a stuck player has no children.  ``state`` is not written.
-        Reading the number of children back to size the outputs is ONE host synchronisation per call."""
+    def _check_state(self, state) -> None:
+        """ValueError unless ``state`` is a DeviceState of contiguous tensors in this engine's dtypes, strides and
+        device (checked on the host, before any device is touched)"""
         lay = self.layout
         if not isinstance(state, DeviceState):
             raise ValueError("state must be a DeviceState, not %s" % type(state).__name__)
@@ -402,6 +410,16 @@ class StrategoEngine:
                 raise ValueError("state.%s must be a contiguous %s tensor of shape (%d, %d) on %s, not %s" % (
                     name, dtype, B, width, self.device,
                     "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor) else type(t).__name__))
+
+    def expand_moves(self, state: DeviceState) -> "Expansion":
+        """The children of every game (sx_count_moves + sx_expand_moves): one per legal move of the player to move, in
+        ascending flat spatial index (that player's frame, the index step / step_all / sample_policy take).  Child j of
+        game b is row offsets[b] + j of every field and equals, byte for byte, what ``step`` (spatial actions, no flags)
+        makes of a copy of game b with action actions[row]: state rows and the reward, done, winner, ending_invalid,
+        illegal and player it returns.  A finished game or a stuck player has no children.  ``state`` is not written.
+        Reading the number of children back to size the outputs is ONE host synchronisation per call."""
+        self._check_state(state)
+        B = state.num_envs
         d = self.device
         counts = torch.empty(B, dtype=torch.int32, device=d)
         offsets = torch.zeros(B + 1, dtype=torch.int64, device=d)
@@ -418,6 +436,29 @@ class StrategoEngine:
                        "sx_expand_moves")
             parent = torch.repeat_interleave(torch.arange(B, device=d), counts, output_size=T)
         return Expansion(states=out, actions=actions, parent=parent, offsets=offsets, **scalars)
+
+    def playout(self, state: DeviceState, max_plies: Optional[int] = None, seed: int = 0, env_base: int = 0) -> "Playout":
+        """Random playouts (sx_playout): every game of ``state`` is played on, in place, with uniformly random legal
+        moves until it ends or ``max_plies`` plies have been played (None: to the end).  The move of each ply is the
+        draw ``step_all(..., sample_next=True, seed=seed, env_base=env_base)`` makes for the state before that ply, so a
+        playout of n plies equals, byte for byte, n such chained steps (without auto-reset) stopped at the first that
+        reports done, and continues the chain of a caller's last ``step_all`` with that seed.  A game over at entry plays
+        0 plies and is not written; a player to move without a legal move (only an imported state can be so) loses, as
+        with the noop action.  Returns the plies played and, per game, the reward, done, winner, ending_invalid, illegal
+        and player as the step that ended the game reported them.  No host synchronisation."""
+        if max_plies is not None and (isinstance(max_plies, bool) or not isinstance(max_plies, (int, np.integer))
+                                      or not 0 <= max_plies < 1 << 31):
+            raise ValueError("max_plies must be None or an integer in [0, 2^31), not %r" % (max_plies,))
+        self._check_state(state)
+        B = state.num_envs
+        d = self.device
+        plies = torch.empty(B, dtype=torch.int32, device=d)
+        scalars = self.alloc_outputs(B, partial=False, full=False, mask=False)
+        with torch.cuda.device(d):
+            _lib.check(self.lib.sx_playout(self._cfg, state.as_struct(), B, int(env_base),
+                                           (1 << 31) - 1 if max_plies is None else int(max_plies), seed & (2 ** 64 - 1),
+                                           plies.data_ptr(), self._outputs_struct(scalars), _stream()), "sx_playout")
+        return Playout(plies=plies, **scalars)
 
     def export_ref_state(self, state: DeviceState):
         B = state.num_envs
