@@ -321,6 +321,33 @@ int sx_expand_moves(const sx_config *cfg, sx_state st, int64_t num_envs, const i
 int sx_playout(const sx_config *cfg, sx_state st, int64_t num_envs, int64_t env_base, int32_t max_plies,
                uint64_t seed, int32_t *plies_d, sx_outputs out_scalars, void *stream);
 
+/* Position keys, for transposition tables and information-set search: keys_d[b] (uint64) identifies game b.
+ * SX_KEY_STATE: a key of the game as sx_export_ref_state exports it, the dense int64 [34][R][C] state plus the player to
+ * move.  Two states with equal exports have equal keys; what the export does not hold has no effect (the aux episode
+ * counter, board padding, the order of the capture-list entries, the overflow flag).  Two states whose exports differ
+ * get different keys except with probability about 2^-64 per pair: among n distinct states some pair collides with
+ * probability about n^2 / 2^65 (10^8 states: 3e-4).
+ * SX_KEY_INFOSET: the state key of the same export after one change, for the viewer viewer_d[b] (1 = player +1,
+ * anything else = player -1; NULL = the player to move, as sx_sample_hidden_states): on every HIDDEN cell of that call
+ * (a piece of the viewer's opponent, code 1..12, not CELL_REVEALED, on no obstacle) the opponent's true-rank layer
+ * (0 for player +1, 1 for player -1) holds the entry of its partially observable layer (3 / 4), UNKNOWN (13), instead
+ * of the rank; and one more feature names the viewer.  So every state sx_sample_hidden_states draws for a viewer has
+ * the information-set key of its source for that viewer, and a state's state key and its two information-set keys
+ * differ by construction.
+ * Construction (exact; no seed, no env_base, stable across calls and processes): Zobrist form, the XOR of
+ * Z(c, l, x) over every non-zero dense entry x at (layer l, cell c) of layers 0-1 and 3-33 (layer 2, the obstacles, is
+ * fixed by the configuration), plus Z(0, 34, player to move +1 / -1) and, for SX_KEY_INFOSET, Z(0, 35, viewer +1 / -1).
+ * Z(c, l, x) = w0 | w1 << 32 with (w0, w1) the first two words of Philox4x32-10, key (0x53545241, 0x5445474f), counter
+ * (c, l, (uint32_t)x, RNG_KEYS = 0x4b455953); c is the absolute cell index (the data layer: 0 turn, 1 over, 2 winner,
+ * C max_turns, C + 1 invalid).  Captured counters enter as the dense counts: the compact capture list holds at most one
+ * entry per (cell, owner, type), since a capture adds to an existing entry and sx_import_ref_state writes one entry per
+ * non-zero counter.  XOR allows incremental updates (old word out, new word in).
+ * Refused: a null config, state tensor or keys_d, an unknown mode, and a non-null viewer_d with SX_KEY_STATE.
+ * num_envs <= 0: nothing to do. */
+enum { SX_KEY_STATE = 0, SX_KEY_INFOSET = 1 };
+int sx_state_keys(const sx_config *cfg, sx_state st, int64_t num_envs, const int8_t *viewer_d, uint32_t mode,
+                  uint64_t *keys_d, void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

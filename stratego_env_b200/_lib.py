@@ -17,6 +17,7 @@ OBS_PO, OBS_FO, OBS_MASK = 1, 2, 4
 SX_CHANNELS_EXTENDED, SX_CHANNELS_ORIGINAL = 0, 1
 SX_DTYPE_F32, SX_DTYPE_BF16, SX_DTYPE_F16 = 0, 1, 2
 SX_ALLOC_COMPRESSIBLE = 1
+SX_KEY_STATE, SX_KEY_INFOSET = 0, 1
 
 
 class SxConfigDesc(C.Structure):
@@ -73,6 +74,7 @@ SYMBOLS = {
     "sx_count_moves": (C.c_int, [_vp, SxState, _i64, _vp, _vp]),
     "sx_expand_moves": (C.c_int, [_vp, SxState, _i64, _vp, _i64, SxState, _vp, SxOutputs, _vp]),
     "sx_playout": (C.c_int, [_vp, SxState, _i64, _i64, _i32, _u64, _vp, SxOutputs, _vp]),
+    "sx_state_keys": (C.c_int, [_vp, SxState, _i64, _vp, _u32, _vp, _vp]),
     "sx_step_all_launch_info": (C.c_int, [_vp, _u32, C.POINTER(SxLaunchInfo)]),
     "sx_device_alloc": (C.c_int, [_i32, _u64, _u32, C.POINTER(_vp), C.POINTER(_u32)]),
     "sx_device_free": (C.c_int, [_vp]),

@@ -250,6 +250,12 @@ class BatchedStrategoEnv:
         (``player``) are INTERNAL (+1 / -1), as for ``sample_hidden_states``.  One host synchronisation per call."""
         return self.engine.expand_moves(self.state)
 
+    def state_keys(self, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """64-bit keys of the current games (StrategoEngine.state_keys), int64 [num_envs]: of the position, or with
+        info_set=True of what the viewer knows.  viewer: None (the player to move) or an integer tensor [num_envs] of
+        INTERNAL player ids (+1 / -1), as for ``sample_hidden_states``."""
+        return self.engine.state_keys(self.state, info_set=info_set, viewer=viewer)
+
     # ---- checkpoint / interop in the reference's dense layout ---------------------------------------------
     def export_states(self):
         """(int64 [B, 34, R, C], int8 [B] player to move) -- the reference's state layout (impl:16-60)"""

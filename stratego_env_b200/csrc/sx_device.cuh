@@ -122,7 +122,8 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
     return c;
 }
 
-enum : uint32_t { RNG_RESET = 0x52535430u, RNG_SAMPLE = 0x53414d50u, RNG_SHUFFLE = 0x53484600u, RNG_HIDDEN = 0x48494444u };
+enum : uint32_t { RNG_RESET = 0x52535430u, RNG_SAMPLE = 0x53414d50u, RNG_SHUFFLE = 0x53484600u, RNG_HIDDEN = 0x48494444u,
+                  RNG_KEYS = 0x4b455953u };
 
 // ---- this warp's slice of shared memory -----------------------------------------------------------
 struct WarpMem {

@@ -377,9 +377,7 @@ class StrategoEngine:
             raise ValueError("n_samples must be an integer in [1, 2^24), not %r" % (n_samples,))
         B = state.num_envs
         if viewer is not None:
-            if not isinstance(viewer, torch.Tensor) or viewer.dtype not in self._VIEWER_DTYPES or tuple(viewer.shape) != (B,):
-                raise ValueError("viewer must be None or an integer tensor of shape (%d,), not %s" % (
-                    B, "%s %s" % (viewer.dtype, tuple(viewer.shape)) if isinstance(viewer, torch.Tensor) else type(viewer).__name__))
+            self._check_viewer(viewer, B)
             viewer = viewer.to(self.device, dtype=torch.int8).contiguous()
         n_samples = int(n_samples)
         out = self.alloc_state(B * n_samples)
@@ -394,6 +392,12 @@ class StrategoEngine:
             raise ValueError("game(s) %s hide more flags and bombs than unmoved pieces: no consistent placement exists "
                              "(not reachable by play)" % bad)
         return out
+
+    def _check_viewer(self, viewer, B: int) -> None:
+        """ValueError unless ``viewer`` is an integer tensor of shape (B,) (checked on the host)"""
+        if not isinstance(viewer, torch.Tensor) or viewer.dtype not in self._VIEWER_DTYPES or tuple(viewer.shape) != (B,):
+            raise ValueError("viewer must be None or an integer tensor of shape (%d,), not %s" % (
+                B, "%s %s" % (viewer.dtype, tuple(viewer.shape)) if isinstance(viewer, torch.Tensor) else type(viewer).__name__))
 
     def _check_state(self, state) -> None:
         """ValueError unless ``state`` is a DeviceState of contiguous tensors in this engine's dtypes, strides and
@@ -459,6 +463,34 @@ class StrategoEngine:
                                            (1 << 31) - 1 if max_plies is None else int(max_plies), seed & (2 ** 64 - 1),
                                            plies.data_ptr(), self._outputs_struct(scalars), _stream()), "sx_playout")
         return Playout(plies=plies, **scalars)
+
+    def state_keys(self, state: DeviceState, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """64-bit keys that identify positions (sx_state_keys), int64 [B]: the uint64 key bits viewed as int64, so that
+        ``torch.unique`` and ``torch.isin`` take them directly.
+        info_set=False: the key of each game as ``export_ref_state`` exports it (dense state and player to move).  Equal
+        exports give equal keys; the episode counter, board padding and the order of the capture list do not count.
+        Different exports collide with probability about 2^-64 per pair (n states: about n^2 / 2^65).
+        info_set=True: the key of what ``viewer`` knows: the same, but the opponent's unrevealed pieces count as UNKNOWN
+        whatever their true rank, and the viewer is part of the key.  viewer: None (the player to move) or an integer
+        tensor [B], 1 = player +1, anything else = player -1, as for ``sample_hidden_states``; every state that call
+        draws for a viewer has its source's information-set key for that viewer.
+        Keys depend on the position alone (no seed, no env_base), so tables can outlive a call and a process.  No host
+        synchronisation."""
+        self._check_state(state)
+        if not isinstance(info_set, bool):
+            raise ValueError("info_set must be True or False, not %r" % (info_set,))
+        B = state.num_envs
+        if viewer is not None:
+            if not info_set:
+                raise ValueError("viewer is only taken with info_set=True")
+            self._check_viewer(viewer, B)
+            viewer = viewer.to(self.device, dtype=torch.int8).contiguous()
+        keys = torch.empty(B, dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sx_state_keys(self._cfg, state.as_struct(), B, _ptr(viewer),
+                                              _lib.SX_KEY_INFOSET if info_set else _lib.SX_KEY_STATE, keys.data_ptr(),
+                                              _stream()), "sx_state_keys")
+        return keys
 
     def export_ref_state(self, state: DeviceState):
         B = state.num_envs
