@@ -348,6 +348,48 @@ enum { SX_KEY_STATE = 0, SX_KEY_INFOSET = 1 };
 int sx_state_keys(const sx_config *cfg, sx_state st, int64_t num_envs, const int8_t *viewer_d, uint32_t mode,
                   uint64_t *keys_d, void *stream);
 
+/* Monte Carlo tree search, a fixed number of iterations per root, every tree of the batch in one launch (one warp per
+ * tree).  Game b is the root of its own tree of at most max_nodes nodes; node 0 is the root.  The nodes are stored
+ * struct-of-arrays, each field int32 [num_envs, max_nodes] (node j of tree b at b * max_nodes + j):
+ *   visits N; value W, the sum of the evaluations in absolute terms (+1: player +1 won); parent (-1 for the root);
+ *   first_child (-1 while the node is not expanded); n_children; action, the flat spatial index of the move from the
+ *   parent to the node in the frame of the parent's player to move (the sx_expand_moves / sx_step index; -1 for the root).
+ * used (int32 [num_envs]) is the number of nodes allocated; entries at index used[b] and above are not written, and
+ * neither is st.
+ * Iteration i = 0 .. iterations - 1 of each tree:
+ *  1. Descent: s = the root state, v = the root, path = [root].  Repeat: if s is over, stop.  If v has no children: let
+ *     n be the number of legal moves of s's player to move; if n = 0 (a stuck player, only possible in an imported
+ *     root) or used + n > max_nodes, stop (v stays a leaf); otherwise allocate n children at used .. used + n - 1, in
+ *     ascending flat spatial index of their moves (the sx_expand_moves action list).  Choose a child c: the first child
+ *     (lowest index) with N = 0 if there is one, else the argmax of the score below, ties to the lowest index.  Set s =
+ *     the state after c's move (byte for byte what sx_step makes of s with that action), v = c, append c to the path;
+ *     if c had N = 0 before this iteration, stop.
+ *  2. Evaluation z in {-1, 0, +1}: if s is over, player +1's reward (the winner, 0 for a turn-limit ending); otherwise
+ *     a random playout from s of at most max_plies plies, with sx_playout's rules (a stuck player plays the noop and
+ *     loses) but the search's own draw: Philox4x32-10, key (seed lo, seed hi), counter (gid lo, gid hi,
+ *     RNG_SEARCH ^ i, turn & 0xffff of the state before the ply), RNG_SEARCH = 0x54524545, gid = env_base + b, first
+ *     output word w, move number __umulhi(w, n_moves) in ascending flat spatial index (sx_playout's numbering).  z is
+ *     player +1's reward at the end of the playout, 0 if the ply cap cut it off.
+ *  3. Backup: N += 1 and W += z on every node of the path.
+ * Score of child c of node v, with sigma = +1 if player +1 is to move in v's state and -1 otherwise (PUCT with a uniform
+ * prior), every operation float32, rounded to nearest, without FMA contraction:
+ *   q = float(sigma * W_c) / float(N_c);  u = (c_explore * sqrt(float(N_v))) / float(1 + N_c);  score = q + u
+ * with N_v and N_c the counts before this iteration's backup.  iterations <= 2^24 keeps every count and every |W| exact
+ * in float32, so numpy float32 reproduces every score bit for bit.
+ * Consequences: the tree depends only on (seed, gid, root state, iterations, max_nodes, max_plies, c_explore), not on the
+ * batch split or the other games; the root has N = iterations; an expanded non-root node has N = 1 + the sum of its
+ * children's N and an expanded root N = that sum; max_nodes = 1 makes the search `iterations` independent playouts of
+ * the root; iterations = 0 gives used = 1.  One tree is one warp: a batch with fewer trees than the device's resident
+ * warps leaves it partly idle.
+ * Refused: a null config, state tensor or tree pointer, iterations < 0 or > 2^24, max_nodes < 1, max_plies < 0, and a
+ * c_explore that is negative or not finite.  num_envs <= 0: nothing to do. */
+typedef struct {
+    int32_t *visits, *value, *parent, *first_child, *n_children, *action; /* [num_envs * max_nodes] */
+    int32_t *used;                                                          /* [num_envs] */
+} sx_tree;
+int sx_search(const sx_config *cfg, sx_state st, int64_t num_envs, int64_t env_base, int32_t iterations,
+              int32_t max_nodes, int32_t max_plies, float c_explore, uint64_t seed, sx_tree tree, void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

@@ -44,6 +44,10 @@ class SxOutputs(C.Structure):
                                    "terminal_full_obs")]
 
 
+class SxTree(C.Structure):
+    _fields_ = [(n, _vp) for n in ("visits", "value", "parent", "first_child", "n_children", "action", "used")]
+
+
 class SxLaunchInfo(C.Structure):
     _fields_ = [(n, _i32) for n in ("warps_per_block", "blocks_per_sm", "smem_bytes_per_block", "num_sms",
                                     "grid_blocks", "regs_per_thread", "background_bytes", "thread_per_game")]
@@ -75,6 +79,7 @@ SYMBOLS = {
     "sx_expand_moves": (C.c_int, [_vp, SxState, _i64, _vp, _i64, SxState, _vp, SxOutputs, _vp]),
     "sx_playout": (C.c_int, [_vp, SxState, _i64, _i64, _i32, _u64, _vp, SxOutputs, _vp]),
     "sx_state_keys": (C.c_int, [_vp, SxState, _i64, _vp, _u32, _vp, _vp]),
+    "sx_search": (C.c_int, [_vp, SxState, _i64, _i64, _i32, _i32, _i32, C.c_float, _u64, SxTree, _vp]),
     "sx_step_all_launch_info": (C.c_int, [_vp, _u32, C.POINTER(SxLaunchInfo)]),
     "sx_device_alloc": (C.c_int, [_i32, _u64, _u32, C.POINTER(_vp), C.POINTER(_u32)]),
     "sx_device_free": (C.c_int, [_vp]),

@@ -250,6 +250,14 @@ class BatchedStrategoEnv:
         (``player``) are INTERNAL (+1 / -1), as for ``sample_hidden_states``.  One host synchronisation per call."""
         return self.engine.expand_moves(self.state)
 
+    def search(self, iterations: int, seed: int = 0, max_nodes: Optional[int] = None, max_plies: Optional[int] = None,
+               c_explore: float = 1.0):
+        """Monte Carlo tree search from every current game (StrategoEngine.search), with this env's env_base: a
+        SearchTree with one tree per env.  Player ids in it (``root_player``, values in absolute terms) are INTERNAL
+        (+1 / -1).  The games are not changed.  No host synchronisation."""
+        return self.engine.search(self.state, iterations, max_nodes=max_nodes, max_plies=max_plies, c_explore=c_explore,
+                                  seed=seed, env_base=self.env_base)
+
     def state_keys(self, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
         """64-bit keys of the current games (StrategoEngine.state_keys), int64 [num_envs]: of the position, or with
         info_set=True of what the viewer knows.  viewer: None (the player to move) or an integer tensor [num_envs] of

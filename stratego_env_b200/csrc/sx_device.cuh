@@ -123,7 +123,7 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
 }
 
 enum : uint32_t { RNG_RESET = 0x52535430u, RNG_SAMPLE = 0x53414d50u, RNG_SHUFFLE = 0x53484600u, RNG_HIDDEN = 0x48494444u,
-                  RNG_KEYS = 0x4b455953u };
+                  RNG_KEYS = 0x4b455953u, RNG_SEARCH = 0x54524545u };
 
 // ---- this warp's slice of shared memory -----------------------------------------------------------
 struct WarpMem {

@@ -76,6 +76,38 @@ class Playout:
     player: torch.Tensor          # int8 [B] player to move at the end (+1 / -1)
 
 
+@dataclass
+class SearchTree:
+    """The trees StrategoEngine.search builds, one per game of the batch (sx_search).  Node j of tree b is column j of
+    the [B, max_nodes] fields; node 0 is the root.  Columns at used[b] and above are not written (they hold anything)."""
+    visits: torch.Tensor       # int32 [B, max_nodes] N
+    value: torch.Tensor        # int32 [B, max_nodes] W: the sum of the evaluations, +1 = player +1 won
+    parent: torch.Tensor       # int32 [B, max_nodes] -1 for the root
+    first_child: torch.Tensor  # int32 [B, max_nodes] -1 while the node is not expanded
+    n_children: torch.Tensor   # int32 [B, max_nodes]
+    action: torch.Tensor       # int32 [B, max_nodes] flat spatial index of the move from the parent (its player's frame)
+    used: torch.Tensor         # int32 [B] nodes allocated
+    root_player: torch.Tensor  # int8 [B] player to move at the root (+1 / -1)
+    mask_shape: tuple          # (R, C, A): the spatial valid-mask shape of one game
+
+    def root_stats(self):
+        """(visits, values) of the root's children, each int32 [B, R, C, A] shaped like the valid mask: at the entry of
+        each legal move of the root's player to move, its child's N and W, the value seen from the root's player to move
+        (+1 = that player won); zero elsewhere, and everywhere for a root that was never expanded.  Torch ops only (a
+        scatter over the nodes whose parent is the root), no host synchronisation."""
+        B, M = self.visits.shape
+        n = int(np.prod(self.mask_shape))
+        live = (self.parent == 0) & (torch.arange(M, device=self.visits.device)[None, :] < self.used[:, None].long())
+        idx = torch.where(live, self.action.long(), 0)
+        zero = torch.zeros((), dtype=torch.int32, device=self.visits.device)
+        sign = self.root_player.to(torch.int32)[:, None]
+        visits = torch.zeros(B, n, dtype=torch.int32, device=self.visits.device)
+        values = torch.zeros(B, n, dtype=torch.int32, device=self.visits.device)
+        visits.scatter_add_(1, idx, torch.where(live, self.visits, zero))
+        values.scatter_add_(1, idx, torch.where(live, self.value * sign, zero))
+        return visits.view(B, *self.mask_shape), values.view(B, *self.mask_shape)
+
+
 # observation element types (sx_config_desc::obs_dtype)
 OBS_DTYPES = {torch.float32: _lib.SX_DTYPE_F32, torch.bfloat16: _lib.SX_DTYPE_BF16, torch.float16: _lib.SX_DTYPE_F16}
 
@@ -463,6 +495,50 @@ class StrategoEngine:
                                            (1 << 31) - 1 if max_plies is None else int(max_plies), seed & (2 ** 64 - 1),
                                            plies.data_ptr(), self._outputs_struct(scalars), _stream()), "sx_playout")
         return Playout(plies=plies, **scalars)
+
+    @staticmethod
+    def _check_int(name, value, lo, hi, allow_none=False):
+        """ValueError unless ``value`` is an integer (not a bool) in [lo, hi] (or None where allowed)"""
+        if value is None and allow_none:
+            return
+        if isinstance(value, bool) or not isinstance(value, (int, np.integer)) or not lo <= value <= hi:
+            raise ValueError("%s must be %san integer in [%d, %d], not %r" % (
+                name, "None or " if allow_none else "", lo, hi, value))
+
+    def search(self, state: DeviceState, iterations: int, max_nodes: Optional[int] = None,
+               max_plies: Optional[int] = None, c_explore: float = 1.0, seed: int = 0, env_base: int = 0) -> "SearchTree":
+        """Monte Carlo tree search (sx_search), one tree per game of ``state`` with that game as its root, all in one
+        launch.  Each of the ``iterations`` iterations descends from the root (the first unvisited child, else the child
+        of best PUCT score with a uniform prior, q + c_explore * sqrt(N_parent) / (1 + N_child), q seen from the
+        player to move), expands a leaf into all its legal moves (ascending flat spatial index, the ``expand_moves``
+        action list) while the pool of ``max_nodes`` nodes has room, scores the state reached by its outcome or a random
+        playout of at most ``max_plies`` plies (None: to the end), and adds the score to N and W along the path.
+        max_nodes=None: 1 + 32 * iterations.  The tree depends only on (seed, env_base + b, the root, iterations,
+        max_nodes, max_plies, c_explore); ``state`` is not written.  Returns a SearchTree; ``root_stats()`` gives the
+        root children's visits and values in the valid-mask shape.  No host synchronisation."""
+        self._check_int("iterations", iterations, 0, 1 << 24)
+        if max_nodes is None and not isinstance(iterations, bool) and isinstance(iterations, (int, np.integer)):
+            max_nodes = 1 + 32 * int(iterations)
+        self._check_int("max_nodes", max_nodes, 1, (1 << 31) - 1)
+        self._check_int("max_plies", max_plies, 0, (1 << 31) - 1, allow_none=True)
+        with np.errstate(over="ignore"):
+            bad = (isinstance(c_explore, bool) or not isinstance(c_explore, (int, float, np.integer, np.floating))
+                   or not np.isfinite(np.float32(c_explore)) or not c_explore >= 0)
+        if bad:
+            raise ValueError("c_explore must be a finite number >= 0 (in float32), not %r" % (c_explore,))
+        self._check_state(state)
+        B, M = state.num_envs, int(max_nodes)
+        d = self.device
+        f = [torch.empty((B, M), dtype=torch.int32, device=d) for _ in range(6)]
+        used = torch.empty(B, dtype=torch.int32, device=d)
+        tree = _lib.SxTree(*(t.data_ptr() for t in f), used.data_ptr())
+        with torch.cuda.device(d):
+            _lib.check(self.lib.sx_search(self._cfg, state.as_struct(), B, int(env_base), int(iterations), M,
+                                          (1 << 31) - 1 if max_plies is None else int(max_plies), float(c_explore),
+                                          seed & (2 ** 64 - 1), tree, _stream()), "sx_search")
+            root_player = torch.where(((state.aux[:, 2] >> 4) & 1) == 0, 1, -1).to(torch.int8)  # aux_pack: to_move
+        return SearchTree(*f, used=used, root_player=root_player,
+                          mask_shape=(self.rows, self.columns, self.spatial_channels))
 
     def state_keys(self, state: DeviceState, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
         """64-bit keys that identify positions (sx_state_keys), int64 [B]: the uint64 key bits viewed as int64, so that
