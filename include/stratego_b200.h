@@ -390,6 +390,62 @@ typedef struct {
 int sx_search(const sx_config *cfg, sx_state st, int64_t num_envs, int64_t env_base, int32_t iterations,
               int32_t max_nodes, int32_t max_plies, float c_explore, uint64_t seed, sx_tree tree, void *stream);
 
+/* Guided tree search: PUCT selection and backup on the device, leaves evaluated by the caller (a policy prior and a
+ * value from a network, AlphaZero style).  A simulation is three steps, none of which synchronises the host and all of
+ * fixed shape (so they can run back to back or be captured in a CUDA graph):
+ *   sx_guided_select (one launch) -> the caller's network on the leaf states -> sx_guided_backup (one launch).
+ * Tree: game b is the root (node 0) of its own tree of at most max_nodes nodes, stored struct-of-arrays
+ * [num_envs, max_nodes] (node j of tree b at b * max_nodes + j), with sx_tree's fields and two differences: value W is
+ * float32, the sum of the values backed up in absolute terms (+1 = player +1 wins), and prior P (float32) is each
+ * node's prior under its parent.  An empty tree is the root alone: used = 1, N = 0, W = 0, parent = -1,
+ * first_child = -1, n_children = 0, action = -1, P = 1 in column 0; the caller writes it.  Columns at used[b] and above
+ * hold anything.  A caller may rewrite the priors of existing nodes between calls (Dirichlet noise on the root's
+ * children, say); nothing else in the tree is meant to be edited.
+ * sx_guided_select reads the roots st and the tree and writes neither.  For every tree it descends from the root: at a
+ * node v with children it takes the child c of highest score, ties to the lowest index, and steps into it (the state
+ * sx_step makes of v's state with c's action); it stops at the first node without children or whose state is over.
+ * Score, sigma = +1 if player +1 is to move at v and -1 otherwise, every operation float32, rounded to nearest, without
+ * FMA contraction:
+ *   q = N_c > 0 ? (sigma * W_c) / float(N_c) : fpu;  u = ((c_puct * P_c) * sqrt(float(N_v))) / float(1 + N_c);
+ *   score = q + u
+ * fpu is the value of an unvisited child from the mover's side.  Outputs per tree: leaf_states row b, the leaf's compact
+ * state, byte for byte what the chain of steps along the path makes of the root (ready for sx_observe,
+ * sx_valid_mask, sx_export_ref_state); leaf_node_d[b] (int32); leaf_kind_d[b] (int8, SX_LEAF_*): EVAL, the state is
+ * not over and its player to move has a move; OVER; STUCK, the player to move has no move (only an imported root).
+ * sx_guided_backup takes the leaves of the last select, logits_d [num_envs, R, C, A] (SX_DTYPE_F32 / BF16 / F16, the
+ * layout of sx_sample_policy: the player to move's frame) and values_d (float32 [num_envs], from the side of the leaf's
+ * player to move).  It needs no roots: the leaf's moves are regenerated from its leaf_states row.  For each tree:
+ *  - expansion: an EVAL leaf without children gets, if used + n <= max_nodes, its n legal moves as children at
+ *    used .. used + n - 1 in ascending flat spatial index (the sx_expand_moves list), with N = 0, W = 0,
+ *    first_child = -1, n_children = 0, and P = the softmax of the logits over the legal entries only (expf, a float32
+ *    sum, a correctly rounded division; a legal logit of -inf gets P = 0, and if every legal logit is -inf each child
+ *    gets 1/n; NaN or +inf logits are undefined); used grows by n;
+ *  - value z: EVAL sigma_leaf * values_d[b] (not clamped or checked); OVER player +1's reward (the winner, 0 for a
+ *    turn-limit ending); STUCK -sigma_leaf (the stuck player loses, as in sx_search and sx_playout);
+ *  - update: every node from the leaf to the root gets N += 1 and W += z (float32 add).
+ * Consequences: the tree depends only on (root, the logits and values given, max_nodes, c_puct, fpu): no RNG, no
+ * env_base, not the batch split; two selects without a backup between them return the same leaves; every expanded node,
+ * the root included, has N = 1 + the sum of its children's N; after r rounds the root has N = r; a pool too small for
+ * the next expansion stops the growth while values still back up.  The priors are the only transcendental result:
+ * given them, every selection is reproduced bit for bit by numpy float32.
+ * Refused: a null config, root state, tree field, leaf output, logits or values; leaf_states.board == st.board;
+ * max_nodes < 1; a c_puct that is negative or not finite; an fpu that is not finite; an unknown logits dtype.
+ * num_envs <= 0: nothing to do. */
+enum { SX_LEAF_EVAL = 0, SX_LEAF_OVER = 1, SX_LEAF_STUCK = 2 };
+typedef struct {
+    int32_t *visits;                                          /* [num_envs * max_nodes] N */
+    float *value;                                             /* W */
+    int32_t *parent, *first_child, *n_children, *action;
+    float *prior;                                             /* P */
+    int32_t *used;                                            /* [num_envs] */
+} sx_guided_tree;
+int sx_guided_select(const sx_config *cfg, sx_state st, int64_t num_envs, sx_guided_tree tree, int32_t max_nodes,
+                     float c_puct, float fpu, sx_state leaf_states, int32_t *leaf_node_d, int8_t *leaf_kind_d,
+                     void *stream);
+int sx_guided_backup(const sx_config *cfg, sx_state leaf_states, int64_t num_envs, sx_guided_tree tree,
+                     int32_t max_nodes, const int32_t *leaf_node_d, const int8_t *leaf_kind_d, const void *logits_d,
+                     int32_t logits_dtype, const float *values_d, void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

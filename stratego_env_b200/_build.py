@@ -5,7 +5,8 @@ import subprocess
 
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc")
 LIB_PATH = os.path.join(CSRC, "libstratego_b200.so")
-SOURCES = ["sx_kernels.cu", "sx_policy.cu", "sx_alloc.cu", "sx_hidden.cu", "sx_expand.cu", "sx_playout.cu", "sx_keys.cu", "sx_search.cu"]
+SOURCES = ["sx_kernels.cu", "sx_policy.cu", "sx_alloc.cu", "sx_hidden.cu", "sx_expand.cu", "sx_playout.cu", "sx_keys.cu", "sx_search.cu",
+           "sx_guided.cu"]
 HEADERS = ["sx_device.cuh", "sx_toy.cuh", os.path.join("..", "..", "include", "stratego_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

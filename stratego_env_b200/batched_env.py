@@ -28,7 +28,7 @@ import torch
 
 from . import sharding
 from .config import HUMAN_INIT_TABLE, VERSION_CONFIGS, as_version
-from .engine import DeviceState, Expansion, StrategoEngine, load_setup_table, obs_dtype_code
+from .engine import DeviceState, Expansion, Leaves, SearchTree, StrategoEngine, load_setup_table, obs_dtype_code
 from .enums import GameVersions, ObservationComponents, ObservationModes
 from .stratego_multiagent_env import DEFAULT_CONFIG, with_base_config
 
@@ -257,6 +257,15 @@ class BatchedStrategoEnv:
         (+1 / -1).  The games are not changed.  No host synchronisation."""
         return self.engine.search(self.state, iterations, max_nodes=max_nodes, max_plies=max_plies, c_explore=c_explore,
                                   seed=seed, env_base=self.env_base)
+
+    def guided_tree(self, max_nodes: int) -> SearchTree:
+        """An empty guided tree per current game (StrategoEngine.guided_tree)."""
+        return self.engine.guided_tree(self.state, max_nodes)
+
+    def guided_select(self, tree: SearchTree, c_puct: float = 1.25, fpu: float = 0.0) -> Leaves:
+        """One leaf per tree rooted at the current games (StrategoEngine.guided_select); back the evaluated leaves up
+        with ``self.engine.guided_backup``, which needs no roots."""
+        return self.engine.guided_select(self.state, tree, c_puct=c_puct, fpu=fpu)
 
     def state_keys(self, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
         """64-bit keys of the current games (StrategoEngine.state_keys), int64 [num_envs]: of the position, or with

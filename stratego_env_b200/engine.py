@@ -78,10 +78,11 @@ class Playout:
 
 @dataclass
 class SearchTree:
-    """The trees StrategoEngine.search builds, one per game of the batch (sx_search).  Node j of tree b is column j of
-    the [B, max_nodes] fields; node 0 is the root.  Columns at used[b] and above are not written (they hold anything)."""
+    """The trees StrategoEngine.search builds, one per game of the batch (sx_search), or the trees of a guided search
+    (StrategoEngine.guided_tree / guided_select / guided_backup).  Node j of tree b is column j of the [B, max_nodes]
+    fields; node 0 is the root.  Columns at used[b] and above are not written (they hold anything)."""
     visits: torch.Tensor       # int32 [B, max_nodes] N
-    value: torch.Tensor        # int32 [B, max_nodes] W: the sum of the evaluations, +1 = player +1 won
+    value: torch.Tensor        # int32 (search) / float32 (guided) [B, max_nodes] W: sum of the values, +1 = player +1 won
     parent: torch.Tensor       # int32 [B, max_nodes] -1 for the root
     first_child: torch.Tensor  # int32 [B, max_nodes] -1 while the node is not expanded
     n_children: torch.Tensor   # int32 [B, max_nodes]
@@ -89,24 +90,36 @@ class SearchTree:
     used: torch.Tensor         # int32 [B] nodes allocated
     root_player: torch.Tensor  # int8 [B] player to move at the root (+1 / -1)
     mask_shape: tuple          # (R, C, A): the spatial valid-mask shape of one game
+    prior: Optional[torch.Tensor] = None  # float32 [B, max_nodes] P, the prior under the parent (guided trees only)
 
     def root_stats(self):
-        """(visits, values) of the root's children, each int32 [B, R, C, A] shaped like the valid mask: at the entry of
-        each legal move of the root's player to move, its child's N and W, the value seen from the root's player to move
-        (+1 = that player won); zero elsewhere, and everywhere for a root that was never expanded.  Torch ops only (a
-        scatter over the nodes whose parent is the root), no host synchronisation."""
+        """(visits, values) of the root's children, shaped like the valid mask [B, R, C, A]: visits int32, values in the
+        dtype of ``value``.  At the entry of each legal move of the root's player to move, its child's N and W, the value
+        seen from the root's player to move (+1 = that player won); zero elsewhere, and everywhere for a root that was
+        never expanded.  Torch ops only (a scatter over the nodes whose parent is the root), no host synchronisation."""
         B, M = self.visits.shape
         n = int(np.prod(self.mask_shape))
         live = (self.parent == 0) & (torch.arange(M, device=self.visits.device)[None, :] < self.used[:, None].long())
         idx = torch.where(live, self.action.long(), 0)
         zero = torch.zeros((), dtype=torch.int32, device=self.visits.device)
-        sign = self.root_player.to(torch.int32)[:, None]
+        vzero = torch.zeros((), dtype=self.value.dtype, device=self.visits.device)
+        sign = self.root_player.to(self.value.dtype)[:, None]
         visits = torch.zeros(B, n, dtype=torch.int32, device=self.visits.device)
-        values = torch.zeros(B, n, dtype=torch.int32, device=self.visits.device)
+        values = torch.zeros(B, n, dtype=self.value.dtype, device=self.visits.device)
         visits.scatter_add_(1, idx, torch.where(live, self.visits, zero))
-        values.scatter_add_(1, idx, torch.where(live, self.value * sign, zero))
+        values.scatter_add_(1, idx, torch.where(live, self.value * sign, vzero))
         return visits.view(B, *self.mask_shape), values.view(B, *self.mask_shape)
 
+
+@dataclass
+class Leaves:
+    """The leaves StrategoEngine.guided_select picked, one per tree (B rows each)."""
+    states: DeviceState        # the leaf's state: byte for byte what the steps along its path make of the root
+    node: torch.Tensor         # int32 [B] the leaf's node index in its tree
+    kind: torch.Tensor         # int8 [B] LEAF_EVAL (to be evaluated), LEAF_OVER (game over) or LEAF_STUCK (no move)
+
+
+LEAF_EVAL, LEAF_OVER, LEAF_STUCK = _lib.SX_LEAF_EVAL, _lib.SX_LEAF_OVER, _lib.SX_LEAF_STUCK
 
 # observation element types (sx_config_desc::obs_dtype)
 OBS_DTYPES = {torch.float32: _lib.SX_DTYPE_F32, torch.bfloat16: _lib.SX_DTYPE_BF16, torch.float16: _lib.SX_DTYPE_F16}
@@ -505,6 +518,16 @@ class StrategoEngine:
             raise ValueError("%s must be %san integer in [%d, %d], not %r" % (
                 name, "None or " if allow_none else "", lo, hi, value))
 
+    @staticmethod
+    def _check_float(name, value, lo=None):
+        """ValueError unless ``value`` is a real number (not a bool) that is finite in float32 (and >= lo)"""
+        with np.errstate(over="ignore"):
+            bad = (isinstance(value, bool) or not isinstance(value, (int, float, np.integer, np.floating))
+                   or not np.isfinite(np.float32(value)) or (lo is not None and not value >= lo))
+        if bad:
+            raise ValueError("%s must be a finite number%s (in float32), not %r" % (
+                name, "" if lo is None else " >= %g" % lo, value))
+
     def search(self, state: DeviceState, iterations: int, max_nodes: Optional[int] = None,
                max_plies: Optional[int] = None, c_explore: float = 1.0, seed: int = 0, env_base: int = 0) -> "SearchTree":
         """Monte Carlo tree search (sx_search), one tree per game of ``state`` with that game as its root, all in one
@@ -521,11 +544,7 @@ class StrategoEngine:
             max_nodes = 1 + 32 * int(iterations)
         self._check_int("max_nodes", max_nodes, 1, (1 << 31) - 1)
         self._check_int("max_plies", max_plies, 0, (1 << 31) - 1, allow_none=True)
-        with np.errstate(over="ignore"):
-            bad = (isinstance(c_explore, bool) or not isinstance(c_explore, (int, float, np.integer, np.floating))
-                   or not np.isfinite(np.float32(c_explore)) or not c_explore >= 0)
-        if bad:
-            raise ValueError("c_explore must be a finite number >= 0 (in float32), not %r" % (c_explore,))
+        self._check_float("c_explore", c_explore, lo=0)
         self._check_state(state)
         B, M = state.num_envs, int(max_nodes)
         d = self.device
@@ -539,6 +558,103 @@ class StrategoEngine:
             root_player = torch.where(((state.aux[:, 2] >> 4) & 1) == 0, 1, -1).to(torch.int8)  # aux_pack: to_move
         return SearchTree(*f, used=used, root_player=root_player,
                           mask_shape=(self.rows, self.columns, self.spatial_channels))
+
+    # ---- guided search: PUCT select and backup on the device, leaves evaluated by the caller -------------------------
+    def guided_tree(self, roots: DeviceState, max_nodes: int) -> "SearchTree":
+        """An empty guided tree per game of ``roots`` (sx_guided_select / sx_guided_backup): the root alone, used = 1,
+        N = 0, W = 0, parent = first_child = -1, n_children = 0, action = -1, P = 1; ``value`` and ``prior`` are float32
+        [B, max_nodes], the other node fields int32.  Written with torch fills, no host synchronisation."""
+        self._check_int("max_nodes", max_nodes, 1, (1 << 31) - 1)
+        self._check_state(roots)
+        B, M, d = roots.num_envs, int(max_nodes), self.device
+        visits, parent, first_child, n_children, action = (torch.empty((B, M), dtype=torch.int32, device=d)
+                                                           for _ in range(5))
+        value, prior = (torch.empty((B, M), dtype=torch.float32, device=d) for _ in range(2))
+        for t, x in ((visits, 0), (value, 0.0), (parent, -1), (first_child, -1), (n_children, 0), (action, -1),
+                     (prior, 1.0)):
+            t[:, 0].fill_(x)
+        used = torch.ones(B, dtype=torch.int32, device=d)
+        root_player = torch.where(((roots.aux[:, 2] >> 4) & 1) == 0, 1, -1).to(torch.int8)  # aux_pack: to_move
+        return SearchTree(visits, value, parent, first_child, n_children, action, used=used, root_player=root_player,
+                          mask_shape=(self.rows, self.columns, self.spatial_channels), prior=prior)
+
+    def _check_guided_tree(self, tree, B: int) -> int:
+        """max_nodes of ``tree``; ValueError unless it is a guided SearchTree of B trees on this engine's device"""
+        if not isinstance(tree, SearchTree) or not isinstance(tree.prior, torch.Tensor):
+            raise ValueError("tree must be a SearchTree made by guided_tree, not %s" % type(tree).__name__)
+        M = tree.visits.shape[1] if isinstance(tree.visits, torch.Tensor) and tree.visits.dim() == 2 else -1
+        for name in ("visits", "value", "parent", "first_child", "n_children", "action", "prior", "used"):
+            t = getattr(tree, name)
+            dtype = torch.float32 if name in ("value", "prior") else torch.int32
+            shape = (B,) if name == "used" else (B, M)
+            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != shape or not t.is_contiguous()
+                    or t.device != self.device):
+                raise ValueError("tree.%s must be a contiguous %s tensor of shape %s on %s, not %s" % (
+                    name, dtype, shape, self.device,
+                    "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor) else type(t).__name__))
+        if M < 1:
+            raise ValueError("tree must have max_nodes >= 1, not %d" % M)
+        return M
+
+    def _guided_struct(self, tree) -> "_lib.SxGuidedTree":
+        return _lib.SxGuidedTree(*(getattr(tree, n).data_ptr() for n, _ in _lib.SxGuidedTree._fields_))
+
+    def guided_select(self, roots: DeviceState, tree: "SearchTree", c_puct: float = 1.25, fpu: float = 0.0) -> "Leaves":
+        """One leaf per tree (sx_guided_select): descend from the root of ``tree`` (the game of ``roots``) by the PUCT
+        score q + c_puct * P * sqrt(N_parent) / (1 + N), q = the mean value from the mover's side or ``fpu`` for an
+        unvisited child, ties to the lowest index, to the first node without children or whose state is over.  Returns
+        the leaves' states (ready for ``observe``, ``valid_mask``, ``export_ref_state``), node indices and kinds
+        (LEAF_EVAL, LEAF_OVER, LEAF_STUCK).  Neither ``roots`` nor ``tree`` is written, so two selects without a backup
+        between them return the same leaves.  No host synchronisation."""
+        self._check_state(roots)
+        B = roots.num_envs
+        M = self._check_guided_tree(tree, B)
+        self._check_float("c_puct", c_puct, lo=0)
+        self._check_float("fpu", fpu)
+        leaves = Leaves(self.alloc_state(B), torch.empty(B, dtype=torch.int32, device=self.device),
+                        torch.empty(B, dtype=torch.int8, device=self.device))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sx_guided_select(self._cfg, roots.as_struct(), B, self._guided_struct(tree), M,
+                                                 float(c_puct), float(fpu), leaves.states.as_struct(),
+                                                 leaves.node.data_ptr(), leaves.kind.data_ptr(), _stream()),
+                       "sx_guided_select")
+        return leaves
+
+    def guided_backup(self, tree: "SearchTree", leaves: "Leaves", logits: torch.Tensor, values: torch.Tensor) -> None:
+        """Expand and back up the leaves of the last ``guided_select`` (sx_guided_backup).  logits: float32, bfloat16 or
+        float16 [B, R, C, A] (or [B, R * C * A]) in the layout of ``sample_policy`` (the leaf's player-to-move frame);
+        values: float32 [B], the leaf's value from the side of its player to move.  An evaluable leaf without children
+        gets its legal moves as children (the ``expand_moves`` order) with the softmax of its logits over them as priors,
+        if the pool has room; then the leaf and its ancestors get N += 1 and W += the value in absolute terms (a finished
+        leaf's outcome, or a loss for a stuck player to move).  No host synchronisation."""
+        if not isinstance(leaves, Leaves):
+            raise ValueError("leaves must be the Leaves guided_select returned, not %s" % type(leaves).__name__)
+        self._check_state(leaves.states)
+        B = leaves.states.num_envs
+        M = self._check_guided_tree(tree, B)
+        for name, t, dtype in (("node", leaves.node, torch.int32), ("kind", leaves.kind, torch.int8)):
+            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != (B,) or not t.is_contiguous()
+                    or t.device != self.device):
+                raise ValueError("leaves.%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dtype, B,
+                                                                                                   self.device))
+        n = self.layout.spatial_actions
+        shapes = ((B,) + tuple(self.spatial_action_size), (B, n))
+        if (not isinstance(logits, torch.Tensor) or logits.dtype not in OBS_DTYPES or tuple(logits.shape) not in shapes
+                or not logits.is_contiguous() or logits.device != self.device):
+            raise ValueError("logits must be a contiguous float32 / bfloat16 / float16 tensor of shape %s or %s on %s, "
+                             "not %s" % (shapes[0], shapes[1], self.device, "%s %s on %s" % (
+                                 logits.dtype, tuple(logits.shape), logits.device)
+                                 if isinstance(logits, torch.Tensor) else type(logits).__name__))
+        if (not isinstance(values, torch.Tensor) or values.dtype != torch.float32 or tuple(values.shape) != (B,)
+                or not values.is_contiguous() or values.device != self.device):
+            raise ValueError("values must be a contiguous float32 tensor of shape (%d,) on %s, not %s" % (
+                B, self.device, "%s %s on %s" % (values.dtype, tuple(values.shape), values.device)
+                if isinstance(values, torch.Tensor) else type(values).__name__))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sx_guided_backup(self._cfg, leaves.states.as_struct(), B, self._guided_struct(tree), M,
+                                                 leaves.node.data_ptr(), leaves.kind.data_ptr(), logits.data_ptr(),
+                                                 OBS_DTYPES[logits.dtype], values.data_ptr(), _stream()),
+                       "sx_guided_backup")
 
     def state_keys(self, state: DeviceState, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
         """64-bit keys that identify positions (sx_state_keys), int64 [B]: the uint64 key bits viewed as int64, so that
