@@ -4,8 +4,9 @@ One tree per root, node 0 the root, fields as in include/stratego_b200.h, W and 
 root by the numpy float32 PUCT score (one rounding per operation, ties to the lowest index) to the first node without
 children or whose state is over; the step is the oracle's maenv:684-692 step (orc.apply_spatial_action).  backup()
 expands an evaluable leaf without children into the _expand_ref.action_list moves when the pool has room, with priors
-checked against the float64 softmax of the logits over the legal entries and then taken from the device (the only
-transcendental result), and adds the value to N and W (float32) along the path.  net() is a deterministic "network" of
+checked against the float64 softmax of the logits over the legal entries (within prior_bound) and then taken from the
+device (the only transcendental result), and adds the value to N and W (float32) along the path.  softmax_f32 emulates
+the kernel's float32 softmax, so that the bound can be checked without a device.  net() is a deterministic "network" of
 the dense state for the tests: logits are small multiples of 1/8 with ties and some -inf entries, the value a multiple
 of 1/16, so float32, bfloat16 and float16 hold them exactly."""
 import numpy as np
@@ -33,6 +34,28 @@ def net(dense, player, n_logits):
     return logits, value
 
 
+LOGIT_CASES = ("sigma1", "sigma4", "sigma10", "sigma30", "dominant", "extremes", "all_inf")
+
+
+def network_logits(rng, case, n, big):
+    """float32 [n]: logits of n legal moves as a policy head gives them.  sigmaS: N(0, S); dominant: one logit near 5,
+    the others more than 110 below it (their priors are exactly 0 in float32, also after rounding to bfloat16 / float16);
+    extremes: +-big (the dtype's largest finite value) mixed with N(0, 3); all_inf: every entry -inf"""
+    if case.startswith("sigma"):
+        return (rng.standard_normal(n) * float(case[5:])).astype(f32)
+    if case == "dominant":
+        x = 5 + rng.standard_normal() - 112 - np.abs(rng.standard_normal(n)) * 8
+        x[rng.integers(n)] = 5 + rng.standard_normal()
+        return x.astype(f32)
+    if case == "extremes":
+        x = rng.standard_normal(n) * 3
+        r = rng.random(n)
+        x[r < 0.15], x[(r >= 0.15) & (r < 0.3)] = big, -big
+        return x.astype(f32)
+    assert case == "all_inf", case
+    return np.full(n, -np.inf, f32)
+
+
 def scores(W, N, P, n_parent, sigma, c_puct, fpu):
     """numpy float32 PUCT scores of children (W, N, P) of a node with n_parent visits, as the kernel rounds them"""
     W, P = np.asarray(W, f32), np.asarray(P, f32)
@@ -52,15 +75,43 @@ def softmax64(x):
     return e / e.sum()
 
 
+def prior_bound(x):
+    """float64 [n]: how far each float32 prior of the legal logits x may lie from the float64 softmax w,
+    (n + 8 + |x - max|) * 2^-24 * w + 2^-146.  fl(x - max) is off by up to 2^-24 |x - max| absolute, which exp turns into
+    the same relative error; n + 8 covers the float32 sum, expf's 2 ulp and the division; 2^-146 covers priors that
+    round into or below the subnormal range.  An entry at -inf (w = 0) counts |x - max| as 0."""
+    x = np.asarray(x, np.float64)
+    w = softmax64(x)
+    y = np.abs(x - x.max()) if np.any(x > -np.inf) else np.zeros(x.size)
+    y = np.where(np.isfinite(y), y, 0.0)
+    return (x.size + 8 + y) * 2.0 ** -24 * w + 2.0 ** -146
+
+
 def check_priors(got, x):
-    """device priors of one child block against the float64 softmax: (n + 8) * 2^-24 relative each, sum 1 within
-    n * 2^-23"""
+    """device priors of one child block against the float64 softmax: each within prior_bound(x), the block's sum 1
+    within n * 2^-23"""
     got = np.asarray(got, f32)
     want = softmax64(x)
     n = want.size
     err = np.abs(got.astype(np.float64) - want)
-    assert np.all(err <= (n + 8) * 2.0 ** -24 * want), (got.tolist(), want.tolist())
+    assert np.all(err <= prior_bound(x)), (got.tolist(), want.tolist())
     assert abs(float(got.astype(np.float64).sum()) - 1.0) <= n * 2.0 ** -23, got.tolist()
+
+
+def softmax_f32(x, exp_ulps=None):
+    """the kernel's softmax of the legal logits x in numpy float32: fl(x - max), exp correctly rounded to float32 (then
+    scaled by 1 + exp_ulps * 2^-23 if given, to stand for expf's error), a float32 sum in ascending order and a float32
+    division; 1/n each when every entry is -inf"""
+    x = np.asarray(x, f32)
+    if not np.any(x > -np.inf):
+        return np.full(x.size, f32(1) / f32(x.size), f32)
+    with np.errstate(over="ignore"):
+        y = x - x.max()  # float32 -FLT_MAX - FLT_MAX overflows to -inf, as __fsub_rn does
+        e = np.exp(y.astype(np.float64)).astype(f32)
+    if exp_ulps is not None:
+        e = (e * (1 + np.asarray(exp_ulps, np.float64) * 2.0 ** -23)).astype(f32)
+    s = np.cumsum(e, dtype=f32)[-1]  # add.accumulate is sequential: one float32 rounding per term
+    return e / s
 
 
 class GuidedTree:
@@ -128,6 +179,11 @@ class GuidedTree:
             t["visits"][x] += 1
             t["value"][x] = f32(t["value"][x] + z)
             x = t["parent"][x]
+
+    def set_prior(self, first, values):
+        """the caller's rewrite of P of nodes first, first + 1, ... (float32), as on the device between calls"""
+        for k, val in enumerate(np.asarray(values, f32)):
+            self.t["prior"][first + k] = f32(val)
 
     def arrays(self):
         """dict of arrays [used] per field of FIELDS (W and P float32, the rest int64), and "used" """

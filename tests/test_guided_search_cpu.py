@@ -9,7 +9,8 @@ import torch
 
 from _expand_ref import action_list, logic
 from _golden import traj
-from _guided_ref import LEAF_EVAL, LEAF_OVER, GuidedTree, check_invariants, net, scores, softmax64
+from _guided_ref import (LEAF_EVAL, LEAF_OVER, LOGIT_CASES, GuidedTree, check_invariants, check_priors, net,
+                         network_logits, prior_bound, scores, softmax64, softmax_f32)
 from _playout_ref import OVER, data
 from test_expand_moves_cpu import _config, _fake_state, _no_device_engine, _state
 
@@ -94,6 +95,69 @@ def test_softmax_reference_edges():
     assert np.allclose(softmax64([-np.inf, -np.inf, -np.inf]), 1 / 3)
     p = softmax64([0.0, -np.inf, 0.0])
     assert p[1] == 0 and p[0] == p[2] == 0.5
+
+
+# ---- the prior bound, on a numpy float32 emulation of the kernel's softmax ------------------------------------------
+def _rounded(x, dtype):
+    """float32 logits after rounding to dtype, as the kernel reads them"""
+    return torch.from_numpy(np.ascontiguousarray(x)).to(dtype).float().numpy()
+
+
+def _blocks(case, dtype, count, seed):
+    """count child blocks of 1-120 legal logits of LOGIT_CASES case, rounded to dtype; a fifth of them with about 30 %
+    of the entries at -inf"""
+    rng = np.random.default_rng(seed)
+    big = float(torch.finfo(dtype).max)
+    for _ in range(count):
+        n = int(rng.integers(1, 121))
+        x = network_logits(rng, case, n, big)
+        if case != "all_inf" and rng.random() < 0.2:
+            hole = rng.random(n) < 0.3
+            if not hole.all():
+                x[hole] = -np.inf
+        yield _rounded(x, dtype), rng
+
+
+@pytest.mark.parametrize("case", LOGIT_CASES)
+@pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16, torch.float16], ids=["f32", "bf16", "f16"])
+def test_prior_bound_holds_for_the_kernels_arithmetic(case, dtype):
+    """float32 x - max, exp correctly rounded and then moved by up to 2 ulp (expf's error), a float32 sum and a float32
+    division stay within prior_bound, and every block sums to 1 within n * 2^-23"""
+    for x, rng in _blocks(case, dtype, 1500, 7):
+        check_priors(softmax_f32(x, rng.uniform(-2, 2, x.size)), x)
+
+
+def test_the_old_prior_bound_fails_on_ordinary_logits():
+    """(n + 8) * 2^-24 relative, without the |x - max| term, fails on N(0, 10) logits even with exp correctly rounded:
+    fl(x - max) alone is off by up to 2^-24 |x - max|, and exp keeps that as relative error.  prior_bound holds on the
+    same blocks."""
+    old = new = 0
+    for x, _ in _blocks("sigma10", torch.float32, 2000, 11):
+        p, w = softmax_f32(x).astype(np.float64), softmax64(x)
+        ok = w >= 2.0 ** -126  # normal priors only: below them the old bound, having no absolute term, fails anyway
+        old += bool(np.any((np.abs(p - w) > (x.size + 8) * 2.0 ** -24 * w) & ok))
+        new += bool(np.any(np.abs(p - w) > prior_bound(x)))
+    assert new == 0 and old >= 50, (old, new)  # 132 of the 2000 blocks break the old bound
+
+
+def test_prior_bound_edges():
+    """exact results the bound must allow: a single move, uniform -inf blocks, priors that underflow to 0"""
+    one = softmax_f32([3.25])
+    assert one[0] == 1 and prior_bound([3.25])[0] >= 2.0 ** -146
+    for n in (1, 3, 7, 100):
+        x = np.full(n, -np.inf, np.float32)
+        p = softmax_f32(x)
+        assert np.all(p == np.float32(1) / np.float32(n))
+        check_priors(p, x)
+    x = np.array([5, -107, -150, -np.inf], np.float32)
+    p = softmax_f32(x)
+    assert p[0] == 1 and np.all(p[1:] == 0)
+    check_priors(p, x)
+    big = np.finfo(np.float32).max
+    x = np.array([big, -big, 0, big], np.float32)
+    p = softmax_f32(x)
+    assert p[0] == p[3] == 0.5 and p[1] == p[2] == 0
+    check_priors(p, x)
 
 
 # ---- argument checks without a device -------------------------------------------------------------------------------

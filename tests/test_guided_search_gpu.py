@@ -2,7 +2,8 @@
 (seven node fields and used) against the reference of tests/_guided_ref.py on recorded states of every variant, with
 float32, bfloat16 and float16 logits; finished and stuck roots; pool exhaustion; the root's children against
 expand_moves; what select leaves alone; determinism and the batch split; no host synchronisation; a full-size batch
-with an evaluator on the device; the env forwarders."""
+with an evaluator on the device; the env forwarders.  _against_reference also serves
+tests/test_guided_search_edges_gpu.py, which brings its own networks."""
 import numpy as np
 import pytest
 import torch
@@ -36,9 +37,13 @@ def _same(got, want, what):
         assert bad.size == 0, (what, k, bad[:8].tolist(), g[bad[:4]].tolist(), w[bad[:4]].tolist())
 
 
-def _against_reference(e, version, dense, player, rows, rounds, max_nodes, c_puct=1.25, fpu=0.0, dtype=torch.float32):
+def _against_reference(e, version, dense, player, rows, rounds, max_nodes, c_puct=1.25, fpu=0.0, dtype=torch.float32,
+                       net_of=None, after_round=None, log=None):
     """grow trees from the imported states round by round, each round's leaves and the final trees against the
-    reference, the network being _guided_ref.net of each exported leaf state"""
+    reference.  The network is net_of(b, leaf state, player, n_logits) -> (float32 logits, value), by default
+    _guided_ref.net of the exported leaf state; the logits reach the device in `dtype` and the reference as the device
+    reads them (rounded to dtype).  after_round(r, tree, refs) runs after each round's backups; log (a list) receives
+    each round's (node, kind) arrays."""
     orc = logic(version)
     B = len(player)
     st = e.import_ref_state(torch.as_tensor(dense, device="cuda"),
@@ -47,12 +52,15 @@ def _against_reference(e, version, dense, player, rows, rounds, max_nodes, c_puc
     refs = [GuidedTree(orc, dense[b], int(player[b]), max_nodes) for b in range(B)]
     n = e.layout.spatial_actions
     kinds = np.zeros(3, np.int64)
+    if net_of is None:
+        net_of = lambda b, s, p, n_logits: net(s, p, n_logits)  # noqa: E731
     for r in range(rounds):
         leaves = e.guided_select(st, tree, c_puct=c_puct, fpu=fpu)
         ld, lp = (x.cpu().numpy() for x in e.export_ref_state(leaves.states))
         node, kind = leaves.node.cpu().numpy(), leaves.kind.cpu().numpy()
-        nets = [net(ld[b], int(lp[b]), n) for b in range(B)]
+        nets = [net_of(b, ld[b], int(lp[b]), n) for b in range(B)]
         logits = torch.as_tensor(np.stack([x for x, _ in nets])).to("cuda", dtype).view(B, *e.spatial_action_size)
+        seen = logits.float().view(B, n).cpu().numpy()
         values = torch.as_tensor(np.array([v for _, v in nets], np.float32), device="cuda")
         e.guided_backup(tree, leaves, logits, values)
         prior = tree.prior.cpu().numpy()
@@ -61,8 +69,12 @@ def _against_reference(e, version, dense, player, rows, rounds, max_nodes, c_puc
             what = (version, rows[b], r)
             assert (int(node[b]), int(kind[b])) == (v, k), (what, int(node[b]), int(kind[b]), v, k)
             assert np.array_equal(ld[b], s) and int(lp[b]) == p, what
-            refs[b].backup(v, s, p, k, nets[b][0], nets[b][1], prior[b])
+            refs[b].backup(v, s, p, k, seen[b], nets[b][1], prior[b])
             kinds[k] += 1
+        if log is not None:
+            log.append((node, kind))
+        if after_round is not None:
+            after_round(r, tree, refs)
     for b in range(B):
         want = refs[b].arrays()
         _same(_host(tree, b), want, (version, rows[b]))
