@@ -2,9 +2,11 @@
 
 At each of its turns the searcher, for every game in the batch at once:
 1. draws K complete worlds that agree with what it knows (sample_hidden_states, viewer = the player to move);
-2. grows one guided tree per world for --simulations rounds, every tree of every game in each launch:
+2. grows one guided tree per world for --simulations simulations, every tree of every game in each launch:
    guided_select (one leaf per tree) -> the evaluator on the leaves -> guided_backup (priors from the evaluator's
-   logits, its value backed up);
+   logits, its value backed up).  With --leaves-per-tree L > 1 a round selects L leaves per tree under a virtual loss:
+   one round of one leaf (in an empty tree every leaf would be the root), then ceil((simulations - 1) / L) rounds of
+   L, so the evaluator sees L times the rows in far fewer rounds;
 3. sums the root children's visit counts (root_stats) over the K worlds and plays the most visited move, ties to the
    lowest flat index.
 No step of a round synchronises the host.  Evaluators:
@@ -19,11 +21,12 @@ random opponent).  --opponent mcts plays player -1 with determinized_mcts's sear
 the same worlds and playout cap).
 
     python examples/guided_mcts.py [--games 256] [--worlds 16] [--simulations 128] [--rollout-plies 100]
-                                   [--evaluator rollout|conv] [--opponent random|mcts]
+                                   [--evaluator rollout|conv] [--opponent random|mcts] [--leaves-per-tree 1]
 
 With the defaults (rollout evaluator) the searcher won 250 and lost 6 of 256 games against the random player, in
 7.7 s, and won 139 and lost 117 of 256 against determinized MCTS, in 8.9 s, on a B200 at 1 000 W
-(profiles/r7f_examples.txt).
+(profiles/r7f_examples.txt).  With --leaves-per-tree 8 (129 simulations in 17 rounds) it won 137 and lost 119 against
+determinized MCTS with the search taking 2.2 s instead of 5.3 s, same card (profiles/r7h_examples.txt).
 """
 import argparse
 import os
@@ -48,16 +51,17 @@ class RolloutEvaluator:
 
     def __init__(self, e, plies, seed):
         self.e, self.plies, self.seed, self.calls = e, plies, seed, 0
-        self.logits = None
+        self.logits = {}  # rows -> zeros
 
     def __call__(self, leaves):
         B = leaves.node.shape[0]
-        if self.logits is None or self.logits.shape[0] != B:
-            self.logits = torch.zeros((B,) + tuple(self.e.spatial_action_size), dtype=torch.float32, device=self.e.device)
+        if B not in self.logits:
+            self.logits[B] = torch.zeros((B,) + tuple(self.e.spatial_action_size), dtype=torch.float32,
+                                         device=self.e.device)
         copy = leaves.states.clone()
         self.calls += 1
         res = self.e.playout(copy, max_plies=self.plies, seed=self.seed, env_base=self.calls * B)
-        return self.logits, res.reward * to_move_sign(leaves.states)
+        return self.logits[B], res.reward * to_move_sign(leaves.states)
 
 
 class ConvEvaluator:
@@ -74,28 +78,36 @@ class ConvEvaluator:
         self.value = torch.nn.Linear(channels, 1).to(e.device, dtype)
         for m in (self.trunk, self.policy):
             m.to(memory_format=torch.channels_last)
-        self.out = None
+        self.out = {}  # rows -> observation buffers
 
     @torch.no_grad()
     def __call__(self, leaves):
         B = leaves.node.shape[0]
-        if self.out is None or self.out["partial_obs"].shape[0] != B:
-            self.out = self.e.alloc_outputs(B, partial=True, full=False, mask=False)
-        obs = self.e.observe(leaves.states, out=self.out, partial=True, full=False, mask=False)["partial_obs"]
+        if B not in self.out:
+            self.out[B] = self.e.alloc_outputs(B, partial=True, full=False, mask=False)
+        obs = self.e.observe(leaves.states, out=self.out[B], partial=True, full=False, mask=False)["partial_obs"]
         h = self.trunk(obs.permute(0, 3, 1, 2).to(self.dtype))
         logits = self.policy(h).permute(0, 2, 3, 1).contiguous()
         values = torch.tanh(self.value(h.mean((2, 3)))).float().view(B)
         return logits, values
 
 
-def search(e, st, games, K, simulations, evaluator, seed, draw, c_puct=1.25):
+def schedule(simulations, leaves_per_tree):
+    """leaves per tree of each round: `simulations` rounds of one leaf, or with L > 1 one round of one leaf and then
+    ceil((simulations - 1) / L) rounds of L"""
+    L = leaves_per_tree
+    return [1] * simulations if L == 1 else [1] + [L] * -(-(simulations - 1) // L)
+
+
+def search(e, st, games, K, simulations, evaluator, seed, draw, c_puct=1.25, leaves_per_tree=1):
     """the searcher's move (flat spatial index, its own frame) in each game of `games` (all with the searcher to move)"""
     n = games.numel()
     sub = DeviceState(st.board[games], st.aux[games], st.captured[games])
     worlds = e.sample_hidden_states(sub, n_samples=K, seed=seed, draw=draw)  # row g * K + k: world k of game g
-    tree = e.guided_tree(worlds, 1 + 48 * simulations)
-    for _ in range(simulations):
-        leaves = e.guided_select(worlds, tree, c_puct=c_puct)
+    plan = schedule(simulations, leaves_per_tree)
+    tree = e.guided_tree(worlds, 1 + 48 * sum(plan))
+    for L in plan:
+        leaves = e.guided_select(worlds, tree, c_puct=c_puct, leaves_per_tree=L)
         logits, values = evaluator(leaves)
         e.guided_backup(tree, leaves, logits, values)
     visits, _ = tree.root_stats()
@@ -113,6 +125,7 @@ def main():
     ap.add_argument("--opponent", choices=("random", "mcts"), default="random")
     ap.add_argument("--mcts-iterations", type=int, default=128)
     ap.add_argument("--seed", type=int, default=1)
+    ap.add_argument("--leaves-per-tree", type=int, default=1)
     args = ap.parse_args()
     G, K = args.games, args.worlds
     if args.opponent == "mcts":
@@ -138,11 +151,12 @@ def main():
         if games.numel():
             torch.cuda.synchronize()
             ts = time.time()
-            actions[games] = search(e, st, games, K, args.simulations, evaluator, args.seed, ply)
+            actions[games] = search(e, st, games, K, args.simulations, evaluator, args.seed, ply,
+                                    leaves_per_tree=args.leaves_per_tree)
             torch.cuda.synchronize()
             t_search += time.time() - ts
             decisions += games.numel()
-            simulations += games.numel() * K * args.simulations
+            simulations += games.numel() * K * sum(schedule(args.simulations, args.leaves_per_tree))
         if args.opponent == "mcts":
             other = torch.nonzero((to_move == -1) & ~finished).flatten()
             if other.numel():
@@ -161,8 +175,11 @@ def main():
     opponent = ("uniform random" if args.opponent == "random" else
                 "determinized MCTS (%d worlds, %d iterations, %d-ply playouts)" % (K, args.mcts_iterations,
                                                                                    args.rollout_plies))
-    print("guided search, %s evaluator (%d worlds, %d simulations%s) vs %s, %d Barrage games, %d plies, %.1f s" % (
-        args.evaluator, K, args.simulations, ", %d-ply playouts" % args.rollout_plies if args.evaluator == "rollout"
+    plan = schedule(args.simulations, args.leaves_per_tree)
+    per_tree = ("%d simulations" % args.simulations if args.leaves_per_tree == 1 else
+                "%d simulations in %d rounds of up to %d leaves per tree" % (sum(plan), len(plan), args.leaves_per_tree))
+    print("guided search, %s evaluator (%d worlds, %s%s) vs %s, %d Barrage games, %d plies, %.1f s" % (
+        args.evaluator, K, per_tree, ", %d-ply playouts" % args.rollout_plies if args.evaluator == "rollout"
         else "", opponent, G, ply + 1, elapsed))
     print("searcher wins %d, losses %d, unfinished or turn limit %d; %d searcher decisions" % (
         wins, losses, G - wins - losses, decisions))

@@ -446,6 +446,42 @@ int sx_guided_backup(const sx_config *cfg, sx_state leaf_states, int64_t num_env
                      int32_t max_nodes, const int32_t *leaf_node_d, const int8_t *leaf_kind_d, const void *logits_d,
                      int32_t logits_dtype, const float *values_d, void *stream);
 
+/* Several leaves per tree in one round: L = leaves_per_tree leaves (1 <= L <= SX_GUIDED_MAX_LEAVES) under a virtual
+ * loss, so that the caller's network evaluates num_envs * L leaves at once and S simulations take S / L rounds.  L is
+ * chosen per call; different rounds may use different L.  num_envs counts trees; the leaf outputs have num_envs * L
+ * rows, leaf j of tree b at row b * L + j.
+ * sx_guided_select_many chooses the leaves of each tree in order j = 0 .. L-1, each a full descent from the root with
+ * sx_guided_select's stopping rule.  Before leaf j is chosen, every node on the paths of leaves 0 .. j-1 (root and leaf
+ * included) carries V = the number of those paths through it (all V are 0 for leaf 0), and the score of child c of v is
+ *   n_c = N_c + V_c;  q = n_c > 0 ? (sigma * W_c - vl * float(V_c)) / float(n_c) : fpu;
+ *   u = ((c_puct * P_c) * sqrt(float(N_v + V_v))) / float(1 + n_c);  score = q + u
+ * float32, one rounding per operation, no contraction, ties to the lowest index.  vl = virtual_loss (finite,
+ * 0 <= vl <= 2^24) is what each pending visit takes from the mover's value; vl = 0 is the "virtual visit" variant.
+ * With V = 0, vl * 0 = +0 and sigma * W - (+0) = sigma * W (-0 included), so L = 1 gives sx_guided_select's leaves bit for
+ * bit.  The pending visits live in inflight_d (int32 [num_envs * max_nodes], all zero before the call; it is all zero
+ * again when the call's work is done; unused and may be null when L = 1).  The tree's fields are not written: two selects
+ * without a backup return the same leaves.  Exactness needs N + V < 2^24 on every node.
+ * sx_guided_backup_many takes those num_envs * L leaves, logits_d [num_envs * L, R, C, A] and values_d
+ * [num_envs * L].  Per tree it processes the leaves in order j: an EVAL leaf whose node has no children at that point is
+ * expanded with row j's logits if the pool has room after the expansions of leaves 0 .. j-1; then leaf j's z is added
+ * along its path, as in sx_guided_backup.
+ * Consequences: a node reached by several leaves of one round is expanded once, by the first of them, and every one of
+ * them backs up its own value; the root gains N = L per round; every node has N = e + the sum of its children's N, e the
+ * number of selections that ended at it; the tree depends only on (root, the logits and values given, max_nodes, c_puct,
+ * fpu, vl, the L of each round), not on the batch split.  In the first round of an empty tree all L leaves are the root
+ * (correct but wasteful: open with one L = 1 round).  L = 1 calls are sx_guided_select / sx_guided_backup exactly.
+ * Refused: what sx_guided_select / sx_guided_backup refuse, L outside [1, SX_GUIDED_MAX_LEAVES], a virtual_loss that is
+ * negative, not finite or above 2^24 (the bound keeps vl * V and sigma * W - vl * V finite), and a null inflight_d with
+ * L > 1. */
+enum { SX_GUIDED_MAX_LEAVES = 1024 };
+int sx_guided_select_many(const sx_config *cfg, sx_state st, int64_t num_envs, sx_guided_tree tree, int32_t max_nodes,
+                          float c_puct, float fpu, int32_t leaves_per_tree, float virtual_loss, int32_t *inflight_d,
+                          sx_state leaf_states, int32_t *leaf_node_d, int8_t *leaf_kind_d, void *stream);
+int sx_guided_backup_many(const sx_config *cfg, sx_state leaf_states, int64_t num_envs, sx_guided_tree tree,
+                          int32_t max_nodes, int32_t leaves_per_tree, const int32_t *leaf_node_d,
+                          const int8_t *leaf_kind_d, const void *logits_d, int32_t logits_dtype, const float *values_d,
+                          void *stream);
+
 /* Kernel/launch facts for the benchmark's roofline accounting. */
 typedef struct {
     int32_t warps_per_block, blocks_per_sm, smem_bytes_per_block, num_sms, grid_blocks, regs_per_thread;

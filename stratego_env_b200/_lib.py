@@ -19,6 +19,7 @@ SX_DTYPE_F32, SX_DTYPE_BF16, SX_DTYPE_F16 = 0, 1, 2
 SX_ALLOC_COMPRESSIBLE = 1
 SX_KEY_STATE, SX_KEY_INFOSET = 0, 1
 SX_LEAF_EVAL, SX_LEAF_OVER, SX_LEAF_STUCK = 0, 1, 2
+SX_GUIDED_MAX_LEAVES = 1024
 
 
 class SxConfigDesc(C.Structure):
@@ -87,6 +88,9 @@ SYMBOLS = {
     "sx_search": (C.c_int, [_vp, SxState, _i64, _i64, _i32, _i32, _i32, C.c_float, _u64, SxTree, _vp]),
     "sx_guided_select": (C.c_int, [_vp, SxState, _i64, SxGuidedTree, _i32, C.c_float, C.c_float, SxState, _vp, _vp, _vp]),
     "sx_guided_backup": (C.c_int, [_vp, SxState, _i64, SxGuidedTree, _i32, _vp, _vp, _vp, _i32, _vp, _vp]),
+    "sx_guided_select_many": (C.c_int, [_vp, SxState, _i64, SxGuidedTree, _i32, C.c_float, C.c_float, _i32, C.c_float,
+                                        _vp, SxState, _vp, _vp, _vp]),
+    "sx_guided_backup_many": (C.c_int, [_vp, SxState, _i64, SxGuidedTree, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp]),
     "sx_step_all_launch_info": (C.c_int, [_vp, _u32, C.POINTER(SxLaunchInfo)]),
     "sx_device_alloc": (C.c_int, [_i32, _u64, _u32, C.POINTER(_vp), C.POINTER(_u32)]),
     "sx_device_free": (C.c_int, [_vp]),

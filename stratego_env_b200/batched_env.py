@@ -262,10 +262,12 @@ class BatchedStrategoEnv:
         """An empty guided tree per current game (StrategoEngine.guided_tree)."""
         return self.engine.guided_tree(self.state, max_nodes)
 
-    def guided_select(self, tree: SearchTree, c_puct: float = 1.25, fpu: float = 0.0) -> Leaves:
-        """One leaf per tree rooted at the current games (StrategoEngine.guided_select); back the evaluated leaves up
-        with ``self.engine.guided_backup``, which needs no roots."""
-        return self.engine.guided_select(self.state, tree, c_puct=c_puct, fpu=fpu)
+    def guided_select(self, tree: SearchTree, c_puct: float = 1.25, fpu: float = 0.0, leaves_per_tree: int = 1,
+                      virtual_loss: float = 1.0) -> Leaves:
+        """``leaves_per_tree`` leaves per tree rooted at the current games (StrategoEngine.guided_select); back the
+        evaluated leaves up with ``self.engine.guided_backup``, which needs no roots."""
+        return self.engine.guided_select(self.state, tree, c_puct=c_puct, fpu=fpu, leaves_per_tree=leaves_per_tree,
+                                         virtual_loss=virtual_loss)
 
     def state_keys(self, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
         """64-bit keys of the current games (StrategoEngine.state_keys), int64 [num_envs]: of the position, or with

@@ -16,6 +16,15 @@
 // index).  Backup regenerates the leaf's moves from its state row (gen_moves), gathers each lane's logits at
 // p * A + channel, and forms the softmax with a warp max, expf, a warp sum and a correctly rounded division; the children
 // are written at each lane's prefix-sum offset, and lane 0 walks the parent links.
+//
+// Several leaves per tree (sx_guided_select_many / sx_guided_backup_many): the same two kernels take L.  Select loops
+// over the L leaves inside the warp, each a replay from the root; after leaf j, lane 0 adds a pending visit along its
+// path in the per-node int32 buffer `inflight`, which the next descents read next to N, W and P (the virtual-loss
+// score), and before the warp ends it walks the L - 1 paths again and takes the visits back, so the buffer is zero
+// before and after every call.  Leaf 0 never reads the buffer and V = 0 leaves the score unchanged, so L = 1 is the
+// one-leaf select.  Backup takes the L leaves of its tree in order with the one-leaf code, so a node reached twice is
+// expanded by the first leaf.  One code path for every L: at L = 1 it is no slower than the one-leaf kernels were
+// (DESIGN.md §3.3), so there is no separate L = 1 instantiation.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -42,8 +51,8 @@ __device__ __forceinline__ float guided_logit(const void *row, int dtype, int i)
 template <int K, bool CM>
 __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_select_kernel(
     const __grid_constant__ DevConfig cfg, const uint8_t *board, const int16_t *aux, const uint16_t *cap,
-    long long num_envs, int max_nodes, float c_puct, float fpu, sx_guided_tree tree, uint8_t *leaf_board,
-    int16_t *leaf_aux, uint16_t *leaf_cap, int32_t *leaf_node, int8_t *leaf_kind, int warp_bytes)
+    long long num_envs, int max_nodes, float c_puct, float fpu, int L, float vl, int32_t *inflight, sx_guided_tree tree,
+    uint8_t *leaf_board, int16_t *leaf_aux, uint16_t *leaf_cap, int32_t *leaf_node, int8_t *leaf_kind, int warp_bytes)
 {
     using GT = Grp<1>;
     extern __shared__ __align__(16) uint8_t smem[];
@@ -55,68 +64,84 @@ __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_select_kernel(
     const long long row = b * (long long)max_nodes;
     const int32_t *const N = tree.visits + row, *const first_child = tree.first_child + row;
     const int32_t *const n_children = tree.n_children + row, *const action = tree.action + row;
+    const int32_t *const parent = tree.parent + row;
     const float *const W = tree.value + row, *const P = tree.prior + row;
-    Aux a;
-    unpack(load_game(cfg, board, aux, cap, b, m.board, m.cap), a);
-    __syncwarp();
-    // ---- descent: v and the state after its path; `fresh`: m.moves holds the moves of the state's player to move
-    int v = 0;
-    bool fresh = false, any = false;
-    for (;;) {
-        if (a.over) break;
-        const int f = first_child[v], n = n_children[v];
-        if (f < 0 || n <= 0) break;
-        // the argmax of q + u over the children, 32 per pass (lowest index on a tie)
-        const float sqrt_nv = __fsqrt_rn(float(N[v]));
-        const bool plus = a.to_move == 0;
-        float best = 0.0f;
-        int best_j = -1;
-        for (int j0 = 0; j0 < n; j0 += 32) {
-            const int j = j0 + lane;
-            if (j < n) {
-                const int nc = N[f + j];
-                const float wc = W[f + j], pc = P[f + j];
-                const float q = nc > 0 ? __fdiv_rn(plus ? wc : -wc, float(nc)) : fpu;
-                const float u = __fdiv_rn(__fmul_rn(__fmul_rn(c_puct, pc), sqrt_nv), float(1 + nc));
-                const float s = __fadd_rn(q, u);
-                if (best_j < 0 || s > best) { best = s; best_j = j; }  // j ascends: ties keep the lower index
+    int32_t *const V = inflight + row;  // pending visits of this round's earlier leaves; read from leaf 1 on
+#pragma unroll 1
+    for (int j = 0; j < L; ++j) {
+        const long long r = b * L + j;  // the leaf's output row
+        const bool pend = j > 0;        // pending visits exist from leaf 1 on
+        Aux a;
+        unpack(load_game(cfg, board, aux, cap, b, m.board, m.cap), a);
+        __syncwarp();
+        // ---- descent: v and the state after its path; `fresh`: m.moves holds the moves of the state's player to move
+        int v = 0;
+        bool fresh = false, any = false;
+        for (;;) {
+            if (a.over) break;
+            const int f = first_child[v], n = n_children[v];
+            if (f < 0 || n <= 0) break;
+            // the argmax of q + u over the children, 32 per pass (lowest index on a tie); with V = 0 (leaf 0, and
+            // nodes off the earlier paths) vl * 0 = +0 and sigma * W - (+0) = sigma * W, so this is the one-leaf score
+            const float sqrt_nv = __fsqrt_rn(float(N[v] + (pend ? V[v] : 0)));
+            const bool plus = a.to_move == 0;
+            float best = 0.0f;
+            int best_j = -1;
+            for (int c0 = 0; c0 < n; c0 += 32) {
+                const int c = c0 + lane;
+                if (c < n) {
+                    const int vc = pend ? V[f + c] : 0, nc = N[f + c] + vc;
+                    const float wc = W[f + c], pc = P[f + c];
+                    const float sw = __fsub_rn(plus ? wc : -wc, __fmul_rn(vl, float(vc)));  // sigma W - vl V
+                    const float q = nc > 0 ? __fdiv_rn(sw, float(nc)) : fpu;
+                    const float u = __fdiv_rn(__fmul_rn(__fmul_rn(c_puct, pc), sqrt_nv), float(1 + nc));
+                    const float s = __fadd_rn(q, u);
+                    if (best_j < 0 || s > best) { best = s; best_j = c; }  // c ascends: ties keep the lower index
+                }
             }
-        }
 #pragma unroll
-        for (int d = 16; d >= 1; d >>= 1) {
-            const float ob = __shfl_xor_sync(FULL, best, d);
-            const int oj = __shfl_xor_sync(FULL, best_j, d);
-            if (oj >= 0 && (best_j < 0 || ob > best || (ob == best && oj < best_j))) { best = ob; best_j = oj; }
+            for (int d = 16; d >= 1; d >>= 1) {
+                const float ob = __shfl_xor_sync(FULL, best, d);
+                const int oj = __shfl_xor_sync(FULL, best_j, d);
+                if (oj >= 0 && (best_j < 0 || ob > best || (ob == best && oj < best_j))) { best = ob; best_j = oj; }
+            }
+            // ---- step to the child: what expand_moves / sx_step make of the state with that action
+            const int mover = a.to_move;
+            int attack;
+            apply_move<GT>(cfg, m, a, decode_spatial(cfg, action[f + best_j], mover), false, attack);
+            any = after_move<K, GT, CM>(cfg, m, a, mover);
+            fresh = true;
+            v = f + best_j;
         }
-        // ---- step to the child: what expand_moves / sx_step make of the state with that action
-        const int mover = a.to_move;
-        int attack;
-        apply_move<GT>(cfg, m, a, decode_spatial(cfg, action[f + best_j], mover), false, attack);
-        any = after_move<K, GT, CM>(cfg, m, a, mover);
-        fresh = true;
-        v = f + best_j;
+        if (!a.over && !fresh) any = gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
+        __syncwarp();
+        // ---- the leaf's state row, as sx_playout writes a game back
+        const int board_words = cfg.board_stride >> 2, cap_words = cfg.cap_stride >> 1;
+        uint32_t *gb = reinterpret_cast<uint32_t *>(leaf_board + r * cfg.board_stride);
+        for (int w = lane; w < board_words; w += 32) gb[w] = reinterpret_cast<const uint32_t *>(m.board)[w];
+        uint32_t *gc = reinterpret_cast<uint32_t *>(leaf_cap + r * cfg.cap_stride);
+        for (int w = lane; w < cap_words; w += 32) gc[w] = reinterpret_cast<const uint32_t *>(m.cap)[w];
+        if (lane == 0) {
+            uint32_t w4[4];
+            aux_pack(a, w4);
+            *reinterpret_cast<uint4 *>(leaf_aux + r * 8) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+            leaf_node[r] = v;
+            leaf_kind[r] = int8_t(a.over ? SX_LEAF_OVER : any ? SX_LEAF_EVAL : SX_LEAF_STUCK);
+            if (j < L - 1)  // a pending visit on the path, for the leaves after this one
+                for (int x = v; x >= 0; x = parent[x]) V[x] += 1;
+        }
+        __syncwarp();  // the pending visits and the shared slice are the whole warp's before the next descent
     }
-    if (!a.over && !fresh) any = gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
-    __syncwarp();
-    // ---- the leaf's state row, as sx_playout writes a game back
-    const int board_words = cfg.board_stride >> 2, cap_words = cfg.cap_stride >> 1;
-    uint32_t *gb = reinterpret_cast<uint32_t *>(leaf_board + b * cfg.board_stride);
-    for (int w = lane; w < board_words; w += 32) gb[w] = reinterpret_cast<const uint32_t *>(m.board)[w];
-    uint32_t *gc = reinterpret_cast<uint32_t *>(leaf_cap + b * cfg.cap_stride);
-    for (int w = lane; w < cap_words; w += 32) gc[w] = reinterpret_cast<const uint32_t *>(m.cap)[w];
-    if (lane == 0) {
-        uint32_t w4[4];
-        aux_pack(a, w4);
-        *reinterpret_cast<uint4 *>(leaf_aux + b * 8) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-        leaf_node[b] = v;
-        leaf_kind[b] = int8_t(a.over ? SX_LEAF_OVER : any ? SX_LEAF_EVAL : SX_LEAF_STUCK);
-    }
+    // ---- take the pending visits back: the buffer is all zero again
+    if (lane == 0)
+        for (int j = 0; j < L - 1; ++j)
+            for (int x = leaf_node[b * L + j]; x >= 0; x = parent[x]) V[x] -= 1;
 }
 
 template <int K, bool CM>
 __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_backup_kernel(
     const __grid_constant__ DevConfig cfg, const uint8_t *leaf_board, const int16_t *leaf_aux, const uint16_t *leaf_cap,
-    long long num_envs, int max_nodes, sx_guided_tree tree, const int32_t *leaf_node, const int8_t *leaf_kind,
+    long long num_envs, int max_nodes, int L, sx_guided_tree tree, const int32_t *leaf_node, const int8_t *leaf_kind,
     const uint8_t *logits, int dtype, int logit_bytes, const float *values, int warp_bytes)
 {
     using GT = Grp<1>;
@@ -128,54 +153,45 @@ __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_backup_kernel(
     int32_t *const N = tree.visits + row, *const parent = tree.parent + row, *const first_child = tree.first_child + row;
     int32_t *const n_children = tree.n_children + row, *const action = tree.action + row;
     float *const W = tree.value + row, *const P = tree.prior + row;
-    const int v = leaf_node[b], kind = leaf_kind[b];
-    Aux a;
-    unpack(*reinterpret_cast<const uint4 *>(leaf_aux + b * 8), a);
-    // z: the value backed up, in absolute terms (+1 = player +1 wins)
-    const float z = kind == SX_LEAF_EVAL ? (a.to_move == 0 ? values[b] : -values[b])
-                  : kind == SX_LEAF_OVER ? float(a.over && !a.invalid ? a.winner : 0)
-                                         : (a.to_move == 0 ? -1.0f : 1.0f);  // STUCK: the player to move loses
-    int used = tree.used[b], f = -1, n = 0;
-    if (kind == SX_LEAF_EVAL && first_child[v] < 0) {
-        WarpMem m;
-        carve_warp(cfg, smem + size_t(warp) * warp_bytes, &m);
-        load_game(cfg, leaf_board, leaf_aux, leaf_cap, b, m.board, m.cap);
-        __syncwarp();
-        gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
-        // this lane's moves (its K cells) and their place in the ascending list
-        int mine = 0;
+    int used = tree.used[b];
+    // the leaves in order: leaf j sees the expansions of leaves 0 .. j-1, so a node reached by several is expanded once
 #pragma unroll 1
-        for (int k = 0; k < K; ++k) {
-            const int p = lane * K + k;
-            if (p < cfg.N) mine += __popc(m.moves[p].x) + __popc(m.moves[p].y);
-        }
-        int incl = mine;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const int x = __shfl_up_sync(FULL, incl, d);
-            if (lane >= d) incl += x;
-        }
-        const int total = __shfl_sync(FULL, incl, 31);
-        if (total > 0 && total <= max_nodes - used) {
-            f = used;
-            n = total;
-            const uint8_t *lrow = logits + b * (long long)(cfg.N * cfg.A) * logit_bytes;
-            // softmax over the legal entries: max, then sum of expf(x - max), both reduced over the warp
-            float mx = -INFINITY;
+    for (int j = 0; j < L; ++j) {
+        const long long r = b * L + j;  // the leaf's row
+        const int v = leaf_node[r], kind = leaf_kind[r];
+        Aux a;
+        unpack(*reinterpret_cast<const uint4 *>(leaf_aux + r * 8), a);
+        // z: the value backed up, in absolute terms (+1 = player +1 wins)
+        const float z = kind == SX_LEAF_EVAL ? (a.to_move == 0 ? values[r] : -values[r])
+                      : kind == SX_LEAF_OVER ? float(a.over && !a.invalid ? a.winner : 0)
+                                             : (a.to_move == 0 ? -1.0f : 1.0f);  // STUCK: the player to move loses
+        int f = -1, n = 0;
+        if (kind == SX_LEAF_EVAL && first_child[v] < 0) {
+            WarpMem m;
+            carve_warp(cfg, smem + size_t(warp) * warp_bytes, &m);
+            load_game(cfg, leaf_board, leaf_aux, leaf_cap, r, m.board, m.cap);
+            __syncwarp();
+            gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
+            // this lane's moves (its K cells) and their place in the ascending list
+            int mine = 0;
 #pragma unroll 1
             for (int k = 0; k < K; ++k) {
                 const int p = lane * K + k;
-                if (p >= cfg.N) break;
-#pragma unroll 1
-                for (int h = 0; h < 2; ++h)
-                    for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1)
-                        mx = fmaxf(mx, guided_logit(lrow, dtype, p * cfg.A + h * 32 + __ffs(w) - 1));
+                if (p < cfg.N) mine += __popc(m.moves[p].x) + __popc(m.moves[p].y);
             }
+            int incl = mine;
 #pragma unroll
-            for (int d = 16; d >= 1; d >>= 1) mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, d));
-            const bool uniform = !(mx > -INFINITY);  // every legal logit is -inf: each child gets 1 / n
-            float sum = 0.0f;
-            if (!uniform) {
+            for (int d = 1; d < 32; d <<= 1) {
+                const int x = __shfl_up_sync(FULL, incl, d);
+                if (lane >= d) incl += x;
+            }
+            const int total = __shfl_sync(FULL, incl, 31);
+            if (total > 0 && total <= max_nodes - used) {
+                f = used;
+                n = total;
+                const uint8_t *lrow = logits + r * (long long)(cfg.N * cfg.A) * logit_bytes;
+                // softmax over the legal entries: max, then sum of expf(x - max), both reduced over the warp
+                float mx = -INFINITY;
 #pragma unroll 1
                 for (int k = 0; k < K; ++k) {
                     const int p = lane * K + k;
@@ -183,38 +199,57 @@ __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_backup_kernel(
 #pragma unroll 1
                     for (int h = 0; h < 2; ++h)
                         for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1)
-                            sum = __fadd_rn(sum, expf(__fsub_rn(guided_logit(lrow, dtype, p * cfg.A + h * 32 + __ffs(w) - 1), mx)));
+                            mx = fmaxf(mx, guided_logit(lrow, dtype, p * cfg.A + h * 32 + __ffs(w) - 1));
                 }
 #pragma unroll
-                for (int d = 16; d >= 1; d >>= 1) sum = __fadd_rn(sum, __shfl_xor_sync(FULL, sum, d));  // same on every lane
-            }
-            int t = f + incl - mine;
+                for (int d = 16; d >= 1; d >>= 1) mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, d));
+                const bool uniform = !(mx > -INFINITY);  // every legal logit is -inf: each child gets 1 / n
+                float sum = 0.0f;
+                if (!uniform) {
 #pragma unroll 1
-            for (int k = 0; k < K; ++k) {
-                const int p = lane * K + k;
-                if (p >= cfg.N) break;
+                    for (int k = 0; k < K; ++k) {
+                        const int p = lane * K + k;
+                        if (p >= cfg.N) break;
 #pragma unroll 1
-                for (int h = 0; h < 2; ++h) {
-                    for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1) {
-                        const int c = t++, act = p * cfg.A + h * 32 + __ffs(w) - 1;
-                        N[c] = 0; W[c] = 0.0f; parent[c] = v; first_child[c] = -1; n_children[c] = 0; action[c] = act;
-                        P[c] = uniform ? __fdiv_rn(1.0f, float(n))
-                                       : __fdiv_rn(expf(__fsub_rn(guided_logit(lrow, dtype, act), mx)), sum);
+                        for (int h = 0; h < 2; ++h)
+                            for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1)
+                                sum = __fadd_rn(sum, expf(__fsub_rn(guided_logit(lrow, dtype, p * cfg.A + h * 32 + __ffs(w) - 1), mx)));
+                    }
+#pragma unroll
+                    for (int d = 16; d >= 1; d >>= 1) sum = __fadd_rn(sum, __shfl_xor_sync(FULL, sum, d));  // same on every lane
+                }
+                int t = f + incl - mine;
+#pragma unroll 1
+                for (int k = 0; k < K; ++k) {
+                    const int p = lane * K + k;
+                    if (p >= cfg.N) break;
+#pragma unroll 1
+                    for (int h = 0; h < 2; ++h) {
+                        for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1) {
+                            const int c = t++, act = p * cfg.A + h * 32 + __ffs(w) - 1;
+                            N[c] = 0; W[c] = 0.0f; parent[c] = v; first_child[c] = -1; n_children[c] = 0; action[c] = act;
+                            P[c] = uniform ? __fdiv_rn(1.0f, float(n))
+                                           : __fdiv_rn(expf(__fsub_rn(guided_logit(lrow, dtype, act), mx)), sum);
+                        }
                     }
                 }
             }
         }
+        // ---- backup: the leaf and its ancestors
+        if (lane == 0) {
+            if (n > 0) { first_child[v] = f; n_children[v] = n; }
+            for (int x = v; x >= 0; x = parent[x]) { N[x] += 1; W[x] = __fadd_rn(W[x], z); }
+        }
+        used += n;
+        __syncwarp();  // lane 0's links are the whole warp's before the next leaf reads them
     }
-    // ---- backup: the leaf and its ancestors
-    if (lane == 0) {
-        if (n > 0) { first_child[v] = f; n_children[v] = n; tree.used[b] = used + n; }
-        for (int x = v; x >= 0; x = parent[x]) { N[x] += 1; W[x] = __fadd_rn(W[x], z); }
-    }
+    if (lane == 0 && used != tree.used[b]) tree.used[b] = used;
 }
 
 typedef void (*guided_select_fn)(DevConfig, const uint8_t *, const int16_t *, const uint16_t *, long long, int, float,
-                                 float, sx_guided_tree, uint8_t *, int16_t *, uint16_t *, int32_t *, int8_t *, int);
-typedef void (*guided_backup_fn)(DevConfig, const uint8_t *, const int16_t *, const uint16_t *, long long, int,
+                                 float, int, float, int32_t *, sx_guided_tree, uint8_t *, int16_t *, uint16_t *, int32_t *,
+                                 int8_t *, int);
+typedef void (*guided_backup_fn)(DevConfig, const uint8_t *, const int16_t *, const uint16_t *, long long, int, int,
                                  sx_guided_tree, const int32_t *, const int8_t *, const uint8_t *, int, int, const float *,
                                  int);
 
@@ -223,24 +258,28 @@ static bool null_tree(const sx_guided_tree &t)
     return !t.visits || !t.value || !t.parent || !t.first_child || !t.n_children || !t.action || !t.prior || !t.used;
 }
 
-}  // namespace sx
+static std::string fn_error(const char *fn, const std::string &what) { return std::string(fn) + ": " + what; }
 
-extern "C" int sx_guided_select(const sx_config *cfg, sx_state st, int64_t num_envs, sx_guided_tree tree,
-                                int32_t max_nodes, float c_puct, float fpu, sx_state leaf_states, int32_t *leaf_node_d,
-                                int8_t *leaf_kind_d, void *stream)
+static int guided_select(const char *fn, const sx_config *cfg, sx_state st, int64_t num_envs, sx_guided_tree tree,
+                         int32_t max_nodes, float c_puct, float fpu, int32_t L, float vl, int32_t *inflight_d,
+                         sx_state leaf_states, int32_t *leaf_node_d, int8_t *leaf_kind_d, void *stream)
 {
-    using namespace sx;
-    if (!cfg) return sx_set_error("sx_guided_select: null config");
-    if (!st.board || !st.aux || !st.captured) return sx_set_error("sx_guided_select: null state tensor");
-    if (null_tree(tree)) return sx_set_error("sx_guided_select: null tree pointer");
+    if (!cfg) return sx_set_error(fn_error(fn, "null config"));
+    if (!st.board || !st.aux || !st.captured) return sx_set_error(fn_error(fn, "null state tensor"));
+    if (null_tree(tree)) return sx_set_error(fn_error(fn, "null tree pointer"));
     if (!leaf_states.board || !leaf_states.aux || !leaf_states.captured || !leaf_node_d || !leaf_kind_d)
-        return sx_set_error("sx_guided_select: null leaf output");
-    if (leaf_states.board == st.board) return sx_set_error("sx_guided_select: leaf_states.board is st.board");
-    if (max_nodes < 1) return sx_set_error("sx_guided_select: max_nodes must be >= 1, got " + std::to_string(max_nodes));
+        return sx_set_error(fn_error(fn, "null leaf output"));
+    if (leaf_states.board == st.board) return sx_set_error(fn_error(fn, "leaf_states.board is st.board"));
+    if (max_nodes < 1) return sx_set_error(fn_error(fn, "max_nodes must be >= 1, got " + std::to_string(max_nodes)));
     if (!(c_puct >= 0.0f) || c_puct > 3.4028235e38f)  // NaN fails the first test, +inf the second
-        return sx_set_error("sx_guided_select: c_puct must be finite and >= 0, got " + std::to_string(c_puct));
+        return sx_set_error(fn_error(fn, "c_puct must be finite and >= 0, got " + std::to_string(c_puct)));
     if (!(fpu >= -3.4028235e38f && fpu <= 3.4028235e38f))
-        return sx_set_error("sx_guided_select: fpu must be finite, got " + std::to_string(fpu));
+        return sx_set_error(fn_error(fn, "fpu must be finite, got " + std::to_string(fpu)));
+    if (L < 1 || L > SX_GUIDED_MAX_LEAVES)
+        return sx_set_error(fn_error(fn, "leaves_per_tree must be in [1, 1024], got " + std::to_string(L)));
+    if (!(vl >= 0.0f && vl <= 16777216.0f))  // NaN fails both
+        return sx_set_error(fn_error(fn, "virtual_loss must be in [0, 2^24], got " + std::to_string(vl)));
+    if (L > 1 && !inflight_d) return sx_set_error(fn_error(fn, "null inflight buffer with leaves_per_tree > 1"));
     if (num_envs <= 0) return 0;
     const DevConfig &d = cfg->dev;
     const int warp_bytes = carve_warp(d, nullptr, nullptr);
@@ -250,27 +289,29 @@ extern "C" int sx_guided_select(const sx_config *cfg, sx_state st, int64_t num_e
                                                       sx_guided_select_kernel<8, false>);
     const unsigned grid = unsigned((num_envs + GUIDED_WARPS - 1) / GUIDED_WARPS);
     k<<<grid, GUIDED_WARPS * 32, smem, static_cast<cudaStream_t>(stream)>>>(
-        d, st.board, st.aux, st.captured, num_envs, max_nodes, c_puct, fpu, tree, leaf_states.board, leaf_states.aux,
-        leaf_states.captured, leaf_node_d, leaf_kind_d, warp_bytes);
+        d, st.board, st.aux, st.captured, num_envs, max_nodes, c_puct, fpu, L, vl, inflight_d, tree, leaf_states.board,
+        leaf_states.aux, leaf_states.captured, leaf_node_d, leaf_kind_d, warp_bytes);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : fail("sx_guided_select_kernel", e);
 }
 
-extern "C" int sx_guided_backup(const sx_config *cfg, sx_state leaf_states, int64_t num_envs, sx_guided_tree tree,
-                                int32_t max_nodes, const int32_t *leaf_node_d, const int8_t *leaf_kind_d,
-                                const void *logits_d, int32_t logits_dtype, const float *values_d, void *stream)
+static int guided_backup(const char *fn, const sx_config *cfg, sx_state leaf_states, int64_t num_envs,
+                         sx_guided_tree tree, int32_t max_nodes, int32_t L, const int32_t *leaf_node_d,
+                         const int8_t *leaf_kind_d, const void *logits_d, int32_t logits_dtype, const float *values_d,
+                         void *stream)
 {
-    using namespace sx;
-    if (!cfg) return sx_set_error("sx_guided_backup: null config");
+    if (!cfg) return sx_set_error(fn_error(fn, "null config"));
     if (!leaf_states.board || !leaf_states.aux || !leaf_states.captured)
-        return sx_set_error("sx_guided_backup: null leaf state tensor");
-    if (null_tree(tree)) return sx_set_error("sx_guided_backup: null tree pointer");
-    if (!leaf_node_d || !leaf_kind_d) return sx_set_error("sx_guided_backup: null leaf node or kind");
-    if (!logits_d) return sx_set_error("sx_guided_backup: null logits");
-    if (!values_d) return sx_set_error("sx_guided_backup: null values");
-    if (max_nodes < 1) return sx_set_error("sx_guided_backup: max_nodes must be >= 1, got " + std::to_string(max_nodes));
+        return sx_set_error(fn_error(fn, "null leaf state tensor"));
+    if (null_tree(tree)) return sx_set_error(fn_error(fn, "null tree pointer"));
+    if (!leaf_node_d || !leaf_kind_d) return sx_set_error(fn_error(fn, "null leaf node or kind"));
+    if (!logits_d) return sx_set_error(fn_error(fn, "null logits"));
+    if (!values_d) return sx_set_error(fn_error(fn, "null values"));
+    if (max_nodes < 1) return sx_set_error(fn_error(fn, "max_nodes must be >= 1, got " + std::to_string(max_nodes)));
     const int logit_bytes = logits_dtype == SX_DTYPE_F32 ? 4 : logits_dtype == SX_DTYPE_BF16 || logits_dtype == SX_DTYPE_F16 ? 2 : 0;
-    if (!logit_bytes) return sx_set_error("sx_guided_backup: unknown logits dtype " + std::to_string(logits_dtype));
+    if (!logit_bytes) return sx_set_error(fn_error(fn, "unknown logits dtype " + std::to_string(logits_dtype)));
+    if (L < 1 || L > SX_GUIDED_MAX_LEAVES)
+        return sx_set_error(fn_error(fn, "leaves_per_tree must be in [1, 1024], got " + std::to_string(L)));
     if (num_envs <= 0) return 0;
     const DevConfig &d = cfg->dev;
     const int warp_bytes = carve_warp(d, nullptr, nullptr);
@@ -280,8 +321,44 @@ extern "C" int sx_guided_backup(const sx_config *cfg, sx_state leaf_states, int6
                                                       sx_guided_backup_kernel<8, false>);
     const unsigned grid = unsigned((num_envs + GUIDED_WARPS - 1) / GUIDED_WARPS);
     k<<<grid, GUIDED_WARPS * 32, smem, static_cast<cudaStream_t>(stream)>>>(
-        d, leaf_states.board, leaf_states.aux, leaf_states.captured, num_envs, max_nodes, tree, leaf_node_d, leaf_kind_d,
-        static_cast<const uint8_t *>(logits_d), logits_dtype, logit_bytes, values_d, warp_bytes);
+        d, leaf_states.board, leaf_states.aux, leaf_states.captured, num_envs, max_nodes, L, tree, leaf_node_d,
+        leaf_kind_d, static_cast<const uint8_t *>(logits_d), logits_dtype, logit_bytes, values_d, warp_bytes);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : fail("sx_guided_backup_kernel", e);
+}
+
+}  // namespace sx
+
+extern "C" int sx_guided_select(const sx_config *cfg, sx_state st, int64_t num_envs, sx_guided_tree tree,
+                                int32_t max_nodes, float c_puct, float fpu, sx_state leaf_states, int32_t *leaf_node_d,
+                                int8_t *leaf_kind_d, void *stream)
+{
+    return sx::guided_select("sx_guided_select", cfg, st, num_envs, tree, max_nodes, c_puct, fpu, 1, 0.0f, nullptr,
+                             leaf_states, leaf_node_d, leaf_kind_d, stream);
+}
+
+extern "C" int sx_guided_select_many(const sx_config *cfg, sx_state st, int64_t num_envs, sx_guided_tree tree,
+                                     int32_t max_nodes, float c_puct, float fpu, int32_t leaves_per_tree,
+                                     float virtual_loss, int32_t *inflight_d, sx_state leaf_states,
+                                     int32_t *leaf_node_d, int8_t *leaf_kind_d, void *stream)
+{
+    return sx::guided_select("sx_guided_select_many", cfg, st, num_envs, tree, max_nodes, c_puct, fpu, leaves_per_tree,
+                             virtual_loss, inflight_d, leaf_states, leaf_node_d, leaf_kind_d, stream);
+}
+
+extern "C" int sx_guided_backup(const sx_config *cfg, sx_state leaf_states, int64_t num_envs, sx_guided_tree tree,
+                                int32_t max_nodes, const int32_t *leaf_node_d, const int8_t *leaf_kind_d,
+                                const void *logits_d, int32_t logits_dtype, const float *values_d, void *stream)
+{
+    return sx::guided_backup("sx_guided_backup", cfg, leaf_states, num_envs, tree, max_nodes, 1, leaf_node_d,
+                             leaf_kind_d, logits_d, logits_dtype, values_d, stream);
+}
+
+extern "C" int sx_guided_backup_many(const sx_config *cfg, sx_state leaf_states, int64_t num_envs,
+                                     sx_guided_tree tree, int32_t max_nodes, int32_t leaves_per_tree,
+                                     const int32_t *leaf_node_d, const int8_t *leaf_kind_d, const void *logits_d,
+                                     int32_t logits_dtype, const float *values_d, void *stream)
+{
+    return sx::guided_backup("sx_guided_backup_many", cfg, leaf_states, num_envs, tree, max_nodes, leaves_per_tree,
+                             leaf_node_d, leaf_kind_d, logits_d, logits_dtype, values_d, stream);
 }

@@ -91,6 +91,9 @@ class SearchTree:
     root_player: torch.Tensor  # int8 [B] player to move at the root (+1 / -1)
     mask_shape: tuple          # (R, C, A): the spatial valid-mask shape of one game
     prior: Optional[torch.Tensor] = None  # float32 [B, max_nodes] P, the prior under the parent (guided trees only)
+    # int32 [B, max_nodes], all zero between calls: the pending visits of a round with several leaves per tree
+    # (guided_select with leaves_per_tree > 1 creates it the first time; None until then)
+    inflight: Optional[torch.Tensor] = None
 
     def root_stats(self):
         """(visits, values) of the root's children, shaped like the valid mask [B, R, C, A]: visits int32, values in the
@@ -113,10 +116,12 @@ class SearchTree:
 
 @dataclass
 class Leaves:
-    """The leaves StrategoEngine.guided_select picked, one per tree (B rows each)."""
+    """The leaves StrategoEngine.guided_select picked, per_tree per tree (B * per_tree rows each; leaf j of tree b is
+    row b * per_tree + j)."""
     states: DeviceState        # the leaf's state: byte for byte what the steps along its path make of the root
-    node: torch.Tensor         # int32 [B] the leaf's node index in its tree
-    kind: torch.Tensor         # int8 [B] LEAF_EVAL (to be evaluated), LEAF_OVER (game over) or LEAF_STUCK (no move)
+    node: torch.Tensor         # int32 [B * per_tree] the leaf's node index in its tree
+    kind: torch.Tensor         # int8 [B * per_tree] LEAF_EVAL (to be evaluated), LEAF_OVER (game over) or LEAF_STUCK
+    per_tree: int = 1          # leaves per tree (leaves_per_tree of the select)
 
 
 LEAF_EVAL, LEAF_OVER, LEAF_STUCK = _lib.SX_LEAF_EVAL, _lib.SX_LEAF_OVER, _lib.SX_LEAF_STUCK
@@ -519,14 +524,20 @@ class StrategoEngine:
                 name, "None or " if allow_none else "", lo, hi, value))
 
     @staticmethod
-    def _check_float(name, value, lo=None):
-        """ValueError unless ``value`` is a real number (not a bool) that is finite in float32 (and >= lo)"""
-        with np.errstate(over="ignore"):
-            bad = (isinstance(value, bool) or not isinstance(value, (int, float, np.integer, np.floating))
-                   or not np.isfinite(np.float32(value)) or (lo is not None and not value >= lo))
+    def _check_float(name, value, lo=None, hi=None):
+        """ValueError unless ``value`` is a real number (not a bool) that is finite in float32 (and >= lo, <= hi)"""
+        if type(value) is float:  # the common case, without numpy's error-state context (a few us per call)
+            # 2^128 - 2^103, half an ulp above FLT_MAX: the least magnitude float32 rounding sends to infinity
+            bad = (not abs(value) < 3.4028235677973366e38 or (lo is not None and not value >= lo)
+                   or (hi is not None and not value <= hi))
+        else:
+            with np.errstate(over="ignore"):
+                bad = (isinstance(value, bool) or not isinstance(value, (int, float, np.integer, np.floating))
+                       or not np.isfinite(np.float32(value)) or (lo is not None and not value >= lo)
+                       or (hi is not None and not value <= hi))
         if bad:
-            raise ValueError("%s must be a finite number%s (in float32), not %r" % (
-                name, "" if lo is None else " >= %g" % lo, value))
+            raise ValueError("%s must be a finite number%s%s (in float32), not %r" % (
+                name, "" if lo is None else " >= %g" % lo, "" if hi is None else " <= %g" % hi, value))
 
     def search(self, state: DeviceState, iterations: int, max_nodes: Optional[int] = None,
                max_plies: Optional[int] = None, c_explore: float = 1.0, seed: int = 0, env_base: int = 0) -> "SearchTree":
@@ -599,62 +610,93 @@ class StrategoEngine:
     def _guided_struct(self, tree) -> "_lib.SxGuidedTree":
         return _lib.SxGuidedTree(*(getattr(tree, n).data_ptr() for n, _ in _lib.SxGuidedTree._fields_))
 
-    def guided_select(self, roots: DeviceState, tree: "SearchTree", c_puct: float = 1.25, fpu: float = 0.0) -> "Leaves":
-        """One leaf per tree (sx_guided_select): descend from the root of ``tree`` (the game of ``roots``) by the PUCT
-        score q + c_puct * P * sqrt(N_parent) / (1 + N), q = the mean value from the mover's side or ``fpu`` for an
-        unvisited child, ties to the lowest index, to the first node without children or whose state is over.  Returns
-        the leaves' states (ready for ``observe``, ``valid_mask``, ``export_ref_state``), node indices and kinds
-        (LEAF_EVAL, LEAF_OVER, LEAF_STUCK).  Neither ``roots`` nor ``tree`` is written, so two selects without a backup
-        between them return the same leaves.  No host synchronisation."""
+    def _check_inflight(self, tree, B: int, M: int) -> None:
+        """ValueError unless tree.inflight is None or a contiguous int32 [B, M] tensor on this engine's device"""
+        t = tree.inflight
+        if t is not None and (not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or tuple(t.shape) != (B, M)
+                              or not t.is_contiguous() or t.device != self.device):
+            raise ValueError("tree.inflight must be None or a contiguous torch.int32 tensor of shape %s on %s, not %s" % (
+                (B, M), self.device, "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor)
+                else type(t).__name__))
+
+    def guided_select(self, roots: DeviceState, tree: "SearchTree", c_puct: float = 1.25, fpu: float = 0.0,
+                      leaves_per_tree: int = 1, virtual_loss: float = 1.0) -> "Leaves":
+        """``leaves_per_tree`` = L leaves per tree (sx_guided_select_many): descend from the root of ``tree`` (the game of
+        ``roots``) by the PUCT score q + c_puct * P * sqrt(N_parent) / (1 + N), q = the mean value from the mover's side
+        or ``fpu`` for an unvisited child, ties to the lowest index, to the first node without children or whose state
+        is over.  Leaves j = 0 .. L-1 of a tree are chosen in order, each from the root: the paths of leaves 0 .. j-1
+        count as pending visits V (N + V in place of N, and each pending visit takes ``virtual_loss`` from the mover's
+        value, q = (sigma * W - virtual_loss * V) / (N + V)).  L = 1 is the one-leaf select exactly.  Returns the
+        leaves' states (ready for ``observe``, ``valid_mask``, ``export_ref_state``), node indices and kinds (LEAF_EVAL,
+        LEAF_OVER, LEAF_STUCK), B * L rows, leaf j of tree b at row b * L + j.  Neither ``roots`` nor the tree's node
+        fields are written, so two selects without a backup between them return the same leaves.  L in [1, 1024];
+        virtual_loss finite in [0, 2^24].  The first call with L > 1 on a tree gives it ``tree.inflight`` (int32
+        [B, max_nodes] zeros, all zero again after every select), so capture a CUDA graph of L > 1 rounds after one
+        warm-up round.  No host synchronisation."""
         self._check_state(roots)
         B = roots.num_envs
         M = self._check_guided_tree(tree, B)
         self._check_float("c_puct", c_puct, lo=0)
         self._check_float("fpu", fpu)
-        leaves = Leaves(self.alloc_state(B), torch.empty(B, dtype=torch.int32, device=self.device),
-                        torch.empty(B, dtype=torch.int8, device=self.device))
+        self._check_int("leaves_per_tree", leaves_per_tree, 1, _lib.SX_GUIDED_MAX_LEAVES)
+        self._check_float("virtual_loss", virtual_loss, lo=0, hi=2 ** 24)
+        self._check_inflight(tree, B, M)
+        L = int(leaves_per_tree)
+        if L > 1 and tree.inflight is None:
+            tree.inflight = torch.zeros((B, M), dtype=torch.int32, device=self.device)
+        leaves = Leaves(self.alloc_state(B * L), torch.empty(B * L, dtype=torch.int32, device=self.device),
+                        torch.empty(B * L, dtype=torch.int8, device=self.device), per_tree=L)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.sx_guided_select(self._cfg, roots.as_struct(), B, self._guided_struct(tree), M,
-                                                 float(c_puct), float(fpu), leaves.states.as_struct(),
-                                                 leaves.node.data_ptr(), leaves.kind.data_ptr(), _stream()),
-                       "sx_guided_select")
+            _lib.check(self.lib.sx_guided_select_many(self._cfg, roots.as_struct(), B, self._guided_struct(tree), M,
+                                                      float(c_puct), float(fpu), L, float(virtual_loss),
+                                                      _ptr(tree.inflight), leaves.states.as_struct(),
+                                                      leaves.node.data_ptr(), leaves.kind.data_ptr(), _stream()),
+                       "sx_guided_select_many")
         return leaves
 
     def guided_backup(self, tree: "SearchTree", leaves: "Leaves", logits: torch.Tensor, values: torch.Tensor) -> None:
-        """Expand and back up the leaves of the last ``guided_select`` (sx_guided_backup).  logits: float32, bfloat16 or
-        float16 [B, R, C, A] (or [B, R * C * A]) in the layout of ``sample_policy`` (the leaf's player-to-move frame);
-        values: float32 [B], the leaf's value from the side of its player to move.  An evaluable leaf without children
-        gets its legal moves as children (the ``expand_moves`` order) with the softmax of its logits over them as priors,
-        if the pool has room; then the leaf and its ancestors get N += 1 and W += the value in absolute terms (a finished
-        leaf's outcome, or a loss for a stuck player to move).  No host synchronisation."""
+        """Expand and back up the leaves of the last ``guided_select`` (sx_guided_backup_many), L = leaves.per_tree
+        per tree.  logits: float32, bfloat16 or float16 [B * L, R, C, A] (or [B * L, R * C * A]) in the layout of
+        ``sample_policy`` (the leaf's player-to-move frame); values: float32 [B * L], the leaf's value from the side of
+        its player to move.  The leaves of a tree are taken in order: an evaluable leaf whose node has no children yet
+        gets its legal moves as children (the ``expand_moves`` order) with the softmax of its logits over them as
+        priors, if the pool has room; then the leaf and its ancestors get N += 1 and W += the value in absolute terms
+        (a finished leaf's outcome, or a loss for a stuck player to move).  A node several leaves reached is expanded
+        once, by the first of them, and each of them backs up its own value.  No host synchronisation."""
         if not isinstance(leaves, Leaves):
             raise ValueError("leaves must be the Leaves guided_select returned, not %s" % type(leaves).__name__)
+        self._check_int("leaves.per_tree", leaves.per_tree, 1, _lib.SX_GUIDED_MAX_LEAVES)
         self._check_state(leaves.states)
-        B = leaves.states.num_envs
+        L = int(leaves.per_tree)
+        rows = leaves.states.num_envs
+        if rows % L:
+            raise ValueError("leaves must have a multiple of leaves.per_tree = %d rows, not %d" % (L, rows))
+        B = rows // L
         M = self._check_guided_tree(tree, B)
         for name, t, dtype in (("node", leaves.node, torch.int32), ("kind", leaves.kind, torch.int8)):
-            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != (B,) or not t.is_contiguous()
+            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != (rows,) or not t.is_contiguous()
                     or t.device != self.device):
-                raise ValueError("leaves.%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dtype, B,
+                raise ValueError("leaves.%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dtype, rows,
                                                                                                    self.device))
         n = self.layout.spatial_actions
-        shapes = ((B,) + tuple(self.spatial_action_size), (B, n))
+        shapes = ((rows,) + tuple(self.spatial_action_size), (rows, n))
         if (not isinstance(logits, torch.Tensor) or logits.dtype not in OBS_DTYPES or tuple(logits.shape) not in shapes
                 or not logits.is_contiguous() or logits.device != self.device):
             raise ValueError("logits must be a contiguous float32 / bfloat16 / float16 tensor of shape %s or %s on %s, "
                              "not %s" % (shapes[0], shapes[1], self.device, "%s %s on %s" % (
                                  logits.dtype, tuple(logits.shape), logits.device)
                                  if isinstance(logits, torch.Tensor) else type(logits).__name__))
-        if (not isinstance(values, torch.Tensor) or values.dtype != torch.float32 or tuple(values.shape) != (B,)
+        if (not isinstance(values, torch.Tensor) or values.dtype != torch.float32 or tuple(values.shape) != (rows,)
                 or not values.is_contiguous() or values.device != self.device):
             raise ValueError("values must be a contiguous float32 tensor of shape (%d,) on %s, not %s" % (
-                B, self.device, "%s %s on %s" % (values.dtype, tuple(values.shape), values.device)
+                rows, self.device, "%s %s on %s" % (values.dtype, tuple(values.shape), values.device)
                 if isinstance(values, torch.Tensor) else type(values).__name__))
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.sx_guided_backup(self._cfg, leaves.states.as_struct(), B, self._guided_struct(tree), M,
-                                                 leaves.node.data_ptr(), leaves.kind.data_ptr(), logits.data_ptr(),
-                                                 OBS_DTYPES[logits.dtype], values.data_ptr(), _stream()),
-                       "sx_guided_backup")
+            _lib.check(self.lib.sx_guided_backup_many(self._cfg, leaves.states.as_struct(), B, self._guided_struct(tree),
+                                                      M, L, leaves.node.data_ptr(), leaves.kind.data_ptr(),
+                                                      logits.data_ptr(), OBS_DTYPES[logits.dtype], values.data_ptr(),
+                                                      _stream()),
+                       "sx_guided_backup_many")
 
     def state_keys(self, state: DeviceState, info_set: bool = False, viewer: Optional[torch.Tensor] = None) -> torch.Tensor:
         """64-bit keys that identify positions (sx_state_keys), int64 [B]: the uint64 key bits viewed as int64, so that
