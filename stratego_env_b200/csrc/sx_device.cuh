@@ -12,6 +12,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/stratego_b200.h"
+
 // The per-lane cell loops (k < K) of the hot functions stay rolled (`#pragma unroll 1`): that keeps the fused loop small
 // enough for the instruction cache; unrolling them cost 9 % on Barrage / Standard (profiles/r2n_register_budget_sweep.txt).
 
@@ -720,6 +722,32 @@ __device__ __forceinline__ void unpack(uint4 aw, Aux &a)
     aux_unpack(w, a);
 }
 
+// writes the game staged in shared memory (board with padding, capture list) and the packed aux words `aw` to row `row`
+// of a state (one warp; the inverse of load_game)
+__device__ __forceinline__ void store_game(const DevConfig &cfg, const WarpMem &m, const uint32_t aw[4], uint8_t *board,
+                                           int16_t *aux, uint16_t *cap, long long row)
+{
+    const int lane = threadIdx.x & 31;
+    uint32_t *gb = reinterpret_cast<uint32_t *>(board + row * cfg.board_stride);
+    for (int w = lane; w < (cfg.board_stride >> 2); w += 32) gb[w] = reinterpret_cast<const uint32_t *>(m.board)[w];
+    uint32_t *gc = reinterpret_cast<uint32_t *>(cap + row * cfg.cap_stride);
+    for (int w = lane; w < (cfg.cap_stride >> 1); w += 32) gc[w] = reinterpret_cast<const uint32_t *>(m.cap)[w];
+    if (lane == 0) *reinterpret_cast<uint4 *>(aux + row * 8) = make_uint4(aw[0], aw[1], aw[2], aw[3]);
+}
+
+// the six scalars of a step that left the game in `a`, as sx_fused_kernel writes them (one lane); the caller says
+// whether the game is done and what `illegal` holds
+__device__ __forceinline__ void store_step_scalars(const sx_outputs &o, long long row, const Aux &a, bool done, int illegal)
+{
+    const int win = a.winner;
+    if (o.done) o.done[row] = done ? 1 : 0;
+    if (o.winner) o.winner[row] = int8_t(done ? win : 0);
+    if (o.ending_invalid) o.ending_invalid[row] = (done && a.invalid) ? 1 : 0;
+    if (o.illegal) o.illegal[row] = uint8_t(illegal);
+    if (o.reward) o.reward[row] = (done && !a.invalid) ? float(win) : 0.0f;  // maenv:777-801
+    if (o.player) o.player[row] = a.to_move == 0 ? 1 : -1;
+}
+
 // ---- setups / reset (impl:213-249, util:13-53, util:241-319) ---------------------------------------
 // own_map[i], i < setup_len: piece code at own-frame cell i (row-major over the usable rows).
 template <class GT>
@@ -1064,6 +1092,77 @@ __device__ __forceinline__ int sample_move(const DevConfig &cfg, const WarpMem &
     }
     const uint32_t who = GT::ballot(owner);
     return GT::shfl(action, __ffs(who) - 1);
+}
+
+// ---- per-warp helpers of the search kernels (sx_expand.cu, sx_playout.cu, sx_search.cu, sx_guided.cu; Grp<1>) ------
+
+// the moves in m.moves of this lane's K cells
+template <int K>
+__device__ __forceinline__ int lane_moves(const DevConfig &cfg, const WarpMem &m)
+{
+    const int lane = threadIdx.x & 31;
+    int mine = 0;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        const int p = lane * K + k;
+        if (p < cfg.N) mine += __popc(m.moves[p].x) + __popc(m.moves[p].y);
+    }
+    return mine;
+}
+
+// `mine`: lane_moves; `incl`: its inclusive prefix sum over the warp, so this lane's moves are numbers
+// incl - mine .. incl - 1 of the ascending list.  Returns the warp's total.
+template <int K>
+__device__ __forceinline__ int lane_move_scan(const DevConfig &cfg, const WarpMem &m, int &mine, int &incl)
+{
+    const int lane = threadIdx.x & 31;
+    mine = lane_moves<K>(cfg, m);
+    incl = mine;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int v = __shfl_up_sync(FULL, incl, d);
+        if (lane >= d) incl += v;
+    }
+    return __shfl_sync(FULL, incl, 31);
+}
+
+// fn(action) for each move of this lane's K cells in m.moves, in ascending flat spatial index
+template <int K, class F>
+__device__ __forceinline__ void for_each_lane_move(const DevConfig &cfg, const WarpMem &m, F fn)
+{
+    const int lane = threadIdx.x & 31;
+#pragma unroll 1
+    for (int k = 0; k < K; ++k) {
+        const int p = lane * K + k;
+        if (p >= cfg.N) break;
+#pragma unroll 1
+        for (int h = 0; h < 2; ++h)
+            for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1) fn(p * cfg.A + h * 32 + __ffs(w) - 1);
+    }
+}
+
+// the warp's largest (best, best_j) by score, the lowest index on a tie, on every lane; best_j < 0: the lane has none
+__device__ __forceinline__ void warp_argmax(float &best, int &best_j)
+{
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) {
+        const float ob = __shfl_xor_sync(FULL, best, d);
+        const int oj = __shfl_xor_sync(FULL, best_j, d);
+        if (oj >= 0 && (best_j < 0 || ob > best || (ob == best && oj < best_j))) { best = ob; best_j = oj; }
+    }
+}
+
+// the next game of this block's range [blockIdx.x * per_block, + per_block) below num_envs for the calling warp, or -1
+// once the range is handed out.  `claimed` is the block's __shared__ count of games handed out, zero before the first
+// call.  Games differ a lot in length, so the warps of a block take them as they finish (claim_grid sizes the launch).
+__device__ __forceinline__ long long claim_next(unsigned long long &claimed, long long per_block, long long num_envs)
+{
+    const long long first = (long long)blockIdx.x * per_block;
+    const long long end = first + per_block < num_envs ? first + per_block : num_envs;
+    long long b = 0;
+    if ((threadIdx.x & 31) == 0) b = first + (long long)atomicAdd(&claimed, 1ull);
+    b = __shfl_sync(FULL, b, 0);
+    return b < end ? b : -1;
 }
 
 }  // namespace sx

@@ -99,12 +99,7 @@ __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_select_kernel(
                     if (best_j < 0 || s > best) { best = s; best_j = c; }  // c ascends: ties keep the lower index
                 }
             }
-#pragma unroll
-            for (int d = 16; d >= 1; d >>= 1) {
-                const float ob = __shfl_xor_sync(FULL, best, d);
-                const int oj = __shfl_xor_sync(FULL, best_j, d);
-                if (oj >= 0 && (best_j < 0 || ob > best || (ob == best && oj < best_j))) { best = ob; best_j = oj; }
-            }
+            warp_argmax(best, best_j);
             // ---- step to the child: what expand_moves / sx_step make of the state with that action
             const int mover = a.to_move;
             int attack;
@@ -115,16 +110,11 @@ __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_select_kernel(
         }
         if (!a.over && !fresh) any = gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
         __syncwarp();
-        // ---- the leaf's state row, as sx_playout writes a game back
-        const int board_words = cfg.board_stride >> 2, cap_words = cfg.cap_stride >> 1;
-        uint32_t *gb = reinterpret_cast<uint32_t *>(leaf_board + r * cfg.board_stride);
-        for (int w = lane; w < board_words; w += 32) gb[w] = reinterpret_cast<const uint32_t *>(m.board)[w];
-        uint32_t *gc = reinterpret_cast<uint32_t *>(leaf_cap + r * cfg.cap_stride);
-        for (int w = lane; w < cap_words; w += 32) gc[w] = reinterpret_cast<const uint32_t *>(m.cap)[w];
+        // ---- the leaf's state row
+        uint32_t w4[4];
+        aux_pack(a, w4);
+        store_game(cfg, m, w4, leaf_board, leaf_aux, leaf_cap, r);
         if (lane == 0) {
-            uint32_t w4[4];
-            aux_pack(a, w4);
-            *reinterpret_cast<uint4 *>(leaf_aux + r * 8) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
             leaf_node[r] = v;
             leaf_kind[r] = int8_t(a.over ? SX_LEAF_OVER : any ? SX_LEAF_EVAL : SX_LEAF_STUCK);
             if (j < L - 1)  // a pending visit on the path, for the leaves after this one
@@ -172,67 +162,33 @@ __global__ void __launch_bounds__(GUIDED_WARPS * 32, 4) sx_guided_backup_kernel(
             load_game(cfg, leaf_board, leaf_aux, leaf_cap, r, m.board, m.cap);
             __syncwarp();
             gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false);
-            // this lane's moves (its K cells) and their place in the ascending list
-            int mine = 0;
-#pragma unroll 1
-            for (int k = 0; k < K; ++k) {
-                const int p = lane * K + k;
-                if (p < cfg.N) mine += __popc(m.moves[p].x) + __popc(m.moves[p].y);
-            }
-            int incl = mine;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int x = __shfl_up_sync(FULL, incl, d);
-                if (lane >= d) incl += x;
-            }
-            const int total = __shfl_sync(FULL, incl, 31);
+            int mine, incl;
+            const int total = lane_move_scan<K>(cfg, m, mine, incl);
             if (total > 0 && total <= max_nodes - used) {
                 f = used;
                 n = total;
                 const uint8_t *lrow = logits + r * (long long)(cfg.N * cfg.A) * logit_bytes;
                 // softmax over the legal entries: max, then sum of expf(x - max), both reduced over the warp
                 float mx = -INFINITY;
-#pragma unroll 1
-                for (int k = 0; k < K; ++k) {
-                    const int p = lane * K + k;
-                    if (p >= cfg.N) break;
-#pragma unroll 1
-                    for (int h = 0; h < 2; ++h)
-                        for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1)
-                            mx = fmaxf(mx, guided_logit(lrow, dtype, p * cfg.A + h * 32 + __ffs(w) - 1));
-                }
+                for_each_lane_move<K>(cfg, m, [&](int act) { mx = fmaxf(mx, guided_logit(lrow, dtype, act)); });
 #pragma unroll
                 for (int d = 16; d >= 1; d >>= 1) mx = fmaxf(mx, __shfl_xor_sync(FULL, mx, d));
                 const bool uniform = !(mx > -INFINITY);  // every legal logit is -inf: each child gets 1 / n
                 float sum = 0.0f;
                 if (!uniform) {
-#pragma unroll 1
-                    for (int k = 0; k < K; ++k) {
-                        const int p = lane * K + k;
-                        if (p >= cfg.N) break;
-#pragma unroll 1
-                        for (int h = 0; h < 2; ++h)
-                            for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1)
-                                sum = __fadd_rn(sum, expf(__fsub_rn(guided_logit(lrow, dtype, p * cfg.A + h * 32 + __ffs(w) - 1), mx)));
-                    }
+                    for_each_lane_move<K>(cfg, m, [&](int act) {
+                        sum = __fadd_rn(sum, expf(__fsub_rn(guided_logit(lrow, dtype, act), mx)));
+                    });
 #pragma unroll
                     for (int d = 16; d >= 1; d >>= 1) sum = __fadd_rn(sum, __shfl_xor_sync(FULL, sum, d));  // same on every lane
                 }
-                int t = f + incl - mine;
-#pragma unroll 1
-                for (int k = 0; k < K; ++k) {
-                    const int p = lane * K + k;
-                    if (p >= cfg.N) break;
-#pragma unroll 1
-                    for (int h = 0; h < 2; ++h) {
-                        for (uint32_t w = h ? m.moves[p].y : m.moves[p].x; w; w &= w - 1) {
-                            const int c = t++, act = p * cfg.A + h * 32 + __ffs(w) - 1;
-                            N[c] = 0; W[c] = 0.0f; parent[c] = v; first_child[c] = -1; n_children[c] = 0; action[c] = act;
-                            P[c] = uniform ? __fdiv_rn(1.0f, float(n))
-                                           : __fdiv_rn(expf(__fsub_rn(guided_logit(lrow, dtype, act), mx)), sum);
-                        }
-                    }
-                }
+                int t = f + incl - mine;  // this lane's children
+                for_each_lane_move<K>(cfg, m, [&](int act) {
+                    const int c = t++;
+                    N[c] = 0; W[c] = 0.0f; parent[c] = v; first_child[c] = -1; n_children[c] = 0; action[c] = act;
+                    P[c] = uniform ? __fdiv_rn(1.0f, float(n))
+                                   : __fdiv_rn(expf(__fsub_rn(guided_logit(lrow, dtype, act), mx)), sum);
+                });
             }
         }
         // ---- backup: the leaf and its ancestors
@@ -265,10 +221,9 @@ static int guided_select(const char *fn, const sx_config *cfg, sx_state st, int6
                          sx_state leaf_states, int32_t *leaf_node_d, int8_t *leaf_kind_d, void *stream)
 {
     if (!cfg) return sx_set_error(fn_error(fn, "null config"));
-    if (!st.board || !st.aux || !st.captured) return sx_set_error(fn_error(fn, "null state tensor"));
+    if (null_state(st)) return sx_set_error(fn_error(fn, "null state tensor"));
     if (null_tree(tree)) return sx_set_error(fn_error(fn, "null tree pointer"));
-    if (!leaf_states.board || !leaf_states.aux || !leaf_states.captured || !leaf_node_d || !leaf_kind_d)
-        return sx_set_error(fn_error(fn, "null leaf output"));
+    if (null_state(leaf_states) || !leaf_node_d || !leaf_kind_d) return sx_set_error(fn_error(fn, "null leaf output"));
     if (leaf_states.board == st.board) return sx_set_error(fn_error(fn, "leaf_states.board is st.board"));
     if (max_nodes < 1) return sx_set_error(fn_error(fn, "max_nodes must be >= 1, got " + std::to_string(max_nodes)));
     if (!(c_puct >= 0.0f) || c_puct > 3.4028235e38f)  // NaN fails the first test, +inf the second
@@ -301,8 +256,7 @@ static int guided_backup(const char *fn, const sx_config *cfg, sx_state leaf_sta
                          void *stream)
 {
     if (!cfg) return sx_set_error(fn_error(fn, "null config"));
-    if (!leaf_states.board || !leaf_states.aux || !leaf_states.captured)
-        return sx_set_error(fn_error(fn, "null leaf state tensor"));
+    if (null_state(leaf_states)) return sx_set_error(fn_error(fn, "null leaf state tensor"));
     if (null_tree(tree)) return sx_set_error(fn_error(fn, "null tree pointer"));
     if (!leaf_node_d || !leaf_kind_d) return sx_set_error(fn_error(fn, "null leaf node or kind"));
     if (!logits_d) return sx_set_error(fn_error(fn, "null logits"));

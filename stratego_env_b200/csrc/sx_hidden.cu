@@ -174,8 +174,8 @@ extern "C" int sx_sample_hidden_states(const sx_config *cfg, sx_state st, int64_
 {
     using namespace sx;
     if (!cfg) return sx_set_error("sx_sample_hidden_states: null config");
-    if (!st.board || !st.aux || !st.captured) return sx_set_error("sx_sample_hidden_states: null state tensor");
-    if (!out.board || !out.aux || !out.captured) return sx_set_error("sx_sample_hidden_states: null out tensor");
+    if (null_state(st)) return sx_set_error("sx_sample_hidden_states: null state tensor");
+    if (null_state(out)) return sx_set_error("sx_sample_hidden_states: null out tensor");
     if (n_samples < 1 || n_samples >= (1 << 24))
         return sx_set_error("sx_sample_hidden_states: n_samples must be in [1, 2^24), got " + std::to_string(n_samples));
     // rows * board_stride (<= 240 bytes) must stay a valid int64 byte offset
@@ -195,5 +195,5 @@ extern "C" int sx_sample_hidden_states(const sx_config *cfg, sx_state st, int64_
         d, st.board, st.aux, st.captured, num_envs, env_base, viewer_d, n_samples, key, draw, out.board, out.aux,
         out.captured, status_d, warp_bytes);
     const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : sx_set_error(std::string("sx_sample_hidden_kernel: ") + cudaGetErrorString(e));
+    return e == cudaSuccess ? 0 : fail("sx_sample_hidden_kernel", e);
 }

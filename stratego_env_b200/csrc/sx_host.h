@@ -39,7 +39,7 @@ bool sx_in_compressible_allocation(const void *p);
 
 namespace sx {
 
-// the instantiation of a one-warp-per-game search kernel (sx_expand.cu, sx_playout.cu), as launch_policy
+// the instantiation of a one-warp-per-game search kernel (sx_expand.cu, sx_playout.cu, sx_search.cu, sx_guided.cu), as launch_policy
 // (sx_policy.cu) picks it: cells per lane by board size, compact movers where configured
 template <class F>
 inline F pick(const sx_config *cfg, F k2, F k4, F k4cm, F k8)
@@ -49,6 +49,17 @@ inline F pick(const sx_config *cfg, F k2, F k4, F k4cm, F k8)
 }
 
 inline int fail(const char *who, cudaError_t e) { return sx_set_error(std::string(who) + ": " + cudaGetErrorString(e)); }
+
+inline bool null_state(const sx_state &s) { return !s.board || !s.aux || !s.captured; }
+
+// expand and playout write the six step scalars of sx_outputs and nothing else
+inline bool scalars_only(const sx_outputs &o)
+{
+    return !o.partial_obs && !o.full_obs && !o.valid_mask && !o.next_action && !o.terminal_partial_obs &&
+           !o.terminal_full_obs;
+}
+constexpr const char *NOT_SCALARS_ONLY = ": only reward, done, winner, ending_invalid, illegal and player are written; "
+                                         "observation, mask, next_action and terminal outputs must be null";
 
 // the blocks of `threads` threads and `smem` bytes of shared memory that the current device holds at once, at most
 // `wanted`, at least 1
@@ -61,6 +72,18 @@ inline cudaError_t resident_grid(F kernel, int threads, size_t smem, long long w
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
     const long long most = (long long)(per_sm > 1 ? per_sm : 1) * sms;
     grid = unsigned(wanted < 1 ? 1 : wanted < most ? wanted : most);
+    return e;
+}
+
+// the launch of a kernel of `warps`-warp blocks that take their games with claim_next (sx_device.cuh): the resident
+// blocks, at most one per `warps` games, each with a contiguous range of per_block games, and no block without one
+template <class F>
+inline cudaError_t claim_grid(F kernel, int warps, size_t smem, long long num_envs, unsigned &grid, long long &per_block)
+{
+    const cudaError_t e = resident_grid(kernel, warps * 32, smem, (num_envs + warps - 1) / warps, grid);
+    if (e != cudaSuccess) return e;
+    per_block = (num_envs + grid - 1) / grid;
+    grid = unsigned((num_envs + per_block - 1) / per_block);
     return e;
 }
 

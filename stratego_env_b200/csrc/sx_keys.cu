@@ -141,7 +141,7 @@ extern "C" int sx_state_keys(const sx_config *cfg, sx_state st, int64_t num_envs
 {
     using namespace sx;
     if (!cfg) return sx_set_error("sx_state_keys: null config");
-    if (!st.board || !st.aux || !st.captured) return sx_set_error("sx_state_keys: null state tensor");
+    if (null_state(st)) return sx_set_error("sx_state_keys: null state tensor");
     if (!keys_d) return sx_set_error("sx_state_keys: null keys");
     if (mode != SX_KEY_STATE && mode != SX_KEY_INFOSET)
         return sx_set_error("sx_state_keys: unknown mode " + std::to_string(mode));

@@ -39,14 +39,7 @@ __global__ void __launch_bounds__(PLAYOUT_WARPS * 32, 4) sx_playout_kernel(
     __syncthreads();
     WarpMem m;
     carve_warp(cfg, smem + size_t(warp) * warp_bytes, &m);
-    const long long first = (long long)blockIdx.x * per_block;
-    const long long end = first + per_block < num_envs ? first + per_block : num_envs;
-    const int board_words = cfg.board_stride >> 2, cap_words = cfg.cap_stride >> 1;
-    for (;;) {
-        long long b = 0;
-        if (lane == 0) b = first + (long long)atomicAdd(&claimed, 1ull);
-        b = __shfl_sync(FULL, b, 0);
-        if (b >= end) break;
+    for (long long b; (b = claim_next(claimed, per_block, num_envs)) >= 0;) {
         Aux a;
         unpack(load_game(cfg, board, aux, cap, b, m.board, m.cap), a);
         __syncwarp();
@@ -69,26 +62,13 @@ __global__ void __launch_bounds__(PLAYOUT_WARPS * 32, 4) sx_playout_kernel(
                 any = after_move<K, GT, CM>(cfg, m, a, mover);
                 if (a.over || plies >= max_plies) break;
             }
-            uint32_t *gb = reinterpret_cast<uint32_t *>(board + b * cfg.board_stride);
-            for (int w = lane; w < board_words; w += 32) gb[w] = reinterpret_cast<const uint32_t *>(m.board)[w];
-            uint32_t *gc = reinterpret_cast<uint32_t *>(cap + b * cfg.cap_stride);
-            for (int w = lane; w < cap_words; w += 32) gc[w] = reinterpret_cast<const uint32_t *>(m.cap)[w];
-            if (lane == 0) {
-                uint32_t w4[4];
-                aux_pack(a, w4);
-                *reinterpret_cast<uint4 *>(aux + b * 8) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-            }
+            uint32_t w4[4];
+            aux_pack(a, w4);
+            store_game(cfg, m, w4, board, aux, cap, b);
         }
-        if (lane == 0) {  // the scalars of the step that ended the game, as sx_fused_kernel writes them
-            const bool done = a.over;
-            const int win = a.winner;
+        if (lane == 0) {  // the scalars of the step that ended the game
             if (plies_out) plies_out[b] = plies;
-            if (o.done) o.done[b] = done ? 1 : 0;
-            if (o.winner) o.winner[b] = int8_t(done ? win : 0);
-            if (o.ending_invalid) o.ending_invalid[b] = (done && a.invalid) ? 1 : 0;
-            if (o.illegal) o.illegal[b] = a.overflow ? 2 : 0;
-            if (o.reward) o.reward[b] = (done && !a.invalid) ? float(win) : 0.0f;  // maenv:777-801
-            if (o.player) o.player[b] = a.to_move == 0 ? 1 : -1;
+            store_step_scalars(o, b, a, a.over, a.overflow ? 2 : 0);
         }
         __syncwarp();  // the next game overwrites this one's slice
     }
@@ -104,12 +84,10 @@ extern "C" int sx_playout(const sx_config *cfg, sx_state st, int64_t num_envs, i
 {
     using namespace sx;
     if (!cfg) return sx_set_error("sx_playout: null config");
-    if (!st.board || !st.aux || !st.captured) return sx_set_error("sx_playout: null state tensor");
+    if (null_state(st)) return sx_set_error("sx_playout: null state tensor");
     if (max_plies < 0) return sx_set_error("sx_playout: max_plies must be >= 0, got " + std::to_string(max_plies));
     const sx_outputs &o = out_scalars;
-    if (o.partial_obs || o.full_obs || o.valid_mask || o.next_action || o.terminal_partial_obs || o.terminal_full_obs)
-        return sx_set_error("sx_playout: only reward, done, winner, ending_invalid, illegal and player are written; "
-                            "observation, mask, next_action and terminal outputs must be null");
+    if (!scalars_only(o)) return sx_set_error(std::string("sx_playout") + NOT_SCALARS_ONLY);
     if (num_envs <= 0) return 0;
     const DevConfig &d = cfg->dev;
     const int warp_bytes = carve_warp(d, nullptr, nullptr);
@@ -117,10 +95,9 @@ extern "C" int sx_playout(const sx_config *cfg, sx_state st, int64_t num_envs, i
     const playout_fn k = pick<playout_fn>(cfg, sx_playout_kernel<2, false>, sx_playout_kernel<4, false>,
                                           sx_playout_kernel<4, true>, sx_playout_kernel<8, false>);
     unsigned grid = 0;
-    cudaError_t e = resident_grid(k, PLAYOUT_WARPS * 32, smem, (num_envs + PLAYOUT_WARPS - 1) / PLAYOUT_WARPS, grid);
+    long long per_block = 0;
+    cudaError_t e = claim_grid(k, PLAYOUT_WARPS, smem, num_envs, grid, per_block);
     if (e != cudaSuccess) return fail("sx_playout", e);
-    const long long per_block = (num_envs + grid - 1) / grid;
-    grid = unsigned((num_envs + per_block - 1) / per_block);
     const uint2 key = make_uint2(uint32_t(seed), uint32_t(seed >> 32));
     k<<<grid, PLAYOUT_WARPS * 32, smem, static_cast<cudaStream_t>(stream)>>>(d, st.board, st.aux, st.captured, num_envs,
                                                                            env_base, per_block, max_plies, key, plies_d, o,

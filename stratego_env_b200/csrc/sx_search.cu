@@ -43,13 +43,7 @@ __global__ void __launch_bounds__(SEARCH_WARPS * 32, 4) sx_search_kernel(
     __syncthreads();
     WarpMem m;
     carve_warp(cfg, smem + size_t(warp) * warp_bytes, &m);
-    const long long first = (long long)blockIdx.x * per_block;
-    const long long end = first + per_block < num_envs ? first + per_block : num_envs;
-    for (;;) {
-        long long b = 0;
-        if (lane == 0) b = first + (long long)atomicAdd(&claimed, 1ull);
-        b = __shfl_sync(FULL, b, 0);
-        if (b >= end) break;
+    for (long long b; (b = claim_next(claimed, per_block, num_envs)) >= 0;) {
         const uint64_t gid = uint64_t(env_base + b);
         const long long row = b * (long long)max_nodes;
         int32_t *const N = tree.visits + row, *const W = tree.value + row, *const parent = tree.parent + row;
@@ -69,39 +63,15 @@ __global__ void __launch_bounds__(SEARCH_WARPS * 32, 4) sx_search_kernel(
                 int f = first_child[v], n = n_children[v];
                 if (f < 0) {
                     if (!fresh) { any = gen_moves<K, GT, CM>(cfg, m, a, a.to_move, false); fresh = true; }
-                    // this lane's moves (its K cells) and their place in the ascending list
-                    int mine = 0;
-#pragma unroll 1
-                    for (int k = 0; k < K; ++k) {
-                        const int p = lane * K + k;
-                        if (p < cfg.N) mine += __popc(m.moves[p].x) + __popc(m.moves[p].y);
-                    }
-                    int incl = mine;
-#pragma unroll
-                    for (int d = 1; d < 32; d <<= 1) {
-                        const int x = __shfl_up_sync(FULL, incl, d);
-                        if (lane >= d) incl += x;
-                    }
-                    n = __shfl_sync(FULL, incl, 31);
+                    int mine, incl;
+                    n = lane_move_scan<K>(cfg, m, mine, incl);
                     if (n == 0 || n > max_nodes - used) break;  // a stuck player, or no room: v stays a leaf
                     f = used;
-                    int t = f + incl - mine;
-#pragma unroll 1
-                    for (int k = 0; k < K; ++k) {
-                        const int p = lane * K + k;
-                        if (p >= cfg.N) break;
-                        const uint2 bits = m.moves[p];
-#pragma unroll 1
-                        for (int h = 0; h < 2; ++h) {
-                            uint32_t w = h ? bits.y : bits.x;
-                            while (w) {
-                                const int c = t++;
-                                N[c] = 0; W[c] = 0; parent[c] = v; first_child[c] = -1; n_children[c] = 0;
-                                action[c] = p * cfg.A + h * 32 + __ffs(w) - 1;
-                                w &= w - 1;
-                            }
-                        }
-                    }
+                    int t = f + incl - mine;  // this lane's children
+                    for_each_lane_move<K>(cfg, m, [&](int act) {
+                        const int c = t++;
+                        N[c] = 0; W[c] = 0; parent[c] = v; first_child[c] = -1; n_children[c] = 0; action[c] = act;
+                    });
                     if (lane == 0) { first_child[v] = f; n_children[v] = n; }
                     used += n;
                     __syncwarp();  // the children's fields, written by their lanes, are read below by others
@@ -128,12 +98,7 @@ __global__ void __launch_bounds__(SEARCH_WARPS * 32, 4) sx_search_kernel(
                 if (fresh_child >= 0) {
                     c = fresh_child;
                 } else {
-#pragma unroll
-                    for (int d = 16; d >= 1; d >>= 1) {
-                        const float ob = __shfl_xor_sync(FULL, best, d);
-                        const int oj = __shfl_xor_sync(FULL, best_j, d);
-                        if (oj >= 0 && (best_j < 0 || ob > best || (ob == best && oj < best_j))) { best = ob; best_j = oj; }
-                    }
+                    warp_argmax(best, best_j);
                     c = best_j;
                 }
                 // ---- step to the child: what expand_moves / sx_step make of s with that action
@@ -184,7 +149,7 @@ extern "C" int sx_search(const sx_config *cfg, sx_state st, int64_t num_envs, in
 {
     using namespace sx;
     if (!cfg) return sx_set_error("sx_search: null config");
-    if (!st.board || !st.aux || !st.captured) return sx_set_error("sx_search: null state tensor");
+    if (null_state(st)) return sx_set_error("sx_search: null state tensor");
     if (!tree.visits || !tree.value || !tree.parent || !tree.first_child || !tree.n_children || !tree.action || !tree.used)
         return sx_set_error("sx_search: null tree pointer");
     if (iterations < 0 || iterations > (1 << 24))
@@ -200,10 +165,9 @@ extern "C" int sx_search(const sx_config *cfg, sx_state st, int64_t num_envs, in
     const search_fn k = pick<search_fn>(cfg, sx_search_kernel<2, false>, sx_search_kernel<4, false>,
                                         sx_search_kernel<4, true>, sx_search_kernel<8, false>);
     unsigned grid = 0;
-    cudaError_t e = resident_grid(k, SEARCH_WARPS * 32, smem, (num_envs + SEARCH_WARPS - 1) / SEARCH_WARPS, grid);
+    long long per_block = 0;
+    cudaError_t e = claim_grid(k, SEARCH_WARPS, smem, num_envs, grid, per_block);
     if (e != cudaSuccess) return fail("sx_search", e);
-    const long long per_block = (num_envs + grid - 1) / grid;
-    grid = unsigned((num_envs + per_block - 1) / per_block);
     const uint2 key = make_uint2(uint32_t(seed), uint32_t(seed >> 32));
     k<<<grid, SEARCH_WARPS * 32, smem, static_cast<cudaStream_t>(stream)>>>(d, st.board, st.aux, st.captured, num_envs,
                                                                           env_base, per_block, iterations, max_nodes,

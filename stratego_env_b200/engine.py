@@ -449,21 +449,31 @@ class StrategoEngine:
             raise ValueError("viewer must be None or an integer tensor of shape (%d,), not %s" % (
                 B, "%s %s" % (viewer.dtype, tuple(viewer.shape)) if isinstance(viewer, torch.Tensor) else type(viewer).__name__))
 
+    def _check_tensor(self, name, t, dtypes, shapes) -> None:
+        """ValueError unless ``t`` is a contiguous tensor of one of ``dtypes`` and one of ``shapes`` on this engine's
+        device (checked on the host, before any device is touched)"""
+        if (not isinstance(t, torch.Tensor) or t.dtype not in dtypes or t.shape not in shapes or not t.is_contiguous()
+                or t.device != self.device):
+            raise ValueError("%s must be a contiguous %s tensor of shape %s on %s, not %s" % (
+                name, " / ".join(map(str, dtypes)), " or ".join(map(str, shapes)), self.device,
+                "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor) else type(t).__name__))
+
     def _check_state(self, state) -> None:
         """ValueError unless ``state`` is a DeviceState of contiguous tensors in this engine's dtypes, strides and
-        device (checked on the host, before any device is touched)"""
+        device"""
         lay = self.layout
         if not isinstance(state, DeviceState):
             raise ValueError("state must be a DeviceState, not %s" % type(state).__name__)
         B = state.num_envs
-        for name, t, dtype, width in (("board", state.board, torch.uint8, lay.board_stride),
-                                      ("aux", state.aux, torch.int16, lay.aux_stride),
-                                      ("captured", state.captured, torch.int16, lay.captured_stride)):
-            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != (B, width)
-                    or not t.is_contiguous() or t.device != self.device):
-                raise ValueError("state.%s must be a contiguous %s tensor of shape (%d, %d) on %s, not %s" % (
-                    name, dtype, B, width, self.device,
-                    "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor) else type(t).__name__))
+        for name, t, dtype, width in (("state.board", state.board, torch.uint8, lay.board_stride),
+                                      ("state.aux", state.aux, torch.int16, lay.aux_stride),
+                                      ("state.captured", state.captured, torch.int16, lay.captured_stride)):
+            self._check_tensor(name, t, (dtype,), ((B, width),))
+
+    @staticmethod
+    def _root_player(state: DeviceState) -> torch.Tensor:
+        """int8 [B]: the player to move in each game (+1 / -1), from aux_pack's to_move bit"""
+        return torch.where(((state.aux[:, 2] >> 4) & 1) == 0, 1, -1).to(torch.int8)
 
     def expand_moves(self, state: DeviceState) -> "Expansion":
         """The children of every game (sx_count_moves + sx_expand_moves): one per legal move of the player to move, in
@@ -566,7 +576,7 @@ class StrategoEngine:
             _lib.check(self.lib.sx_search(self._cfg, state.as_struct(), B, int(env_base), int(iterations), M,
                                           (1 << 31) - 1 if max_plies is None else int(max_plies), float(c_explore),
                                           seed & (2 ** 64 - 1), tree, _stream()), "sx_search")
-            root_player = torch.where(((state.aux[:, 2] >> 4) & 1) == 0, 1, -1).to(torch.int8)  # aux_pack: to_move
+            root_player = self._root_player(state)
         return SearchTree(*f, used=used, root_player=root_player,
                           mask_shape=(self.rows, self.columns, self.spatial_channels))
 
@@ -585,8 +595,8 @@ class StrategoEngine:
                      (prior, 1.0)):
             t[:, 0].fill_(x)
         used = torch.ones(B, dtype=torch.int32, device=d)
-        root_player = torch.where(((roots.aux[:, 2] >> 4) & 1) == 0, 1, -1).to(torch.int8)  # aux_pack: to_move
-        return SearchTree(visits, value, parent, first_child, n_children, action, used=used, root_player=root_player,
+        return SearchTree(visits, value, parent, first_child, n_children, action, used=used,
+                          root_player=self._root_player(roots),
                           mask_shape=(self.rows, self.columns, self.spatial_channels), prior=prior)
 
     def _check_guided_tree(self, tree, B: int) -> int:
@@ -594,30 +604,20 @@ class StrategoEngine:
         if not isinstance(tree, SearchTree) or not isinstance(tree.prior, torch.Tensor):
             raise ValueError("tree must be a SearchTree made by guided_tree, not %s" % type(tree).__name__)
         M = tree.visits.shape[1] if isinstance(tree.visits, torch.Tensor) and tree.visits.dim() == 2 else -1
-        for name in ("visits", "value", "parent", "first_child", "n_children", "action", "prior", "used"):
-            t = getattr(tree, name)
-            dtype = torch.float32 if name in ("value", "prior") else torch.int32
-            shape = (B,) if name == "used" else (B, M)
-            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != shape or not t.is_contiguous()
-                    or t.device != self.device):
-                raise ValueError("tree.%s must be a contiguous %s tensor of shape %s on %s, not %s" % (
-                    name, dtype, shape, self.device,
-                    "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor) else type(t).__name__))
+        i32, f32, nodes = (torch.int32,), (torch.float32,), ((B, M),)
+        for name, t, dtypes, shapes in (("tree.visits", tree.visits, i32, nodes), ("tree.value", tree.value, f32, nodes),
+                                        ("tree.parent", tree.parent, i32, nodes),
+                                        ("tree.first_child", tree.first_child, i32, nodes),
+                                        ("tree.n_children", tree.n_children, i32, nodes),
+                                        ("tree.action", tree.action, i32, nodes), ("tree.prior", tree.prior, f32, nodes),
+                                        ("tree.used", tree.used, i32, ((B,),))):
+            self._check_tensor(name, t, dtypes, shapes)
         if M < 1:
             raise ValueError("tree must have max_nodes >= 1, not %d" % M)
         return M
 
     def _guided_struct(self, tree) -> "_lib.SxGuidedTree":
         return _lib.SxGuidedTree(*(getattr(tree, n).data_ptr() for n, _ in _lib.SxGuidedTree._fields_))
-
-    def _check_inflight(self, tree, B: int, M: int) -> None:
-        """ValueError unless tree.inflight is None or a contiguous int32 [B, M] tensor on this engine's device"""
-        t = tree.inflight
-        if t is not None and (not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or tuple(t.shape) != (B, M)
-                              or not t.is_contiguous() or t.device != self.device):
-            raise ValueError("tree.inflight must be None or a contiguous torch.int32 tensor of shape %s on %s, not %s" % (
-                (B, M), self.device, "%s %s on %s" % (t.dtype, tuple(t.shape), t.device) if isinstance(t, torch.Tensor)
-                else type(t).__name__))
 
     def guided_select(self, roots: DeviceState, tree: "SearchTree", c_puct: float = 1.25, fpu: float = 0.0,
                       leaves_per_tree: int = 1, virtual_loss: float = 1.0) -> "Leaves":
@@ -640,7 +640,8 @@ class StrategoEngine:
         self._check_float("fpu", fpu)
         self._check_int("leaves_per_tree", leaves_per_tree, 1, _lib.SX_GUIDED_MAX_LEAVES)
         self._check_float("virtual_loss", virtual_loss, lo=0, hi=2 ** 24)
-        self._check_inflight(tree, B, M)
+        if tree.inflight is not None:
+            self._check_tensor("tree.inflight", tree.inflight, (torch.int32,), ((B, M),))
         L = int(leaves_per_tree)
         if L > 1 and tree.inflight is None:
             tree.inflight = torch.zeros((B, M), dtype=torch.int32, device=self.device)
@@ -673,24 +674,11 @@ class StrategoEngine:
             raise ValueError("leaves must have a multiple of leaves.per_tree = %d rows, not %d" % (L, rows))
         B = rows // L
         M = self._check_guided_tree(tree, B)
-        for name, t, dtype in (("node", leaves.node, torch.int32), ("kind", leaves.kind, torch.int8)):
-            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != (rows,) or not t.is_contiguous()
-                    or t.device != self.device):
-                raise ValueError("leaves.%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dtype, rows,
-                                                                                                   self.device))
-        n = self.layout.spatial_actions
-        shapes = ((rows,) + tuple(self.spatial_action_size), (rows, n))
-        if (not isinstance(logits, torch.Tensor) or logits.dtype not in OBS_DTYPES or tuple(logits.shape) not in shapes
-                or not logits.is_contiguous() or logits.device != self.device):
-            raise ValueError("logits must be a contiguous float32 / bfloat16 / float16 tensor of shape %s or %s on %s, "
-                             "not %s" % (shapes[0], shapes[1], self.device, "%s %s on %s" % (
-                                 logits.dtype, tuple(logits.shape), logits.device)
-                                 if isinstance(logits, torch.Tensor) else type(logits).__name__))
-        if (not isinstance(values, torch.Tensor) or values.dtype != torch.float32 or tuple(values.shape) != (rows,)
-                or not values.is_contiguous() or values.device != self.device):
-            raise ValueError("values must be a contiguous float32 tensor of shape (%d,) on %s, not %s" % (
-                rows, self.device, "%s %s on %s" % (values.dtype, tuple(values.shape), values.device)
-                if isinstance(values, torch.Tensor) else type(values).__name__))
+        self._check_tensor("leaves.node", leaves.node, (torch.int32,), ((rows,),))
+        self._check_tensor("leaves.kind", leaves.kind, (torch.int8,), ((rows,),))
+        self._check_tensor("logits", logits, tuple(OBS_DTYPES),
+                           ((rows,) + tuple(self.spatial_action_size), (rows, self.layout.spatial_actions)))
+        self._check_tensor("values", values, (torch.float32,), ((rows,),))
         with torch.cuda.device(self.device):
             _lib.check(self.lib.sx_guided_backup_many(self._cfg, leaves.states.as_struct(), B, self._guided_struct(tree),
                                                       M, L, leaves.node.data_ptr(), leaves.kind.data_ptr(),
@@ -825,7 +813,7 @@ class StrategoEngine:
         flat_logits = logits.reshape(B, -1)
         assert flat_mask.dtype == torch.uint8 and flat_mask.is_contiguous() and flat_logits.is_contiguous()
         assert flat_logits.shape == flat_mask.shape, (flat_logits.shape, flat_mask.shape)
-        dtype = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}[flat_logits.dtype]
+        dtype = OBS_DTYPES[flat_logits.dtype]
         actions = torch.empty(B, dtype=torch.int32, device=self.device)
         logprob = torch.empty(B, dtype=torch.float32, device=self.device) if return_logprob else None
         with torch.cuda.device(self.device):
@@ -843,7 +831,7 @@ class StrategoEngine:
         B = state.num_envs
         flat_logits = logits.reshape(B, -1)
         assert flat_logits.is_contiguous() and flat_logits.shape[1] == self.layout.spatial_actions, flat_logits.shape
-        dtype = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}[flat_logits.dtype]
+        dtype = OBS_DTYPES[flat_logits.dtype]
         actions = torch.empty(B, dtype=torch.int32, device=self.device)
         logprob = torch.empty(B, dtype=torch.float32, device=self.device) if return_logprob else None
         with torch.cuda.device(self.device):
